@@ -23,6 +23,9 @@ The line proves itself:
   transit      the transit-geometry configuration (demo BART_transit.cfg shape) on the same GPU
 `--impl reference` times the unmodified reference C (oracle/_ref; else the oracle port) on the host
 cores for the same configuration.
+`--dump-outputs DIR` saves what the last timed step of the device leg and of the two host legs
+returned (band fluxes, spectra and status of a seeded sample of the models), so that two builds can
+be compared output for output on the same seeded inputs.
 """
 import argparse
 import csv
@@ -47,6 +50,10 @@ WORKLOAD = ("WASP-12b eclipse (examples/WASP-12b/BART.cfg shape): 2424 wavenumbe
             "x 100 layers x 27 grid temperatures x 4 molecules (H2O CO2 CO CH4) + H2-H2 CIA, "
             "5 ray angles, toomuch 10, 4 filters")
 PARITY_TOL = 1e-6
+# --dump-outputs keeps the outputs of this many models, the same seeded sample in every array (~10 MB
+# at the W12 shape), and never writes more than DUMP_LIMIT bytes
+DUMP_MODELS = 512
+DUMP_LIMIT = 64 << 20
 
 
 def env_int(name, default):
@@ -251,7 +258,12 @@ def main():
     ap.add_argument("--models", type=int, default=4096, help="proposal models per GPU per step")
     ap.add_argument("--no-cpu-baseline", action="store_true", help="skip the CPU legs (and with them the parity gate)")
     ap.add_argument("--no-extras", action="store_true", help="skip the ncu / hr_lookup / builder / latency legs")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step of each timed leg returned as DIR/<name>.npy "
+                         "(float64, for a fixed sample of %d models per rank)" % DUMP_MODELS)
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         return run_reference_arm(args)
 
@@ -329,6 +341,14 @@ def main():
     L.bart_profile_enable(0)
     stats = api.kernel_stats()
     total_ms = float(np.sum(ms))
+    # --dump-outputs: the band fluxes of the last timed step (the gathered blocks of every rank for N>1,
+    # rank after rank), read before any later leg reuses the buffers
+    dumps = {}
+    if args.dump_outputs:
+        dump_rows = np.sort(np.random.default_rng(0).choice(M, min(M, DUMP_MODELS), replace=False))
+        band = np.empty((world, M, nf))
+        api._check(L.bart_memcpy_d2h(band.ctypes.data, d_all if world > 1 else d_band, band.nbytes))
+        dumps["band_flux"] = band[:, dump_rows].reshape(-1, nf)
 
     # N>1: what the fused all-gather delivered, against a local recompute of a sample of every
     # rank's models (each rank's batch is seeded by its rank, so any rank can rebuild it)
@@ -366,6 +386,9 @@ def main():
         tr.run_batch(h_in.array, out=h_out.array, status=st)
         e2e_ms.append(1e3 * (time.perf_counter() - t0))
     e2e_total = float(np.sum(e2e_ms))
+    if args.dump_outputs:
+        dumps["e2e_spectra"] = h_out.array[dump_rows]
+        dumps["e2e_status"] = st[dump_rows]
     # the same, returning what BART consumes (band fluxes, BARTfunc.py:386-399) instead of spectra
     for _ in range(2):
         tr.bandflux_batch(h_in.array, out=h_band.array, status=st)
@@ -377,6 +400,9 @@ def main():
         tr.bandflux_batch(h_in.array, out=h_band.array, status=st)
         e2b_ms.append(1e3 * (time.perf_counter() - t0))
     e2b_total = float(np.sum(e2b_ms))
+    if args.dump_outputs:
+        dumps["e2e_band_flux"] = h_band.array[dump_rows]
+        dumps["e2e_band_status"] = st[dump_rows]
     # nvidia-smi can take longer to start than a short run lasts (8 ranks on one box): keep the
     # same step running, untimed, until the sampler has seen the GPU under this load
     t_wait = time.time()
@@ -556,6 +582,12 @@ def main():
             line["transit"] = transit
         if rc:
             line["valid"] = False
+        if args.dump_outputs:
+            out = {name: np.ascontiguousarray(a, dtype=np.float64) for name, a in dumps.items()}
+            assert sum(a.nbytes for a in out.values()) <= DUMP_LIMIT, "--dump-outputs over %d bytes" % DUMP_LIMIT
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            for name, a in out.items():
+                np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
         print(json.dumps(line))
     if dist is not None:
         L.bart_comm_finalize()
