@@ -17,8 +17,11 @@ dp = C.POINTER(C.c_double)
 ip = C.POINTER(C.c_int)
 
 REJ_TGRID, REJ_TCIA, REJ_SUMQ, REJ_FEWPTS = 1, 2, 4, 8
+REJ_TBOUNDS = 16        # converter: a layer outside [Tmin, Tmax] (BARTfunc.py:327-330)
+REJ_ABUND = 32          # converter: the metals' abundances sum past 1 (BARTfunc.py:339-344)
 REJ_NOTOOMUCH = 64
 REJ_ENERGY = 128
+REJ_PTMODEL = 256       # converter: PT.py refuses the parameters (BARTfunc.py:323-325)
 
 
 class BartError(RuntimeError):

@@ -1217,6 +1217,16 @@ void upload_exp_table(const DevConfig &c, cudaStream_t s) {
   cudaStreamSynchronize(s);
 }
 
+// Dynamic shared memory of the column kernels.  Every launch stages the model's whole table (one
+// record per layer), so the shared memory of one block bounds the layer count a configuration can
+// run: column_smem_fits() below holds these sizes against the device.
+static size_t eclipse_smem(const DevConfig &c) {          // throughput, slot and scan kernels
+  return ((size_t)c.lay.stride() + ecl_tab_entries(c.nang)) * sizeof(double);
+}
+static size_t transit_tile_smem(const DevConfig &c) {     // the DFMA tile kernel
+  return table_smem(c) + ((size_t)c.nlayer * (kTrRow + kTrW) + (size_t)2 * kTrChunk * kTrW) * sizeof(double);
+}
+
 void launch_grid_relayout(const double *in, double *out, int ncells, int nmol, int gms, int nwave,
                           cudaStream_t s) {
   grid_relayout_kernel<<<148 * 8, 256, 0, s>>>(in, out, ncells, nmol, gms, nwave);
@@ -1265,7 +1275,7 @@ template <int NMOL, int NCIA, int NANG, bool KEEP, int SQ = -1, bool SC = true>
 static void launch_eclipse_t(const DevConfig &c, const double *tabs, const int *status,
                              double *spectra, double *tau_keep, int *last_keep, int nmodels,
                              int use_tma, int small, cudaStream_t s) {
-  const size_t smem = ((size_t)c.lay.stride() + ecl_tab_entries(c.nang)) * sizeof(double);
+  const size_t smem = eclipse_smem(c);
   if constexpr (!KEEP && CellData<NMOL, NCIA>::kStaticCia) {
     if (small == 2) {
       launch_eclipse_scan<NMOL, NCIA, NANG, SQ, SC>(c, tabs, status, spectra, nmodels, use_tma, smem, s);
@@ -1348,20 +1358,69 @@ int eclipse_small_mode(const DevConfig &c, int nmodels) {
   return nslots * nmodels <= 8LL * 148 ? 1 : 0;
 }
 
-void launch_eclipse(const DevConfig &c, const double *tabs, const int *status, double *spectra,
+// Dynamic shared memory one block of `kern` can have on the current device: the opt-in limit less
+// the kernel's static shared memory (0 when either cannot be read).
+static size_t dyn_smem_max(const void *kern) {
+  int dev = 0, optin = 0;
+  cudaFuncAttributes a{};
+  if (cudaGetDevice(&dev) != cudaSuccess ||
+      cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev) != cudaSuccess ||
+      cudaFuncGetAttributes(&a, kern) != cudaSuccess) {
+    cudaGetLastError();
+    return 0;
+  }
+  return (size_t)optin > a.sharedSizeBytes ? (size_t)optin - a.sharedSizeBytes : 0;
+}
+
+// The static shared memory of a kernel family does not depend on its template arguments (the
+// eclipse kernels declare one mbarrier, the transit tile kernel its chunk barriers and flags); the
+// least room over the generic and introspection builds stands for every build.  Read once: a
+// process drives one device.
+static size_t eclipse_dyn_max() {
+  static const size_t v = std::min({dyn_smem_max((const void *)eclipse_column_kernel<0, -1, 0, true, -1, true>),
+                                    dyn_smem_max((const void *)eclipse_column_kernel<0, -1, 0, false, -1, true>),
+                                    dyn_smem_max((const void *)eclipse_slot_kernel<0, -1, 0, -1, true>)});
+  return v;
+}
+static size_t transit_tile_dyn_max() {
+  static const size_t v = std::min(dyn_smem_max((const void *)transit_tile_kernel<0, -1, true>),
+                                   dyn_smem_max((const void *)transit_tile_kernel<0, -1, false>));
+  return v;
+}
+
+bool column_smem_fits(const DevConfig &c) {
+  if (c.eclipse) return eclipse_smem(c) <= eclipse_dyn_max();
+  // transit: the DFMA tile kernel serves the introspection launches and every launch the tensor-core
+  // kernel is not chosen for (transit_uses_mma: well inside the same limit), so it has to fit
+  return tr_nchunks(c.nlayer) <= kTrMaxChunks && transit_tile_smem(c) <= transit_tile_dyn_max();
+}
+
+int column_layer_limit(const DevConfig &c) {
+  DevConfig t = c;
+  int best = 0;
+  for (int nl = 1;; nl++) {
+    t.nlayer = t.lay.nl = nl;
+    if (!column_smem_fits(t)) return best;
+    best = nl;
+  }
+}
+
+bool launch_eclipse(const DevConfig &c, const double *tabs, const int *status, double *spectra,
                     double *tau_keep, int *last_keep, int nmodels, bool keep, bool sc, int use_tma,
                     cudaStream_t s) {
+  if (!column_smem_fits(c)) return false;
   if (keep) {   // introspection path: run-time counts, stores tau[] and last[]
     launch_eclipse_t<0, -1, 0, true>(c, tabs, status, spectra, tau_keep, last_keep, nmodels, use_tma, 0, s);
-    return;
+    return true;
   }
   const int small = eclipse_small_mode(c, nmodels);
   if (c.planck_generic) {   // extreme Planck exponents: the kernel with the per-column clamp, degree 5
     launch_eclipse_t<0, -1, 0, false>(c, tabs, status, spectra, nullptr, nullptr, nmodels, use_tma, small, s);
-    return;
+    return true;
   }
   if (sc) launch_eclipse_nmol<true>(c, tabs, status, spectra, nmodels, use_tma, small, s);
   else launch_eclipse_nmol<false>(c, tabs, status, spectra, nmodels, use_tma, small, s);
+  return true;
 }
 
 void launch_merge_status(int *status, const int *status_col, int nmodels, cudaStream_t s) {
@@ -1387,7 +1446,7 @@ template <int NMOL, int NCIA, bool KEEP>
 static void launch_transit_t(const DevConfig &c, const double *tabs, const double *wts,
                              const int *status, int *status_col, double *spectra, double *tau_keep,
                              int *last_keep, int nmodels, int use_tma, cudaStream_t s) {
-  const size_t smem = table_smem(c) + ((size_t)c.nlayer * (kTrRow + kTrW) + (size_t)2 * kTrChunk * kTrW) * sizeof(double);
+  const size_t smem = transit_tile_smem(c);
   static size_t configured = 0;
   if (smem > 48 * 1024 && smem > configured) {
     cudaFuncSetAttribute(transit_tile_kernel<NMOL, NCIA, KEEP>,
@@ -1395,7 +1454,6 @@ static void launch_transit_t(const DevConfig &c, const double *tabs, const doubl
     configured = smem;
   }
   const int tiles = (c.nwave + kTrW - 1) / kTrW;
-  if (tr_nchunks(c.nlayer) > kTrMaxChunks) return;             // launch_transit checks and reports
   transit_tile_kernel<NMOL, NCIA, KEEP><<<(unsigned)((size_t)tiles * nmodels), kTrThreads, smem, s>>>(
       c, tabs, wts, status, status_col, spectra, tau_keep, last_keep, nmodels, use_tma);
 }
@@ -1449,13 +1507,14 @@ void launch_transit_weights(const DevConfig &c, const double *tabs, double *wts,
       c, tabs, wts, nmodels, transit_uses_mma(c, keep) ? 1 : 0, status_col);
 }
 
-void launch_transit(const DevConfig &c, const double *tabs, const double *wts, const int *status,
+bool launch_transit(const DevConfig &c, const double *tabs, const double *wts, const int *status,
                     int *status_col, double *spectra, double *tau_keep, int *last_keep,
                     int nmodels, bool keep, bool sc, int use_tma, cudaStream_t s) {
+  if (!column_smem_fits(c)) return false;
   g_transit_sc = sc;
   if (keep) {   // introspection path: run-time counts, stores tau[] and last[]
     launch_transit_t<0, -1, true>(c, tabs, wts, status, status_col, spectra, tau_keep, last_keep, nmodels, use_tma, s);
-    return;
+    return true;
   }
   switch (c.ngmol) {
     case 1: launch_transit_ncia<1>(c, tabs, wts, status, status_col, spectra, nmodels, use_tma, s); break;
@@ -1466,6 +1525,7 @@ void launch_transit(const DevConfig &c, const double *tabs, const double *wts, c
       if (transit_uses_mma(c, false)) launch_transit_mma_t<0, -1>(c, tabs, wts, status, status_col, spectra, nmodels, use_tma, s);
       else launch_transit_t<0, -1, false>(c, tabs, wts, status, status_col, spectra, nullptr, nullptr, nmodels, use_tma, s);
   }
+  return true;
 }
 
 void launch_extinction(const DevConfig &c, const double *tabs, double *ext, int nmodels,

@@ -17,8 +17,13 @@ constexpr int kEclPad = kEclThreads * kEclCols;
 void launch_atm_prep(const DevConfig &c, const Knobs &k, const double *profiles, int n_in,
                      double *tabs, int *status, const int *pre_status, int nmodels,
                      cudaStream_t s);
+// Whether the column kernels' shared memory (the model's table is staged whole) fits one block of
+// the current device for configuration `c`; the largest layer count that does, the other counts of
+// `c` unchanged.  launch_eclipse / launch_transit launch nothing and return false when it does not.
+bool column_smem_fits(const DevConfig &c);
+int column_layer_limit(const DevConfig &c);
 // sc: some record of the launch may carry a scattering or cloud term (false: skipped altogether)
-void launch_eclipse(const DevConfig &c, const double *tabs, const int *status, double *spectra,
+bool launch_eclipse(const DevConfig &c, const double *tabs, const int *status, double *spectra,
                     double *tau_keep, int *last_keep, int nmodels, bool keep, bool sc, int use_tma,
                     cudaStream_t s);
 // chord weights of one model in the tiled layout (doubles per model), K2t, and the tile kernel
@@ -27,7 +32,7 @@ size_t transit_weights_stride(int nlayer);
 // status_col (or nullptr): the per-model column-status words of the launch that follows, cleared here
 void launch_transit_weights(const DevConfig &c, const double *tabs, double *wts, int nmodels,
                             bool keep, int *status_col, cudaStream_t s);
-void launch_transit(const DevConfig &c, const double *tabs, const double *wts, const int *status,
+bool launch_transit(const DevConfig &c, const double *tabs, const double *wts, const int *status,
                     int *status_col, double *spectra, double *tau_keep, int *last_keep,
                     int nmodels, bool keep, bool sc, int use_tma, cudaStream_t s);
 void launch_merge_status(int *status, const int *status_col, int nmodels, cudaStream_t s);

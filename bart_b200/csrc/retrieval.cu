@@ -185,7 +185,9 @@ convert_params_kernel(ConvConfig cc, const double *__restrict__ params, int npar
   if (line)
     for (int i = threadIdx.x; i < kE2TableN; i += blockDim.x) s_e2[i] = g_e2_table[i];
   const int nl = cc.nlayer;
-  const int off = cc.npt + cc.nrad + cc.ncloud + cc.nray;
+  // either scattering model takes one parameter slot (polar, nray 2, leaves its value unused): the
+  // molecules' factors follow it (BARTfunc.py:333-338)
+  const int off = cc.npt + cc.nrad + cc.ncloud + (cc.nray ? 1 : 0);
   double *gout = profiles + (size_t)m * n_in;
   const double *press = cc.press_bar, *ratio_a = cc.ratio, *base = cc.base;
   double *out = gout;
@@ -270,7 +272,10 @@ void launch_convert_params(const ConvConfig &cc, const double *params, int npars
     double h[kE2TableN];
     for (int i = 0; i < kE2SeriesN; i++) h[i] = kE2SeriesHost[i];
     for (int i = 0; i < kE2Intervals * kE2ChebN; i++) h[kE2SeriesN + i] = kE2ChebHost[i];
-    cudaMemcpyToSymbol(g_e2_table, h, sizeof(h));
+    // on the launch stream and awaited: `h` is pageable, and the kernel below runs on `s`, which
+    // does not synchronise with the legacy stream a plain cudaMemcpyToSymbol uses
+    cudaMemcpyToSymbolAsync(g_e2_table, h, sizeof(h), 0, cudaMemcpyHostToDevice, s);
+    cudaStreamSynchronize(s);
     table_ready = true;
   }
   size_t smem = ((size_t)cc.nlayer * 3 + (size_t)cc.nspec * cc.nlayer * 2 + cc.nlayer) * sizeof(double);

@@ -220,6 +220,14 @@ static void check_launch(const char *what) {
   if (e != cudaSuccess) fail("kernel launch '%s' failed: %s", what, cudaGetErrorString(e));
 }
 
+// a layer count the column kernels cannot run (column_smem_fits): refused by transit_init
+static void fail_layer_limit() {
+  const DevConfig &c = G.dc;
+  fail("%s geometry supports at most %d layers with %d line-list molecule(s) and %d CIA table(s) "
+       "(%d given): the column kernels stage a model's table whole in the shared memory of one block",
+       c.eclipse ? "eclipse" : "transit", column_layer_limit(c), c.ngmol, c.ncia, c.nlayer);
+}
+
 // ---------------------------------------------------------------------------------------
 // device
 static void ensure_device() {
@@ -449,7 +457,6 @@ static void do_init(int argc, char **argv) {
   read_tli_header(o.linedb, G.tli);
   const int nl = G.atm.nlayer(), ns = G.atm.nspec(), nw = (int)G.wn.size();
   if (ns > kMaxSpec) fail("at most %d atmospheric species are supported", kMaxSpec);
-  if (o.solution != "eclipse" && nl > 320) fail("transit geometry supports at most 320 layers (%d given)", nl);
   // makeradsample's temperature check against the TLI range (makesample.c:488-503)
   for (int i = 0; i < nl; i++) {
     if (G.atm.temp[i] * G.atm.tfct < G.tli.tmin)
@@ -570,6 +577,7 @@ static void do_init(int argc, char **argv) {
   setup_cia();
 
   c.lay.nl = nl; c.lay.ngmol = c.ngmol; c.lay.ncia = c.ncia;
+  if (!column_smem_fits(c)) fail_layer_limit();
   G.init = true;
   info(2, "transit_init done: %d layers, %d species, %d wavenumbers, grid %ld T x %ld mol (%.1f MB "
           "in HBM), %d CIA file(s), %s geometry.\n", nl, ns, nw, G.og.ntemp, G.og.nmol,
@@ -670,7 +678,7 @@ static void launch_models(const double *d_prof, int off, int count, int total, i
                   (k.cloud_flag_all == 1 && k.cloudext_all != 0.0);
   if (c.eclipse) {
     KernelScope ks("eclipse_column");
-    launch_eclipse(c, tabs, status, d_spec, tau, last, count, G.keep, sc, G.use_tma, G.stream);
+    if (!launch_eclipse(c, tabs, status, d_spec, tau, last, count, G.keep, sc, G.use_tma, G.stream)) fail_layer_limit();
     check_launch("eclipse_column");
   } else {
     int *scol = G.d_status_col.p + off;         // cleared by the weights kernel
@@ -682,7 +690,8 @@ static void launch_models(const double *d_prof, int off, int count, int total, i
     }
     {
       KernelScope ks("transit_column");
-      launch_transit(c, tabs, wts, status, scol, d_spec, tau, last, count, G.keep, sc, G.use_tma, G.stream);
+      if (!launch_transit(c, tabs, wts, status, scol, d_spec, tau, last, count, G.keep, sc, G.use_tma, G.stream))
+        fail_layer_limit();
       check_launch("transit_column");
     }
     launch_merge_status(status, scol, count, G.stream);

@@ -30,7 +30,10 @@ extern "C" {
  * extinction line by line inside tau() (src/tau.c:163-175,253-264 -> computemolext with
  * permol = 0, src/extinction.c:281-529): same here, the TLI lines and the Voigt table are made
  * resident and every run_transit / bart_run_batch call evaluates its (model, layer) cells with
- * the builder kernels at the layers' own temperatures.                                    */
+ * the builder kernels at the layers' own temperatures.  A model's table is staged whole in
+ * the shared memory of one block, so the layer count is bounded by the device: a configuration
+ * with more layers than its geometry, molecule and CIA counts allow is refused here, with that
+ * limit in the message.                                                                   */
 void transit_init(int argc, char **argv);
 
 /* replaces get_no_samples (src/transit.c:77-80): number of spectrum wavenumbers.         */
@@ -222,8 +225,8 @@ int  bart_voigt_profile(int idop, int ilor, float *out, long long capacity, long
  * abundances[nlayer][nspecies] as read from the atmosphere file (bottom -> top).  imol: species
  * indices of the fitted molecules; imetals: every species but H2, He, H-, e-.  Parameter vector
  * layout (BARTfunc.py:176-181): [PT (npt) | radius (nrad) | cloud top (ncloud) | scattering
- * (nray: 0 none; 1 Lecavelier log-extinction; 2 polar, whose slot is unused as in BARTfunc) |
- * log10 abundance factors (nmolfit)].                                                           */
+ * (one slot unless nray is 0: 1 Lecavelier log-extinction; 2 polar, whose slot's value is unused as
+ * in BARTfunc) | log10 abundance factors (nmolfit)].                                            */
 int  bart_converter_init(int pt_type, int npt, const double *pt_args, int tint_thorngren,
                          const double *pressure_bar, const double *abundances, int nmolfit,
                          const int *imol, int nmetals, const int *imetals, int iH2, int iHe,

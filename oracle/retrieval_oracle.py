@@ -251,7 +251,9 @@ class Converter:
         self.tmin, self.tmax = tmin, tmax
         self.nrad, self.ncloud, self.nray = nrad, ncloud, nray
         self.npt = PT_NPARS[pt_type]
-        self.npars = self.npt + nrad + ncloud + nray + len(self.imol)
+        # either scattering model takes one slot (polar's value is unused, BARTfunc.py:333-338)
+        self.nscat = 1 if nray else 0
+        self.npars = self.npt + nrad + ncloud + self.nscat + len(self.imol)
 
     def temperature(self, ptpars):
         p = self.press[::-1]                                          # BARTfunc.py:176
@@ -275,7 +277,7 @@ class Converter:
         nl, ns = self.nlayer, self.nspec
         prof = np.zeros((M, (ns + 1) * nl))
         status = np.zeros(M, dtype=np.int32)
-        off = self.npt + self.nrad + self.ncloud + self.nray
+        off = self.npt + self.nrad + self.ncloud + self.nscat
         for m in range(M):
             try:
                 T = self.temperature(params[m, :self.npt])

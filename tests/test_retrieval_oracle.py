@@ -91,6 +91,57 @@ def test_converter_vs_reference(name, workdir):
         assert np.array_equal(knobs["scat_logext"], d["params"][:, c])
 
 
+def test_converter_polar_scattering_takes_one_slot(workdir):
+    """Polar scattering (nray = 2, `scattering = polar`) takes one parameter slot, like Lecavelier
+    scattering, and leaves its value unused: molecule k's factor is parameter
+    npt + nrad + ncloud + 1 + k."""
+    case, spec, extra = cases.build_retrieval("retr_small4_transit", workdir)
+    molfit = spec["molfit"]
+    conv = ro.Converter(case["press_bar"], case["species"], case["abund"], molfit, "line",
+                        pt_args=extra["pt_args"], nrad=1, ncloud=1, nray=2)
+    nPT, nradfit, ncloud, nray = 5, 1, 1, 1          # BARTfunc counts the scattering parameter once
+    nmolfit = len(molfit)
+    assert conv.npars == nPT + nradfit + ncloud + nray + nmolfit == len(spec["params"])
+    rng = np.random.default_rng(31)
+    M = 24
+    params = rng.uniform(spec["pmin"], spec["pmax"], (M, conv.npars))
+    params[:, :nPT] = np.array(spec["params"][:nPT]) + rng.normal(0, 0.05, (M, nPT))
+    params[:, -nmolfit:] = rng.uniform(-2.0, 1.0, (M, nmolfit))
+    params[::5, -2] = 4.2                             # CO: metals past 1
+    prof, status, knobs = conv.profiles(params)
+    assert (status == 0).sum() >= 12 and (status == 32).any()
+    # BARTfunc.py:333-347 on the converter's own temperatures (make_golden_retrieval.golden_converter)
+    species = np.asarray(case["species"])
+    abundances = case["abund"]
+    iH2 = np.where(species == "H2")[0]
+    iHe = np.where(species == "He")[0]
+    ratio = (abundances[:, iH2] / abundances[:, iHe]).squeeze()
+    imetals = np.where((species != "He") & (species != "H2") & (species != "H-") & (species != "e-"))[0]
+    imol = [case["species"].index(m) for m in molfit]
+    nl = len(case["press_bar"])
+    for m in np.where(status == 0)[0]:
+        par = params[m]
+        aprofiles = abundances.T.copy()
+        for i in np.arange(nmolfit):
+            mm = imol[i]
+            aprofiles[mm] = abundances[:, mm] * 10.0 ** par[nPT + nradfit + ncloud + nray + i]
+        q = 1.0 - np.sum(aprofiles[imetals], axis=0)
+        aprofiles[iH2] = ratio * q / (1.0 + ratio)
+        aprofiles[iHe] = q / (1.0 + ratio)
+        assert np.array_equal(prof[m, :nl], conv.temperature(par[:nPT]))
+        assert np.array_equal(prof[m, nl:], aprofiles.ravel())
+    assert np.array_equal(knobs["refradius"], params[:, nPT])
+    assert np.array_equal(knobs["cloudtop"], params[:, nPT + 1])
+    assert np.all(knobs["scat_flag"] == 2) and np.all(knobs["scat_logext"] == 0.0)
+    # whatever the polar slot holds, the profiles are the same bit for bit
+    for v in (-9.0, 3.0, np.nan):
+        p2 = params.copy()
+        p2[:, nPT + nradfit + ncloud] = v
+        prof2, status2, knobs2 = conv.profiles(p2)
+        assert np.array_equal(prof2, prof) and np.array_equal(status2, status)
+        assert all(np.array_equal(knobs2[k], knobs[k]) for k in knobs)
+
+
 @pytest.mark.parametrize("name", list(cases.RETRIEVAL))
 def test_demc_oracle_reproduces_reference_mc3(name, built, workdir):
     """Same seed, same model function -> the reference's chain trace bit for bit."""
