@@ -836,8 +836,12 @@ BART_HD double cell_extinction(const DevConfig &c, const ColPtrs &P, const doubl
 // consecutive columns -- the result equals the NCOL 2 form's to the bit (small-batch kernel).
 // PGEN: Planck exponent clamped per column and evaluated to degree 5 (DevConfig::planck_generic);
 // SC false: no scattering and no cloud in any record of the launch (the terms are skipped).
+// AHEAD: the grid and CIA samples of depth d + 1 are loaded during step d (the slot kernel: one warp
+// per CTA, latency-bound); false: each step loads its own depth's samples (the throughput kernel,
+// whose 20 warps per SM cover the latency; the samples are then not live across D(tau), the
+// register peak of the step, which is what fits it in 96 registers).
 template <int NMOL, int NCIA, int NANG, bool KEEP, int NCOL, int SQ = -1, bool CHAIN = false,
-          int CSTRIDE = 0, bool PGEN = true, bool SC = true>
+          int CSTRIDE = 0, bool PGEN = true, bool SC = true, bool AHEAD = true>
 BART_HD void eclipse_columns(const DevConfig &c, const double *tab, const unsigned long long *etab,
                              int w0, const bool (&valid)[NCOL],
                              double *const (&tau_keep)[NCOL], int *const (&last_keep)[NCOL],
@@ -851,7 +855,7 @@ BART_HD void eclipse_columns(const DevConfig &c, const double *tab, const unsign
   const size_t gstep = (size_t)CSTRIDE * (kStatic ? CellData<NMOL, NCIA>::NG : c.gms) * 8;
   const size_t cstep = (size_t)CSTRIDE * 32;
   double wn4[NCOL], c2n[NCOL];
-  double er1[NCOL], er2[NCOL], S[NCOL], trap[NCOL], Dprev[NCOL], Bprev[NCOL];
+  double er1[NCOL], S[NCOL], trap[NCOL], Dprev[NCOL], Bprev[NCOL];
   int last[NCOL];
   bool alive[NCOL];
   const ColPtrs P = col_ptrs<NCIA>(c, w0);
@@ -887,8 +891,7 @@ BART_HD void eclipse_columns(const DevConfig &c, const double *tab, const unsign
     wn4[k] = (wn * wn) * (wn * wn);
     c2n[k] = cH * wn * cLS / cKB * kExpScale;                  // Planck exponent x N/ln2, per 1/T
     if (CHAIN && NCOL == 1 && upper) c2n[k] = cH * c.wn[wk - CSTRIDE] * cLS / cKB * kExpScale;
-    er1[k] = cell_extinction<NMOL, NCIA, SC>(c, P, tab, wn4[k], false, k * gstep, k * cstep);
-    er2[k] = 0.0; S[k] = 0.0; trap[k] = 0.0; Dprev[k] = c.d0;
+    S[k] = 0.0; trap[k] = 0.0; Dprev[k] = c.d0;
     alive[k] = valid[k] && !(0.0 > c.toomuch);
     last[k] = alive[k] ? nl - 1 : 0;
     if (KEEP && valid[k]) tau_keep[k][0] = 0.0;
@@ -902,49 +905,72 @@ BART_HD void eclipse_columns(const DevConfig &c, const double *tab, const unsign
     return BART_WARP_ANY(a);
   };
 
-  // software pipeline: the loads of depth d + 1 are issued as soon as the data of depth d has
-  // been folded into its extinction (same registers), and complete under the fp64 work of the
-  // rest of the step; their addresses come from offsets read one step earlier still, so that no
-  // load instruction waits on a shared-memory read
-  CellData<NMOL, NCIA> cur[NCOL];
-  const double *row_last = tab + (size_t)(nl - 1) * nf;
-  auto row_after = [&](const double *r) { return r < row_last ? r + nf : r; };   // the bottom depth re-reads itself
-#pragma unroll
-  for (int k = 0; k < NCOL; k++)
-    cell_load<NMOL, NCIA>(c, P, row_after(tab), cur[k], k * gstep, k * cstep);
-  CellOffs<NCIA> offs = cell_offsets<NMOL, NCIA>(row_after(row_after(tab)));    // of depth 2
   // The CIA samples of a column depend on the depth only through the bracket row of the layer's
   // temperature in the table's (coarse) temperature grid: consecutive layers mostly share it, so
-  // cur[k].q is kept and reloaded only when the next depth's row differs (warp-uniform test)
-  CellOffs<NCIA> have = cell_offsets<NMOL, NCIA>(row_after(tab));               // what cur[k].q holds
+  // cur[k].q is kept and reloaded only when a depth's row differs from `have` (warp-uniform test)
+  CellData<NMOL, NCIA> cur[NCOL];
+  CellOffs<NCIA> have = cell_offsets<NMOL, NCIA>(tab);                          // what cur[k].q holds
+  auto fetch = [&](const CellOffs<NCIA> &o) {
+    bool fresh = false;
+#pragma unroll
+    for (int f = 0; f < (NCIA > 0 ? NCIA : 0); f++) fresh = fresh || o.cia[f] != have.cia[f];
+#pragma unroll
+    for (int k = 0; k < NCOL; k++) cell_load_at<NMOL, NCIA>(c, P, o, cur[k], k * gstep, k * cstep, fresh);
+    have = o;
+  };
+#pragma unroll
+  for (int k = 0; k < NCOL; k++) cell_load<NMOL, NCIA>(c, P, tab, cur[k], k * gstep, k * cstep);
+#pragma unroll
+  for (int k = 0; k < NCOL; k++)
+    er1[k] = cell_combine<NMOL, NCIA, SC>(c, P, tab, cur[k], wn4[k], false, k * gstep, k * cstep);
+  // AHEAD: the loads of depth d + 1 are issued as soon as the data of depth d has been folded into
+  // its extinction (same registers) and complete under the fp64 work of the rest of the step; their
+  // addresses come from offsets read one step earlier still, so that no load instruction waits on
+  // a shared-memory read.  Otherwise a step issues its own depth's loads first, ahead of the Planck
+  // function, and folds them into the extinction before D(tau).
+  const double *row_last = tab + (size_t)(nl - 1) * nf;
+  auto row_after = [&](const double *r) { return r < row_last ? r + nf : r; };   // the bottom depth re-reads itself
+  constexpr bool kLoadInStep = kStatic && !AHEAD;
+  CellOffs<NCIA> offs;
+  if (AHEAD) {
+    fetch(cell_offsets<NMOL, NCIA>(row_after(tab)));
+    offs = cell_offsets<NMOL, NCIA>(row_after(row_after(tab)));                 // of depth 2
+  }
 
   auto step = [&](const double *row, int d, bool odd) {
     double tau[NCOL], B[NCOL], D[NCOL];
     bool small[NCOL];
     double erk[NCOL];
+    if (kLoadInStep) {
+      fetch(cell_offsets<NMOL, NCIA>(row));
+      planck(row, B);
+    }
 #pragma unroll
     for (int k = 0; k < NCOL; k++) {
       erk[k] = cell_combine<NMOL, NCIA, SC>(c, P, row, cur[k], wn4[k], false, k * gstep, k * cstep);
     }
-    bool fresh = false;
-#pragma unroll
-    for (int f = 0; f < (NCIA > 0 ? NCIA : 0); f++) fresh = fresh || offs.cia[f] != have.cia[f];
-#pragma unroll
-    for (int k = 0; k < NCOL; k++) cell_load_at<NMOL, NCIA>(c, P, offs, cur[k], k * gstep, k * cstep, fresh);
-    if (kStatic) { have = offs; offs = cell_offsets<NMOL, NCIA>(row_after(row_after(row))); }
+    if (AHEAD && kStatic) {
+      fetch(offs);
+      offs = cell_offsets<NMOL, NCIA>(row_after(row_after(row)));
+    }
 #pragma unroll
     for (int k = 0; k < NCOL; k++) {
       const double er = erk[k];
-      if (odd) tau[k] = fma(row[L::TR], er + er1[k], S[k]);
-      else {
-        const D2 s1 = ld2(row + L::SA);                        // (SA, SB)
-        S[k] = fma(s1.x, er, fma(s1.y, er1[k], fma(row[L::SC], er2[k], S[k])));
+      if (odd) {
+        tau[k] = fma(row[L::TR], er + er1[k], S[k]);
+        // the panel that ends at depth d + 1 takes its terms of depths d - 1 and d now:
+        // S(d+1) = SA er(d+1) + (SB er(d) + (SC er(d-1) + S(d-1))), so no er is carried
+        // across the rest of this step
+        const double *nx = row_after(row);
+        S[k] = fma(nx[L::SB], er, fma(nx[L::SC], er1[k], S[k]));
+      } else {
+        S[k] = fma(row[L::SA], er, S[k]);
         tau[k] = S[k];
+        er1[k] = er;
       }
-      er2[k] = er1[k]; er1[k] = er;
       small[k] = !alive[k] || hi_word(tau[k]) < small_hi;
     }
-    planck(row, B);
+    if (!kLoadInStep) planck(row, B);
     // D(tau): the low-tau polynomial while every live column of a slot (32 consecutive columns: the
     // warp's k-th) is below tau_small, weighted exponentials otherwise
     auto series = [&](int k0, int k1) {

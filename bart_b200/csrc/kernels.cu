@@ -20,6 +20,7 @@
 #include <cstring>
 #include <cstdlib>
 #include <algorithm>
+#include <type_traits>
 
 namespace bart {
 
@@ -212,13 +213,19 @@ atm_prep_kernel(DevConfig c, Knobs knobs, const double *__restrict__ profiles, i
 
 // ---------------------------------------------------------------------------------------
 // fused eclipse column kernel
-// 128 registers, 8 CTAs (16 warps) per SM.  Measured alternatives (W12, 4096 models): 112 registers /
-// 18 warps 4.43 ms (spills go through the L1 data pipe, the busiest unit), 144 registers / 14 warps
-// 5.07 ms, against 4.07 ms.  One column per thread (the slot kernel's arithmetic) in CTAs of 128 threads
-// at 72 registers, 28 warps per SM: 4.30 against 4.12 ms -- the depth's table record is then read per
-// column and the Planck chaining is lost; the kernel is bound by its pipes, not by latency.
-template <int NMOL, int NCIA, int NANG, bool KEEP, int SQ, bool SC>
-__global__ void __launch_bounds__(kEclThreads, 8)
+// Specialised builds with at most one CIA file: 96 registers, 10 CTAs (20 warps) per SM, no spills --
+// each depth step loads its own grid and CIA samples (eclipse_columns with AHEAD false), so they are not
+// live across D(tau).  W12, 4096 models, B200 at 1000 W (profiles/r03_eclipse_column_variants.json):
+// 3.77 ms against 4.12 ms for the former one-depth-ahead prefetch at 128 registers / 16 warps (12 bytes
+// spilled).  Measured alternatives: the same in-step loads at 128 registers / 16 warps 3.94 ms; the lo
+// plane one depth ahead at 96 registers 4.03 ms and the loads issued at the end of the previous step
+// 4.06 ms (both spill 8 bytes).  Before that: 112 registers / 18 warps 4.43 ms (spills go through the
+// L1 data pipe, the busiest unit), 144 registers / 14 warps 5.07 ms.  Two CIA files, the run-time-count
+// and the introspection builds keep 8 CTAs (the two-CIA builds spill at 96).  One column per thread (the slot kernel's
+// arithmetic) in CTAs of 128 threads at 72 registers, 28 warps per SM: 4.30 against 4.12 ms -- the
+// depth's table record is then read per column and the Planck chaining is lost.
+template <int NMOL, int NCIA, int NANG, bool KEEP, int SQ, bool SC, bool AHEAD>
+__global__ void __launch_bounds__(kEclThreads, CellData<NMOL, NCIA>::kStaticCia && NCIA <= 1 && !KEEP && !AHEAD ? 10 : 8)
 eclipse_column_kernel(DevConfig c, const double *__restrict__ tabs, const int *__restrict__ status,
                       double *__restrict__ spectra, double *__restrict__ tau_keep,
                       int *__restrict__ last_keep, int nmodels, int use_tma) {
@@ -258,8 +265,8 @@ eclipse_column_kernel(DevConfig c, const double *__restrict__ tabs, const int *_
   // the specialised instantiations leave the Planck-exponent clamp out and evaluate the Planck
   // exponential to degree 4 (launch_eclipse routes configurations that need more to the
   // run-time-count kernel)
-  eclipse_columns<NMOL, NCIA, NANG, KEEP, kEclCols, SQ, true, kEclThreads, NMOL == 0, SC>(c, s_tab, s_etab, w0,
-                                                                                         valid, tk, lk, flux);
+  eclipse_columns<NMOL, NCIA, NANG, KEEP, kEclCols, SQ, true, kEclThreads, NMOL == 0, SC, AHEAD>(
+      c, s_tab, s_etab, w0, valid, tk, lk, flux);
 #pragma unroll
   for (int k = 0; k < kEclCols; k++)
     if (valid[k]) out[w0 + k * kEclThreads] = flux[k];
@@ -1294,17 +1301,28 @@ static void launch_eclipse_t(const DevConfig &c, const double *tabs, const int *
         c, tabs, status, spectra, nmodels, use_tma);
     return;
   }
-  static size_t configured = 0;
-  if (smem > 48 * 1024 && smem > configured) {
-    cudaFuncSetAttribute(eclipse_column_kernel<NMOL, NCIA, NANG, KEEP, SQ, SC>,
-                         cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    configured = smem;
-  }
   const int per = kEclThreads * kEclCols;
   const int tiles = (c.nwave + per - 1) / per;
-  eclipse_column_kernel<NMOL, NCIA, NANG, KEEP, SQ, SC>
-      <<<(unsigned)((size_t)tiles * nmodels), kEclThreads, smem, s>>>(
-          c, tabs, status, spectra, tau_keep, last_keep, nmodels, use_tma);
+  // Up to one resident wave of 8 CTAs per SM the kernel is latency-bound and the form that loads
+  // one depth ahead is faster (W12, 24 models: 66 against 85 us); beyond, the in-step loads and
+  // their 10 CTAs per SM are (4096 models: 3.77 against 4.12 ms).  Both give the same spectra to the bit.
+  auto launch = [&](auto ahead) {                   // one instantiation (and `configured`) per form
+    const auto kern = eclipse_column_kernel<NMOL, NCIA, NANG, KEEP, SQ, SC, decltype(ahead)::value>;
+    static size_t configured = 0;
+    if (smem > 48 * 1024 && smem > configured) {
+      cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+      configured = smem;
+    }
+    kern<<<(unsigned)((size_t)tiles * nmodels), kEclThreads, smem, s>>>(c, tabs, status, spectra, tau_keep,
+                                                                       last_keep, nmodels, use_tma);
+  };
+  if constexpr (CellData<NMOL, NCIA>::kStatic) {
+    if ((long long)tiles * nmodels <= 8LL * 148) {
+      launch(std::true_type());
+      return;
+    }
+  }
+  launch(std::false_type());
 }
 
 // Specialised instantiations for the shapes BART runs (1-4 line-list molecules, 0-2 CIA files, the
@@ -1377,8 +1395,8 @@ static size_t dyn_smem_max(const void *kern) {
 // least room over the generic and introspection builds stands for every build.  Read once: a
 // process drives one device.
 static size_t eclipse_dyn_max() {
-  static const size_t v = std::min({dyn_smem_max((const void *)eclipse_column_kernel<0, -1, 0, true, -1, true>),
-                                    dyn_smem_max((const void *)eclipse_column_kernel<0, -1, 0, false, -1, true>),
+  static const size_t v = std::min({dyn_smem_max((const void *)eclipse_column_kernel<0, -1, 0, true, -1, true, false>),
+                                    dyn_smem_max((const void *)eclipse_column_kernel<0, -1, 0, false, -1, true, false>),
                                     dyn_smem_max((const void *)eclipse_slot_kernel<0, -1, 0, -1, true>)});
   return v;
 }
