@@ -16,6 +16,7 @@
 // Tensor cores are not used: nothing here is a dense contraction (4 flop per 16 B).
 #include "column_math.cuh"
 #include "kernels.hpp"
+#include "dyn_smem.hpp"
 #include <cuda_runtime.h>
 #include <cstring>
 #include <cstdlib>
@@ -1234,6 +1235,36 @@ static size_t transit_tile_smem(const DevConfig &c) {     // the DFMA tile kerne
   return table_smem(c) + ((size_t)c.nlayer * (kTrRow + kTrW) + (size_t)2 * kTrChunk * kTrW) * sizeof(double);
 }
 
+// Specialised instantiations for the shapes BART runs: f(nmol, ncia) with the grid-molecule and CIA
+// counts as std::integral_constant, (1..4, 0..2) when both are in range, else the run-time-count
+// build (0, -1).  dispatch_nmol is the molecule half: 1..4, else 0.
+template <class F>
+static void dispatch_nmol(int ngmol, F &&f) {
+  switch (ngmol) {
+    case 1: f(std::integral_constant<int, 1>()); break;
+    case 2: f(std::integral_constant<int, 2>()); break;
+    case 3: f(std::integral_constant<int, 3>()); break;
+    case 4: f(std::integral_constant<int, 4>()); break;
+    default: f(std::integral_constant<int, 0>());
+  }
+}
+template <class F>
+static void dispatch_counts(const DevConfig &c, F &&f) {
+  dispatch_nmol(c.ngmol, [&](auto nmol) {
+    const auto generic = [&] { f(std::integral_constant<int, 0>(), std::integral_constant<int, -1>()); };
+    if constexpr (decltype(nmol)::value == 0) {
+      generic();
+    } else {
+      switch (c.ncia) {
+        case 0: f(nmol, std::integral_constant<int, 0>()); break;
+        case 1: f(nmol, std::integral_constant<int, 1>()); break;
+        case 2: f(nmol, std::integral_constant<int, 2>()); break;
+        default: generic();
+      }
+    }
+  });
+}
+
 void launch_grid_relayout(const double *in, double *out, int ncells, int nmol, int gms, int nwave,
                           cudaStream_t s) {
   grid_relayout_kernel<<<148 * 8, 256, 0, s>>>(in, out, ncells, nmol, gms, nwave);
@@ -1246,12 +1277,7 @@ void launch_atm_prep(const DevConfig &c, const Knobs &k, const double *profiles,
   size_t smem = atm_prep_smem_doubles(c) * sizeof(double);
   const int staged = smem <= 160 * 1024;
   if (!staged) smem = ((size_t)c.nspec + 3) * c.nlayer * sizeof(double);
-  static size_t configured = 0;
-  if (smem > 48 * 1024 && smem > configured) {
-    if (cudaFuncSetAttribute(atm_prep_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess)
-      return;                                    // surfaces as the launch error of the call below
-    configured = smem;
-  }
+  if (!allow_dyn_smem<atm_prep_kernel>(smem)) return;
   atm_prep_kernel<<<nmodels, kPrepThreads, smem, s>>>(c, k, profiles, n_in, tabs, status, pre_status, nmodels, staged);
 }
 
@@ -1260,12 +1286,7 @@ void launch_atm_prep(const DevConfig &c, const Knobs &k, const double *profiles,
 template <int NMOL, int NCIA, int NANG, int SQ, bool SC>
 static void launch_eclipse_scan(const DevConfig &c, const double *tabs, const int *status, double *spectra,
                                 int nmodels, int use_tma, size_t smem, cudaStream_t s) {
-  static size_t configured = 0;
-  if (smem > 48 * 1024 && smem > configured) {
-    cudaFuncSetAttribute(eclipse_scan_kernel<NMOL, NCIA, NANG, SQ, SC>,
-                         cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    configured = smem;
-  }
+  if (!allow_dyn_smem<eclipse_scan_kernel<NMOL, NCIA, NANG, SQ, SC>>(smem)) return;
   // about one resident wave of warp tasks (4 columns each): 148 SMs x 6 CTAs x 4 warps
   constexpr int kWarps = kScanThreads / 32;
   const long long tasks = ((long long)(c.nwave + kScanCols - 1) / kScanCols) * nmodels;
@@ -1290,12 +1311,7 @@ static void launch_eclipse_t(const DevConfig &c, const double *tabs, const int *
     }
   }
   if (small && !KEEP) {
-    static size_t configured_s = 0;
-    if (smem > 48 * 1024 && smem > configured_s) {
-      cudaFuncSetAttribute(eclipse_slot_kernel<NMOL, NCIA, NANG, SQ, SC>,
-                           cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-      configured_s = smem;
-    }
+    if (!allow_dyn_smem<eclipse_slot_kernel<NMOL, NCIA, NANG, SQ, SC>>(smem)) return;
     const int nslots = (c.nwave + 31) / 32;
     eclipse_slot_kernel<NMOL, NCIA, NANG, SQ, SC><<<(unsigned)((size_t)nslots * nmodels), 32, smem, s>>>(
         c, tabs, status, spectra, nmodels, use_tma);
@@ -1306,13 +1322,9 @@ static void launch_eclipse_t(const DevConfig &c, const double *tabs, const int *
   // Up to one resident wave of 8 CTAs per SM the kernel is latency-bound and the form that loads
   // one depth ahead is faster (W12, 24 models: 66 against 85 us); beyond, the in-step loads and
   // their 10 CTAs per SM are (4096 models: 3.77 against 4.12 ms).  Both give the same spectra to the bit.
-  auto launch = [&](auto ahead) {                   // one instantiation (and `configured`) per form
-    const auto kern = eclipse_column_kernel<NMOL, NCIA, NANG, KEEP, SQ, SC, decltype(ahead)::value>;
-    static size_t configured = 0;
-    if (smem > 48 * 1024 && smem > configured) {
-      cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-      configured = smem;
-    }
+  auto launch = [&](auto ahead) {                   // one instantiation per form
+    constexpr auto kern = eclipse_column_kernel<NMOL, NCIA, NANG, KEEP, SQ, SC, decltype(ahead)::value>;
+    if (!allow_dyn_smem<kern>(smem)) return;
     kern<<<(unsigned)((size_t)tiles * nmodels), kEclThreads, smem, s>>>(c, tabs, status, spectra, tau_keep,
                                                                        last_keep, nmodels, use_tma);
   };
@@ -1325,9 +1337,8 @@ static void launch_eclipse_t(const DevConfig &c, const double *tabs, const int *
   launch(std::false_type());
 }
 
-// Specialised instantiations for the shapes BART runs (1-4 line-list molecules, 0-2 CIA files, the
-// default 5-angle ray grid, with or without scattering / cloud terms); anything else takes the
-// run-time-count kernel.
+// The specialised eclipse builds take the default 5-angle ray grid as a compile-time count as well
+// (with or without scattering / cloud terms); any other grid takes the run-time angle count.
 template <int NMOL, int NCIA, bool SC>
 static void launch_eclipse_nang(const DevConfig &c, const double *tabs, const int *status,
                                 double *spectra, int nmodels, int use_tma, int small, cudaStream_t s) {
@@ -1335,29 +1346,6 @@ static void launch_eclipse_nang(const DevConfig &c, const double *tabs, const in
   if (c.nang == 5 && c.sq_src == 0 && c.sq_dst == 3)
     launch_eclipse_t<NMOL, NCIA, 5, false, 0x03, SC>(c, tabs, status, spectra, nullptr, nullptr, nmodels, use_tma, small, s);
   else launch_eclipse_t<NMOL, NCIA, 0, false, -1, SC>(c, tabs, status, spectra, nullptr, nullptr, nmodels, use_tma, small, s);
-}
-
-template <int NMOL, bool SC>
-static void launch_eclipse_ncia(const DevConfig &c, const double *tabs, const int *status,
-                                double *spectra, int nmodels, int use_tma, int small, cudaStream_t s) {
-  switch (c.ncia) {
-    case 0: launch_eclipse_nang<NMOL, 0, SC>(c, tabs, status, spectra, nmodels, use_tma, small, s); break;
-    case 1: launch_eclipse_nang<NMOL, 1, SC>(c, tabs, status, spectra, nmodels, use_tma, small, s); break;
-    case 2: launch_eclipse_nang<NMOL, 2, SC>(c, tabs, status, spectra, nmodels, use_tma, small, s); break;
-    default: launch_eclipse_t<0, -1, 0, false>(c, tabs, status, spectra, nullptr, nullptr, nmodels, use_tma, small, s);
-  }
-}
-
-template <bool SC>
-static void launch_eclipse_nmol(const DevConfig &c, const double *tabs, const int *status,
-                                double *spectra, int nmodels, int use_tma, int small, cudaStream_t s) {
-  switch (c.ngmol) {
-    case 1: launch_eclipse_ncia<1, SC>(c, tabs, status, spectra, nmodels, use_tma, small, s); break;
-    case 2: launch_eclipse_ncia<2, SC>(c, tabs, status, spectra, nmodels, use_tma, small, s); break;
-    case 3: launch_eclipse_ncia<3, SC>(c, tabs, status, spectra, nmodels, use_tma, small, s); break;
-    case 4: launch_eclipse_ncia<4, SC>(c, tabs, status, spectra, nmodels, use_tma, small, s); break;
-    default: launch_eclipse_t<0, -1, 0, false>(c, tabs, status, spectra, nullptr, nullptr, nmodels, use_tma, small, s);
-  }
 }
 
 // Which eclipse kernel a batch of `nmodels` takes: 0 = throughput kernel (two columns per thread),
@@ -1436,8 +1424,13 @@ bool launch_eclipse(const DevConfig &c, const double *tabs, const int *status, d
     launch_eclipse_t<0, -1, 0, false>(c, tabs, status, spectra, nullptr, nullptr, nmodels, use_tma, small, s);
     return true;
   }
-  if (sc) launch_eclipse_nmol<true>(c, tabs, status, spectra, nmodels, use_tma, small, s);
-  else launch_eclipse_nmol<false>(c, tabs, status, spectra, nmodels, use_tma, small, s);
+  dispatch_counts(c, [&](auto nmol, auto ncia) {
+    constexpr int NMOL = decltype(nmol)::value, NCIA = decltype(ncia)::value;
+    if constexpr (NCIA < 0)   // the run-time-count build always has the scattering / cloud terms
+      launch_eclipse_t<0, -1, 0, false>(c, tabs, status, spectra, nullptr, nullptr, nmodels, use_tma, small, s);
+    else if (sc) launch_eclipse_nang<NMOL, NCIA, true>(c, tabs, status, spectra, nmodels, use_tma, small, s);
+    else launch_eclipse_nang<NMOL, NCIA, false>(c, tabs, status, spectra, nmodels, use_tma, small, s);
+  });
   return true;
 }
 
@@ -1461,62 +1454,25 @@ bool transit_uses_mma(const DevConfig &c, bool keep) {
 }
 
 template <int NMOL, int NCIA, bool KEEP>
-static void launch_transit_t(const DevConfig &c, const double *tabs, const double *wts,
-                             const int *status, int *status_col, double *spectra, double *tau_keep,
-                             int *last_keep, int nmodels, int use_tma, cudaStream_t s) {
+static void launch_transit_tile(const DevConfig &c, const double *tabs, const double *wts,
+                                const int *status, int *status_col, double *spectra, double *tau_keep,
+                                int *last_keep, int nmodels, int use_tma, cudaStream_t s) {
   const size_t smem = transit_tile_smem(c);
-  static size_t configured = 0;
-  if (smem > 48 * 1024 && smem > configured) {
-    cudaFuncSetAttribute(transit_tile_kernel<NMOL, NCIA, KEEP>,
-                         cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    configured = smem;
-  }
+  if (!allow_dyn_smem<transit_tile_kernel<NMOL, NCIA, KEEP>>(smem)) return;
   const int tiles = (c.nwave + kTrW - 1) / kTrW;
   transit_tile_kernel<NMOL, NCIA, KEEP><<<(unsigned)((size_t)tiles * nmodels), kTrThreads, smem, s>>>(
       c, tabs, wts, status, status_col, spectra, tau_keep, last_keep, nmodels, use_tma);
 }
 
 template <int NMOL, int NCIA, bool SC>
-static void launch_transit_mma_sc(const DevConfig &c, const double *tabs, const double *wts,
-                                  const int *status, int *status_col, double *spectra, int nmodels,
-                                  int use_tma, cudaStream_t s) {
+static void launch_transit_mma(const DevConfig &c, const double *tabs, const double *wts,
+                               const int *status, int *status_col, double *spectra, int nmodels,
+                               int use_tma, cudaStream_t s) {
   const size_t smem = transit_mma_smem(c);
-  static size_t configured = 0;
-  if (smem > 48 * 1024 && smem > configured) {
-    cudaFuncSetAttribute(transit_mma_kernel<NMOL, NCIA, false, SC>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    configured = smem;
-  }
+  if (!allow_dyn_smem<transit_mma_kernel<NMOL, NCIA, false, SC>>(smem)) return;
   const int tiles = (c.nwave + kMmW - 1) / kMmW;
   transit_mma_kernel<NMOL, NCIA, false, SC><<<(unsigned)((size_t)tiles * nmodels), kMmThreads, smem, s>>>(
       c, tabs, wts, status, status_col, spectra, nullptr, nullptr, nmodels, use_tma);
-}
-static bool g_transit_sc = true;       // set by launch_transit for the launch in progress
-template <int NMOL, int NCIA>
-static void launch_transit_mma_t(const DevConfig &c, const double *tabs, const double *wts,
-                                 const int *status, int *status_col, double *spectra, int nmodels,
-                                 int use_tma, cudaStream_t s) {
-  if (g_transit_sc) launch_transit_mma_sc<NMOL, NCIA, true>(c, tabs, wts, status, status_col, spectra, nmodels, use_tma, s);
-  else launch_transit_mma_sc<NMOL, NCIA, false>(c, tabs, wts, status, status_col, spectra, nmodels, use_tma, s);
-}
-
-template <int NMOL>
-static void launch_transit_ncia(const DevConfig &c, const double *tabs, const double *wts,
-                                const int *status, int *status_col, double *spectra, int nmodels,
-                                int use_tma, cudaStream_t s) {
-  if (transit_uses_mma(c, false)) {
-    switch (c.ncia) {
-      case 0: launch_transit_mma_t<NMOL, 0>(c, tabs, wts, status, status_col, spectra, nmodels, use_tma, s); return;
-      case 1: launch_transit_mma_t<NMOL, 1>(c, tabs, wts, status, status_col, spectra, nmodels, use_tma, s); return;
-      case 2: launch_transit_mma_t<NMOL, 2>(c, tabs, wts, status, status_col, spectra, nmodels, use_tma, s); return;
-      default: launch_transit_mma_t<0, -1>(c, tabs, wts, status, status_col, spectra, nmodels, use_tma, s); return;
-    }
-  }
-  switch (c.ncia) {
-    case 0: launch_transit_t<NMOL, 0, false>(c, tabs, wts, status, status_col, spectra, nullptr, nullptr, nmodels, use_tma, s); break;
-    case 1: launch_transit_t<NMOL, 1, false>(c, tabs, wts, status, status_col, spectra, nullptr, nullptr, nmodels, use_tma, s); break;
-    case 2: launch_transit_t<NMOL, 2, false>(c, tabs, wts, status, status_col, spectra, nullptr, nullptr, nmodels, use_tma, s); break;
-    default: launch_transit_t<0, -1, false>(c, tabs, wts, status, status_col, spectra, nullptr, nullptr, nmodels, use_tma, s);
-  }
 }
 
 void launch_transit_weights(const DevConfig &c, const double *tabs, double *wts, int nmodels,
@@ -1529,20 +1485,18 @@ bool launch_transit(const DevConfig &c, const double *tabs, const double *wts, c
                     int *status_col, double *spectra, double *tau_keep, int *last_keep,
                     int nmodels, bool keep, bool sc, int use_tma, cudaStream_t s) {
   if (!column_smem_fits(c)) return false;
-  g_transit_sc = sc;
   if (keep) {   // introspection path: run-time counts, stores tau[] and last[]
-    launch_transit_t<0, -1, true>(c, tabs, wts, status, status_col, spectra, tau_keep, last_keep, nmodels, use_tma, s);
+    launch_transit_tile<0, -1, true>(c, tabs, wts, status, status_col, spectra, tau_keep, last_keep, nmodels, use_tma, s);
     return true;
   }
-  switch (c.ngmol) {
-    case 1: launch_transit_ncia<1>(c, tabs, wts, status, status_col, spectra, nmodels, use_tma, s); break;
-    case 2: launch_transit_ncia<2>(c, tabs, wts, status, status_col, spectra, nmodels, use_tma, s); break;
-    case 3: launch_transit_ncia<3>(c, tabs, wts, status, status_col, spectra, nmodels, use_tma, s); break;
-    case 4: launch_transit_ncia<4>(c, tabs, wts, status, status_col, spectra, nmodels, use_tma, s); break;
-    default:
-      if (transit_uses_mma(c, false)) launch_transit_mma_t<0, -1>(c, tabs, wts, status, status_col, spectra, nmodels, use_tma, s);
-      else launch_transit_t<0, -1, false>(c, tabs, wts, status, status_col, spectra, nullptr, nullptr, nmodels, use_tma, s);
-  }
+  const bool mma = transit_uses_mma(c, false);
+  dispatch_counts(c, [&](auto nmol, auto ncia) {
+    constexpr int NMOL = decltype(nmol)::value, NCIA = decltype(ncia)::value;
+    if (!mma)
+      launch_transit_tile<NMOL, NCIA, false>(c, tabs, wts, status, status_col, spectra, nullptr, nullptr, nmodels, use_tma, s);
+    else if (sc) launch_transit_mma<NMOL, NCIA, true>(c, tabs, wts, status, status_col, spectra, nmodels, use_tma, s);
+    else launch_transit_mma<NMOL, NCIA, false>(c, tabs, wts, status, status_col, spectra, nmodels, use_tma, s);
+  });
   return true;
 }
 
@@ -1551,18 +1505,11 @@ void launch_extinction(const DevConfig &c, const double *tabs, double *ext, int 
   const size_t smem = (size_t)c.lay.stride() * sizeof(double);
   const int tiles = (c.nwave + kColThreads - 1) / kColThreads;
   dim3 grid((unsigned)((size_t)tiles * nmodels), (unsigned)layer_splits);
-  auto go = [&](auto kern) {
-    if (smem > 48 * 1024)
-      cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  dispatch_nmol(c.ngmol, [&](auto nmol) {
+    constexpr auto kern = extinction_kernel<decltype(nmol)::value>;
+    if (!allow_dyn_smem<kern>(smem)) return;
     kern<<<grid, kColThreads, smem, s>>>(c, tabs, ext, nmodels, mol_only, use_tma);
-  };
-  switch (c.ngmol) {
-    case 1: go(extinction_kernel<1>); break;
-    case 2: go(extinction_kernel<2>); break;
-    case 3: go(extinction_kernel<3>); break;
-    case 4: go(extinction_kernel<4>); break;
-    default: go(extinction_kernel<0>);
-  }
+  });
 }
 
 void launch_band_integrate(const double *spectra, const double *wn, const int *fstart,

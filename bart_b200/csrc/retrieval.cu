@@ -19,6 +19,7 @@
 // These are latency-bound kernels over [nchains x npars] doubles: no roofline claim; they exist so
 // that the per-generation host round trip (MPI scatter/gather in the reference) disappears.
 #include "retrieval.hpp"
+#include "dyn_smem.hpp"
 #include <cmath>
 
 namespace bart {
@@ -281,12 +282,7 @@ void launch_convert_params(const ConvConfig &cc, const double *params, int npars
   size_t smem = ((size_t)cc.nlayer * 3 + (size_t)cc.nspec * cc.nlayer * 2 + cc.nlayer) * sizeof(double);
   const int staged = smem <= 96 * 1024;
   if (!staged) smem = (size_t)cc.nlayer * sizeof(double);
-  static size_t configured = 0;
-  if (smem > 48 * 1024 && smem > configured) {
-    if (cudaFuncSetAttribute(convert_params_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess)
-      return;                                   // surfaces as the launch error of the call below
-    configured = smem;
-  }
+  if (!allow_dyn_smem<convert_params_kernel>(smem)) return;
   convert_params_kernel<<<nmodels, kConvThreads, smem, s>>>(cc, params, npars, profiles, n_in, status, kn, nmodels, staged);
 }
 
