@@ -311,8 +311,11 @@ def make_case(workdir, shape="demo", solution="eclipse", seed=12345, nlayer=100,
               nlines=0, wnosamp=2160, extra_cfg=None, nfilters=None, overrides=None,
               cia_path=None, starrad=1.155, refpress=0.1, gsurf=1165.02,
               refradius_km=123820.0, ethresh=1e-6, nwidth=20, outputs=False, verb=0,
-              no_opacity=False, cia_h2he=False, atm_path=None, mol_path=None):
-    """Create every input file of one configuration under `workdir`; returns paths + arrays."""
+              no_opacity=False, cia_h2he=False, atm_path=None, mol_path=None, species=None,
+              abund=None):
+    """Create every input file of one configuration under `workdir`; returns paths + arrays.
+    `species` / `abund`: the atmosphere's species and their uniform abundances (default SPECIES /
+    UNIFORM); every grid molecule of the shape must be one of the species."""
     os.makedirs(workdir, exist_ok=True)
     sh = dict(SHAPES[shape]) if isinstance(shape, str) else dict(shape)
     if overrides:
@@ -321,9 +324,10 @@ def make_case(workdir, shape="demo", solution="eclipse", seed=12345, nlayer=100,
     wn = wn_grid(sh["wnlow"], sh["wnhigh"], sh["wndelt"])
     press = pressure_grid(nlayer)
     temp = temperature_profile(press)
-    abund = np.array(UNIFORM)
+    species = list(SPECIES if species is None else species)
+    abund = np.array(UNIFORM if abund is None else abund, dtype=float)
     case = dict(workdir=workdir, shape=sh, wn=wn, press_bar=press, temp=temp,
-                abund=np.tile(abund, (nlayer, 1)), species=list(SPECIES), solution=solution,
+                abund=np.tile(abund, (nlayer, 1)), species=species, solution=solution,
                 nlayer=nlayer)
     case["molfile"] = mol_path or write_molecules(P("molecules.dat"))
     if atm_path:          # an existing atmosphere file (e.g. the reference's shipped demo atmosphere)
@@ -331,7 +335,7 @@ def make_case(workdir, shape="demo", solution="eclipse", seed=12345, nlayer=100,
         nlayer = len(press)
         case.update(press_bar=press, temp=temp, abund=ab, species=list(sp), nlayer=nlayer, atm=atm_path)
     else:
-        case["atm"] = write_atm(P("atm.dat"), press, temp, abund, gsurf=gsurf,
+        case["atm"] = write_atm(P("atm.dat"), press, temp, abund, species=species, gsurf=gsurf,
                                 r0_km=refradius_km * 0.97)
     if with_cia:
         case["cia"] = cia_path or write_cia(P("CIA_H2H2_synth.dat"))
@@ -353,7 +357,8 @@ def make_case(workdir, shape="demo", solution="eclipse", seed=12345, nlayer=100,
     iso_table = {"CH4": [("61", 16.0313, 0.98827), ("62", 17.03466, 0.0111031)],
                  "H2O": [("161", 18.010565, 0.997317), ("181", 20.014811, 0.00199983)],
                  "CO2": [("626", 43.98983, 0.98420)],
-                 "CO": [("26", 27.994915, 0.98654), ("36", 28.99827, 0.01108)]}
+                 "CO": [("26", 27.994915, 0.98654), ("36", 28.99827, 0.01108)],
+                 "NH3": [("4111", 17.026549, 0.995872)]}
     for m in sh["mols"]:
         dbs.append(("HITRAN " + m, m, iso_table[m]))
     case["tli"] = P("lines.tli")

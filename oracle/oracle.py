@@ -285,10 +285,30 @@ class Oracle:
     def set_scattering(self, flag, logext):
         self.c.scat_flag, self.c.scat_logext = flag, logext
 
+    def status(self, model):
+        """The rejection code (REJ_TGRID 1, REJ_TCIA 2, as bart_b200.api names them) of a model whose
+        layer temperatures leave the opacity grid's or a CIA table's range, where the reference
+        exits (extinction.c:534-581, crosssec.c:293-309); 0 otherwise."""
+        T = np.asarray(model, dtype=np.float64)[:self.c.nlayer]
+        st = 0
+        if self.lbl is None and ((T < self.gtemp[0]).any() or (T > self.gtemp[-1]).any()):
+            st |= 1
+        for t in self.cia:
+            if (T < t["temps"][0]).any() or (T > t["temps"][-1]).any():
+                st |= 2
+        return st
+
     def run(self, model, inter=False):
+        """The spectrum of one model (with inter: a dict of the intermediate arrays, its "status"
+        and "spectrum").  A model the reference would exit on (status() != 0) is not computed:
+        its spectrum is -1, as the product reports a rejected model."""
         model = np.ascontiguousarray(model, dtype=np.float64)
         nl, nw, ns = self.c.nlayer, self.c.nwave, self.c.nspec
         spec = np.zeros(nw)
+        st = self.status(model)
+        if st:
+            spec[:] = -1.0
+            return dict(status=st, spectrum=spec) if inter else spec
         if not inter:
             self._forward(model, spec, None)
             return spec
@@ -304,7 +324,7 @@ class Oracle:
             out["intens"] = np.zeros((self.c.nangle, nw))
             it.intens = _d(out["intens"])
         self._forward(model, spec, C.byref(it))
-        out["spectrum"] = spec
+        out["spectrum"], out["status"] = spec, 0
         return out
 
     def _forward(self, model, spec, it):

@@ -665,7 +665,7 @@ class BandOracle:
         prof, status, knobs = self.conv.profiles(params)
         out = -np.ones((params.shape[0], self.nfilters))
         for m in range(params.shape[0]):
-            if status[m]:
+            if status[m] or self.O.status(prof[m]):      # rejected: -1 band fluxes, as the product
                 continue
             if "refradius" in knobs:
                 self.O.set_radius(knobs["refradius"][m])

@@ -26,6 +26,10 @@ void warn(int, const char *, ...) {}
 
 using namespace bart;
 
+// the throughput kernel's thread shape (kernels.hpp kEclThreads, kEclCols): a thread carries two
+// columns kEclThreads apart, and the grid and the CIA tables are padded by kEclPad samples
+constexpr int kThreads = 64, kCols = 2, kPad = kThreads * kCols;
+
 struct Emu {
   Options opt; Atmosphere atm; Molecules mol; Tli tli; OpacityGrid og;
   std::vector<CiaTable> cia;
@@ -72,7 +76,7 @@ int emu_init(const char *cfg) {
     }
     // the device layout of the grid: [layer][temp][wave][gms] (device.cuh)
     c.gms = g.nmol == 1 ? 1 : (int)((g.nmol + 1) / 2 * 2);
-    E->grid.assign((size_t)g.nlayer * g.ntemp * g.nwave * c.gms, 0.0);
+    E->grid.assign((size_t)g.nlayer * g.ntemp * g.nwave * c.gms + (size_t)kPad * c.gms, 0.0);
     c.lbl = E->lbl ? 1 : 0;
     c.lbl_model0 = 0; c.lbl_dens = nullptr;
     for (size_t cell = 0; !E->lbl && cell < (size_t)(g.nlayer * g.ntemp); cell++)
@@ -92,7 +96,7 @@ int emu_init(const char *cfg) {
       read_cia(o.csfiles[i], E->cia[i]);
       std::vector<double> P, Q;
       fold_cia_table(E->cia[i], E->wn, P, Q);
-      E->PQ[i] = pack_cia_quads(P, Q, (int)E->cia[i].temp.size(), (int)E->wn.size(), 0);
+      E->PQ[i] = pack_cia_quads(P, Q, (int)E->cia[i].temp.size(), (int)E->wn.size(), kPad);
       c.ciaPQ[i] = E->PQ[i].data(); c.ciaT[i] = E->cia[i].temp.data();
       c.cia_nt[i] = (int)E->cia[i].temp.size();
       c.cia_nspec[i] = (int)E->cia[i].species.size();
@@ -114,7 +118,15 @@ int emu_init(const char *cfg) {
       c.wgt[a] = pow(sin(area[a + 1]), 2.0) - pow(sin(area[a]), 2.0);
     }
     fill_angle_consts(c);
-    c.planck_generic = 1;
+    // Planck chaining and the choice of the generic Planck term, as transit_init sets them
+    const int nw = c.nwave;
+    c.planck_cols = 0;
+    if (c.eclipse && nw > kThreads) {
+      c.planck_cols = kThreads;
+      c.planck_step = cH * cLS / cKB * kThreads * (E->wn[nw - 1] - E->wn[0]) / (nw - 1);
+    }
+    const double tmin = g.temp[0], tmax = g.temp[g.ntemp - 1], c2 = cH * cLS / cKB;
+    c.planck_generic = !(tmin > 0) || c2 * E->wn[nw - 1] / tmin > 690.0 || c2 * E->wn[0] / tmax < 0.1;
     double srad = o.starrad * kSUNRADIUS;
     c.inv_srad2 = 1.0 / (srad * srad);
     c.lay.nl = c.nlayer; c.lay.ngmol = c.ngmol; c.lay.ncia = c.ncia;
@@ -143,19 +155,105 @@ void emu_set_radius(double r) { E->k.r0_all = r; }
 void emu_set_cloudtop(double t) { E->k.cloud_flag_all = 1; E->k.cloudext_all = 100; E->k.cloudtop_all = t; E->k.cloudbot_all = t + 10; }
 void emu_set_scattering(int f, double v) { E->k.scat_flag_all = f; E->k.scat_logext_all = v; }
 
+} // extern "C"
+
+// atm_prep of one model: the table records tab[depth][record] and the radii; returns the status
+static int prep_model(const double *in, std::vector<double> &tab, std::vector<double> &rad) {
+  DevConfig &c = E->c;
+  const int nl = c.nlayer, ns = c.nspec;
+  std::vector<double> rho((size_t)ns * nl), mu(nl), hc(nl);
+  tab.assign(c.lay.stride(), 0.0);
+  rad.assign(nl, 0.0);
+  int status = 0;
+  for (int l = 0; l < nl; l++) status |= prep_layer(c, in, l, rho.data() + l, nl, &mu[l]);
+  KnobVals kv = knobs_for(E->k, 0);
+  for (int l = 0; l + 1 < nl; l++) hc[l] = hydro_coef(c, in, mu.data(), l);
+  hydrostatic_radii(c, kv.r0, in, mu.data(), hc.data(), rad.data());
+  for (int d = 0; d < nl; d++) status |= prep_table_row(c, kv, d, in, rho.data(), nl, rad.data(), tab.data());
+  return status;
+}
+
+// The eclipse throughput kernel's column loop (kernels.cu eclipse_column_kernel) over every tile of
+// kThreads x kCols columns: the same eclipse_columns instantiation, one emulated thread at a time
+template <int NMOL, int NCIA, int NANG, int SQ, bool PGEN, bool SC, bool AHEAD>
+static void throughput_tiles(const DevConfig &c, const double *tab, const unsigned long long *etab,
+                             double *spectrum) {
+  for (int t0 = 0; t0 < c.nwave; t0 += kThreads * kCols)
+    for (int x = 0; x < kThreads; x++) {
+      const int w0 = t0 + x;
+      bool valid[kCols];
+      double *tk[kCols];
+      int *lk[kCols];
+      double flux[kCols];
+      for (int k = 0; k < kCols; k++) { valid[k] = w0 + k * kThreads < c.nwave; tk[k] = nullptr; lk[k] = nullptr; }
+      eclipse_columns<NMOL, NCIA, NANG, false, kCols, SQ, true, kThreads, PGEN, SC, AHEAD>(c, tab, etab, w0, valid,
+                                                                                         tk, lk, flux);
+      for (int k = 0; k < kCols; k++) if (valid[k]) spectrum[w0 + k * kThreads] = flux[k];
+    }
+}
+
+extern "C" {
+
+// One eclipse model through the build launch_eclipse (kernels.cu) selects for the configuration: the
+// specialised (grid molecules, CIA files) pair with the default ray grid by squaring or a run-time
+// angle count, with or without the scattering / cloud terms, and the one-depth-ahead (ahead != 0)
+// or the in-step load order; the run-time-count build with the generic Planck term otherwise.
+// build[0..1] receives the (NMOL, NCIA) template arguments that ran (0, -1: run-time counts); a
+// rejected model runs no build.
+int emu_run_build(const double *in, int ahead, double *spectrum, int *build) {
+  DevConfig &c = E->c;
+  const Knobs &k = E->k;
+  if (!c.eclipse) return -1;                                   // eclipse configurations only
+  std::vector<double> tab, rad;
+  const int status = prep_model(in, tab, rad);
+  if (status) { for (int w = 0; w < c.nwave; w++) spectrum[w] = -1; return status; }
+  alignas(16) unsigned long long etab[(1 + kMaxAng) * kExpTabSize];
+  fill_ecl_exp_table(c, etab);
+  const bool sc = k.scat_flag_all != 0 || (k.cloud_flag_all == 1 && k.cloudext_all != 0.0);
+  const bool sq = c.nang == 5 && c.sq_src == 0 && c.sq_dst == 3;
+  const double *t = tab.data();
+  build[0] = 0; build[1] = -1;
+  auto pair = [&](auto nmol, auto ncia) {
+    constexpr int N = decltype(nmol)::value, C = decltype(ncia)::value;
+    build[0] = N; build[1] = C;
+    auto run = [&](auto sqc, auto scc, auto aheadc) {
+      constexpr bool S = decltype(sqc)::value;
+      throughput_tiles<N, C, S ? 5 : 0, S ? 0x03 : -1, false, decltype(scc)::value, decltype(aheadc)::value>(
+          c, t, etab, spectrum);
+    };
+    auto by_ahead = [&](auto sqc, auto scc) {
+      if (ahead) run(sqc, scc, std::true_type()); else run(sqc, scc, std::false_type());
+    };
+    auto by_sc = [&](auto sqc) { if (sc) by_ahead(sqc, std::true_type()); else by_ahead(sqc, std::false_type()); };
+    if (sq) by_sc(std::true_type()); else by_sc(std::false_type());
+  };
+  auto by_ncia = [&](auto nmol) {
+    switch (c.ncia) {
+      case 0: pair(nmol, std::integral_constant<int, 0>()); return true;
+      case 1: pair(nmol, std::integral_constant<int, 1>()); return true;
+      case 2: pair(nmol, std::integral_constant<int, 2>()); return true;
+    }
+    return false;
+  };
+  bool specialised = false;
+  if (!c.planck_generic) switch (c.ngmol) {
+    case 1: specialised = by_ncia(std::integral_constant<int, 1>()); break;
+    case 2: specialised = by_ncia(std::integral_constant<int, 2>()); break;
+    case 3: specialised = by_ncia(std::integral_constant<int, 3>()); break;
+    case 4: specialised = by_ncia(std::integral_constant<int, 4>()); break;
+  }
+  // the run-time-count build has one (in-step) form and always the scattering / cloud terms
+  if (!specialised) throughput_tiles<0, -1, 0, -1, true, true, false>(c, t, etab, spectrum);
+  return 0;
+}
+
 // one model; tau[nwave][nlayer], last[nwave], radius[nlayer] optional
 int emu_run(const double *in, double *spectrum, double *tau, int *last, double *radius,
             double *ext_total) {
   DevConfig &c = E->c;
-  const int nl = c.nlayer, ns = c.nspec, nw = c.nwave;
-  std::vector<double> rho((size_t)ns * nl), mu(nl), rad(nl), tab(c.lay.stride());
-  int status = 0;
-  for (int l = 0; l < nl; l++) status |= prep_layer(c, in, l, rho.data() + l, nl, &mu[l]);
-  KnobVals kv = knobs_for(E->k, 0);
-  std::vector<double> hc(nl);
-  for (int l = 0; l + 1 < nl; l++) hc[l] = hydro_coef(c, in, mu.data(), l);
-  hydrostatic_radii(c, kv.r0, in, mu.data(), hc.data(), rad.data());
-  for (int d = 0; d < nl; d++) status |= prep_table_row(c, kv, d, in, rho.data(), nl, rad.data(), tab.data());
+  const int nl = c.nlayer, nw = c.nwave;
+  std::vector<double> tab, rad;
+  int status = prep_model(in, tab, rad);
   if (radius) for (int l = 0; l < nl; l++) radius[l] = rad[l];
   if (status) { for (int w = 0; w < nw; w++) spectrum[w] = -1; return status; }
   std::vector<double> tk(nl), wts((size_t)nl * (nl + 1) / 2), er(nl);

@@ -48,3 +48,15 @@ class Emu:
             out["last"].ctypes.data_as(C.POINTER(C.c_int)), out["radius"].ctypes.data_as(dp),
             out["ext"].ctypes.data_as(dp))
         return out
+
+    def run_build(self, model, ahead):
+        """One eclipse model through the throughput kernel's build for this configuration
+        (emu_run_build): -> spectrum, status, (NMOL, NCIA) of the build that ran."""
+        model = np.ascontiguousarray(model, dtype=np.float64)
+        spec = np.zeros(self.nwave)
+        build = np.zeros(2, dtype=np.int32)
+        st = self.lib.emu_run_build(model.ctypes.data_as(dp), int(ahead), spec.ctypes.data_as(dp),
+                                    build.ctypes.data_as(C.POINTER(C.c_int)))
+        if st < 0:
+            raise RuntimeError("emu_run_build: not an eclipse configuration")
+        return spec, st, tuple(int(b) for b in build)
