@@ -30,6 +30,7 @@
 //
 // The temperature axis is the sharding axis (bart_build_opacity_slice): planes are independent.
 #include "builder.hpp"
+#include "cuda_host.hpp"
 #include "device.cuh"
 #include "column_math.cuh"
 #include <cuda_runtime.h>
@@ -40,36 +41,29 @@
 #include <map>
 #include <string>
 #include <chrono>
-#include <unistd.h>
-#include <fcntl.h>
 #include <cub/device/device_scan.cuh>
 #include <cub/iterator/transform_input_iterator.cuh>
 
 namespace bart {
 
-#define BCUDA(call)                                                                        \
-  do {                                                                                     \
-    cudaError_t e_ = (call);                                                               \
-    if (e_ != cudaSuccess) fail("CUDA error %s at %s:%d (%s)", cudaGetErrorString(e_),     \
-                                __FILE__, __LINE__, #call);                                \
-  } while (0)
-
-struct DevBuf {           // grow-only device buffer
-  void *p = nullptr; size_t cap = 0;
-  template <class T> T *get(size_t n) {
-    const size_t bytes = std::max<size_t>(1, n) * sizeof(T);
-    if (bytes > cap) {
-      if (p) cudaFree(p);
-      cap = bytes + bytes / 4;
-      BCUDA(cudaMalloc(&p, cap));
-    }
-    return (T *)p;
-  }
-  void release() { if (p) cudaFree(p); p = nullptr; cap = 0; }
-};
-
 constexpr int kMaxIso = 64;
 constexpr int kAccThreads = 128;
+
+struct CellIso;
+
+// Plane / cell work buffers of run_planes, shared by the grid build and the line-by-line forward
+// mode; sized per call (ensure_grow).
+struct PlaneWork {
+  DevBuf<double> T, tq, facfull, fac2, kmax, S;                        // per plane
+  DevBuf<int> blk;
+  DevBuf<long long> total, base, cisobeg;
+  DevBuf<int> c_idx;                                                   // compact pool
+  DevBuf<int> cell_plane;                                              // per cell
+  DevBuf<long long> cell_out;
+  DevBuf<CellIso> cellinfo;
+  DevBuf<int> iso_spec, iso_out;                                       // static tables
+  DevBuf<double> iso_mass, spec_mass, spec_radius;
+};
 
 struct BuilderState {
   // sampling
@@ -82,29 +76,24 @@ struct BuilderState {
   std::vector<double> ziso;                 // [niso][ntemp]
   // lines / groups
   long long nlines = 0, ngroups = 0, neval = 0;
-  double *d_wl = nullptr, *d_elow = nullptr, *d_gf = nullptr, *d_wavn = nullptr;   // raw lines
-  double *d_c_wavn = nullptr, *d_c_elow = nullptr, *d_c_gf = nullptr;             // grouped lines
-  short *d_isoid = nullptr;
-  int *d_iown = nullptr, *d_idwn = nullptr;
-  unsigned char *d_inrange = nullptr;
-  long long *d_gstart = nullptr;            // [ngroups+1]
-  int *d_giown = nullptr, *d_gidwn = nullptr;
-  short *d_giso = nullptr;
-  double *d_gwavn = nullptr;
+  DevBuf<double> d_c_wavn, d_c_elow, d_c_gf;      // grouped lines
+  DevBuf<long long> d_gstart;                     // [ngroups+1]
+  DevBuf<int> d_giown, d_gidwn;
+  DevBuf<short> d_giso;
+  DevBuf<double> d_gwavn;
   std::vector<long long> iso_gbeg;          // [niso+1] group range per isotope
   std::vector<int> h_iown;                  // per-line trace (leader bin, or -2-bin when co-added)
-  int *d_trace = nullptr;                   // the same trace when the grouping ran on the device
+  DevBuf<int> d_trace;                      // the same trace when the grouping ran on the device
   // Voigt table
   int nDop = 0, nLor = 0;
   std::vector<double> aDop, aLor;
   std::vector<long long> prof_off, prof_size;     // [nDop*nLor] offset (floats) and half-size
-  float *d_prof = nullptr;
+  DevBuf<float> d_prof;
   long long prof_total = 0;
-  double *d_aDop = nullptr, *d_aLor = nullptr;
-  long long *d_prof_off = nullptr, *d_prof_size = nullptr;
-  // plane / cell work buffers (run_planes)
-  struct PlaneWork *work = nullptr;
-  DevBuf dens, out;                              // grid build: [cell][nspec], [cell][ngmol][nwave]
+  DevBuf<double> d_aDop, d_aLor;
+  DevBuf<long long> d_prof_off, d_prof_size;
+  PlaneWork work;
+  DevBuf<double> dens, out;                      // grid build: [cell][nspec], [cell][ngmol][nwave]
   std::vector<std::vector<double>> zspline; // [niso] second derivatives of Z(T) (line-by-line mode)
   bool lines_loaded = false, profiles_ready = false, grid_ready = false;
   // per-phase wall/device milliseconds (bart_builder_phase_ms)
@@ -808,12 +797,6 @@ accumulate_kernel(CellArgs a, const CellIso *cells, double *out, int fast) {
 
 // ---------------------------------------------------------------------------------------
 // host side
-template <class T> static T *dev_upload(const std::vector<T> &v) {
-  T *p = nullptr;
-  BCUDA(cudaMalloc((void **)&p, std::max<size_t>(1, v.size()) * sizeof(T)));
-  if (!v.empty()) BCUDA(cudaMemcpy(p, v.data(), v.size() * sizeof(T), cudaMemcpyHostToDevice));
-  return p;
-}
 
 static void setup_static(BuilderState *b, const Options &o, const Atmosphere &a, const Molecules &mol,
                          Tli &t, const std::vector<double> &wn) {
@@ -926,18 +909,19 @@ static void build_profiles(BuilderState *b, const Options &o, cudaStream_t s) {
       jobs.push_back(jb);
     }
   b->prof_total = total;
-  BCUDA(cudaMalloc((void **)&b->d_prof, std::max<long long>(1, total) * sizeof(float)));
-  BCUDA(cudaMemsetAsync(b->d_prof, 0, std::max<long long>(1, total) * sizeof(float), s));
+  b->d_prof.ensure(std::max<long long>(1, total));
+  CUDA_OK(cudaMemsetAsync(b->d_prof.p, 0, std::max<long long>(1, total) * sizeof(float), s));
   // series coefficients 1/(n!(2n+1)) (the table of voigt.c:47-108)
   double ferf[64];
   long double fac = 1.0L;
   ferf[0] = 1.0;
   for (int n = 1; n < 64; n++) { fac *= n; ferf[n] = (double)(1.0L / (fac * (2 * n + 1))); }
-  BCUDA(cudaMemcpyToSymbol(c_ferf, ferf, sizeof(ferf)));
+  CUDA_OK(cudaMemcpyToSymbol(c_ferf, ferf, sizeof(ferf)));
   unsigned long long etab[kExpTabSize];
   fill_exp_table(etab);
-  BCUDA(cudaMemcpyToSymbol(b_exp_table, etab, sizeof(etab)));
-  ProfJob *d_jobs = dev_upload(jobs);
+  CUDA_OK(cudaMemcpyToSymbol(b_exp_table, etab, sizeof(etab)));
+  DevBuf<ProfJob> d_jobs;
+  upload(d_jobs, jobs);
   int maxn = 0;
   for (auto &j : jobs) maxn = std::max(maxn, j.nwn);
   // grid.y is limited to 65535 jobs; 60x60 profiles fit
@@ -946,48 +930,27 @@ static void build_profiles(BuilderState *b, const Options &o, cudaStream_t s) {
   for (size_t j0 = 0; j0 < jobs.size(); j0 += chunk) {
     const int nj = (int)std::min<size_t>(chunk, jobs.size() - j0);
     dim3 grid((maxn + 127) / 128, nj);
-    voigt_table_kernel<<<grid, 128, 0, s>>>(d_jobs + j0, b->d_prof);
+    voigt_table_kernel<<<grid, 128, 0, s>>>(d_jobs.p + j0, b->d_prof.p);
   }
-  BCUDA(cudaGetLastError());
-  BCUDA(cudaStreamSynchronize(s));
-  cudaFree(d_jobs);
-  b->d_aDop = dev_upload(b->aDop);
-  b->d_aLor = dev_upload(b->aLor);
-  b->d_prof_off = dev_upload(b->prof_off);
-  b->d_prof_size = dev_upload(b->prof_size);
+  CUDA_OK(cudaGetLastError());
+  CUDA_OK(cudaStreamSynchronize(s));
+  upload(b->d_aDop, b->aDop);
+  upload(b->d_aLor, b->aLor);
+  upload(b->d_prof_off, b->prof_off);
+  upload(b->d_prof_size, b->prof_size);
   b->profiles_ready = true;
 }
 
-// One column slice set of the TLI file -> device, through two pinned staging buffers: the pread of
-// chunk k + 1 (page cache or disk) overlaps the H2D copy of chunk k.  No host copy of the line list
-// is kept (2.6 GB at 1e8 lines).
-struct PinnedStage {
-  static constexpr size_t kBytes = (size_t)64 << 20;
-  char *buf[2] = {nullptr, nullptr};
-  cudaEvent_t ev[2];
-  int k = 0;
-  PinnedStage() {
-    for (int i = 0; i < 2; i++) {
-      BCUDA(cudaMallocHost((void **)&buf[i], kBytes));
-      BCUDA(cudaEventCreateWithFlags(&ev[i], cudaEventDisableTiming));
-    }
-  }
-  ~PinnedStage() { for (int i = 0; i < 2; i++) { cudaFreeHost(buf[i]); cudaEventDestroy(ev[i]); } }
-};
-
+// One column slice set of the TLI file -> device through the pinned staging.  No host copy of the
+// line list is kept (2.6 GB at 1e8 lines).
 static void upload_file_column(int fd, const TliLineMap &m, long long col_off, int esize, void *d_dst,
                                PinnedStage &st, cudaStream_t s) {
   char *dst = (char *)d_dst;
   for (size_t i = 0; i < m.count.size(); i++) {
     long long off = col_off + m.first[i] * esize, left = m.count[i] * esize;
     while (left > 0) {
-      const size_t chunk = (size_t)std::min<long long>(left, (long long)PinnedStage::kBytes);
-      char *hb = st.buf[st.k];
-      BCUDA(cudaEventSynchronize(st.ev[st.k]));            // the copy that last used this buffer
-      if (!parallel_pread(fd, hb, chunk, off)) fail("TLI file: read failed");
-      BCUDA(cudaMemcpyAsync(dst, hb, chunk, cudaMemcpyHostToDevice, s));
-      BCUDA(cudaEventRecord(st.ev[st.k], s));
-      st.k ^= 1;
+      const size_t chunk = (size_t)std::min<long long>(left, (long long)st.size());
+      if (!st.put(fd, off, chunk, dst, s)) fail("TLI file: read failed");
       dst += chunk; off += (long long)chunk; left -= (long long)chunk;
     }
   }
@@ -1007,125 +970,102 @@ static bool load_lines_device(BuilderState *b, const Options &o, const Tli &t, d
   map_tli_lines(o.linedb, t, lo, hi_hint, m);
   const long long n = m.total;
   const long long na = std::max<long long>(1, n);
-  double *d_wl, *d_elow, *d_gf, *d_wavn;
-  short *d_iso;
-  int *d_iown, *d_idwn, *d_flags, *d_trace;
-  unsigned char *d_inr, *d_spec, *d_fixl, *d_flag;
-  long long *d_lrank, *d_mrank, *d_exit, *d_merge;
-  BCUDA(cudaMalloc((void **)&d_wl, na * 8)); BCUDA(cudaMalloc((void **)&d_elow, na * 8));
-  BCUDA(cudaMalloc((void **)&d_gf, na * 8)); BCUDA(cudaMalloc((void **)&d_iso, na * 2));
+  DevBuf<double> d_wl(na), d_elow(na), d_gf(na);
+  DevBuf<short> d_iso(na);
   {
     PinnedStage st;
-    const int fd = open(o.linedb.c_str(), O_RDONLY);
+    const Fd fd(o.linedb.c_str(), O_RDONLY);
     if (fd < 0) fail("Data file '%s' not found.", o.linedb.c_str());
-    upload_file_column(fd, m, m.wl_off, 8, d_wl, st, s);
-    upload_file_column(fd, m, m.iso_off, 2, d_iso, st, s);
-    upload_file_column(fd, m, m.el_off, 8, d_elow, st, s);
-    upload_file_column(fd, m, m.gf_off, 8, d_gf, st, s);
-    BCUDA(cudaStreamSynchronize(s));
-    close(fd);
+    upload_file_column(fd, m, m.wl_off, 8, d_wl.p, st, s);
+    upload_file_column(fd, m, m.iso_off, 2, d_iso.p, st, s);
+    upload_file_column(fd, m, m.el_off, 8, d_elow.p, st, s);
+    upload_file_column(fd, m, m.gf_off, 8, d_gf.p, st, s);
+    CUDA_OK(cudaStreamSynchronize(s));
   }
   lap("read_tli_host");
-  BCUDA(cudaMalloc((void **)&d_wavn, na * 8)); BCUDA(cudaMalloc((void **)&d_iown, na * 4));
-  BCUDA(cudaMalloc((void **)&d_idwn, na * 4)); BCUDA(cudaMalloc((void **)&d_inr, na));
+  DevBuf<double> d_wavn(na);
+  DevBuf<int> d_iown(na), d_idwn(na);
+  DevBuf<unsigned char> d_inr(na);
   const long long nblocks = (na + kGrpBlock - 1) / kGrpBlock;
-  BCUDA(cudaMalloc((void **)&d_spec, na)); BCUDA(cudaMalloc((void **)&d_fixl, na));
-  BCUDA(cudaMalloc((void **)&d_flag, na));
-  BCUDA(cudaMalloc((void **)&d_trace, na * 4));
-  BCUDA(cudaMalloc((void **)&d_flags, 4));
-  BCUDA(cudaMalloc((void **)&d_exit, nblocks * 8)); BCUDA(cudaMalloc((void **)&d_merge, nblocks * 8));
-  BCUDA(cudaMalloc((void **)&d_lrank, (na + 1) * 8)); BCUDA(cudaMalloc((void **)&d_mrank, (na + 1) * 8));
-  auto drop = [&](std::initializer_list<void *> ps) { for (void *q : ps) cudaFree(q); };
+  DevBuf<unsigned char> d_spec(na), d_fixl(na), d_flag(na);
+  DevBuf<int> d_trace(na), d_flags(1);
+  DevBuf<long long> d_exit(nblocks), d_merge(nblocks), d_lrank(na + 1), d_mrank(na + 1);
   const double own_last = b->wn_lo + (double)(b->nowns - 1) * b->odwn;
   const unsigned grid = (unsigned)((na + 255) / 256);
-  BCUDA(cudaMemsetAsync(d_flags, 0, 4, s));
-  BCUDA(cudaMemsetAsync(d_spec, 0, na, s));
-  BCUDA(cudaMemsetAsync(d_fixl, 0, na, s));
-  BCUDA(cudaMemsetAsync(d_flag, 0, na, s));
-  BCUDA(cudaMemsetAsync(d_trace, 0xff, na * 4, s));                 // -1: in no group
+  CUDA_OK(cudaMemsetAsync(d_flags.p, 0, 4, s));
+  CUDA_OK(cudaMemsetAsync(d_spec.p, 0, na, s));
+  CUDA_OK(cudaMemsetAsync(d_fixl.p, 0, na, s));
+  CUDA_OK(cudaMemsetAsync(d_flag.p, 0, na, s));
+  CUDA_OK(cudaMemsetAsync(d_trace.p, 0xff, na * 4, s));               // -1: in no group
   int flags = 0;
   if (n > 0) {
-    line_index_kernel<<<grid, 256, 0, s>>>(d_wl, n, b->wn_lo, own_last, b->odwn, b->dwn, d_wavn, d_iown,
-                                           d_idwn, d_inr);
-    group_check_kernel<<<grid, 256, 0, s>>>(d_iso, d_inr, n, b->niso, d_flags);
-    BCUDA(cudaGetLastError());
-    BCUDA(cudaMemcpyAsync(&flags, d_flags, 4, cudaMemcpyDeviceToHost, s));
-    BCUDA(cudaStreamSynchronize(s));
+    line_index_kernel<<<grid, 256, 0, s>>>(d_wl.p, n, b->wn_lo, own_last, b->odwn, b->dwn, d_wavn.p, d_iown.p,
+                                           d_idwn.p, d_inr.p);
+    group_check_kernel<<<grid, 256, 0, s>>>(d_iso.p, d_inr.p, n, b->niso, d_flags.p);
+    CUDA_OK(cudaGetLastError());
+    CUDA_OK(cudaMemcpyAsync(&flags, d_flags.p, 4, cudaMemcpyDeviceToHost, s));
+    CUDA_OK(cudaStreamSynchronize(s));
   }
-  auto drop_all = [&]() {
-    drop({d_wl, d_elow, d_gf, d_iso, d_wavn, d_iown, d_idwn, d_inr, d_spec, d_fixl, d_flag, d_trace, d_flags,
-          d_exit, d_merge, d_lrank, d_mrank});
-  };
-  if (flags & 3) drop_all();
   if (flags & 1) fail("a TLI line has an isotope index outside [0,%d)", b->niso);
   if (flags & 2) fail("TLI lines are not grouped by isotope");
   long long ngroups = 0, nmember = 0;
   if (n > 0) {
-    GroupArgs ga{d_wavn, d_iso, d_inr, d_iown, n, b->wn_lo, b->odwn};
-    group_spec_kernel<<<(unsigned)((nblocks + 127) / 128), 128, 0, s>>>(ga, nblocks, d_spec, d_exit);
-    group_fix_kernel<<<1, 1, 0, s>>>(ga, nblocks, d_spec, d_exit, d_fixl, d_merge, d_flags);
-    BCUDA(cudaGetLastError());
-    BCUDA(cudaMemcpyAsync(&flags, d_flags, 4, cudaMemcpyDeviceToHost, s));
-    BCUDA(cudaStreamSynchronize(s));
-    if (flags) {                                   // the walks never merged: host path
-      drop_all();
-      return false;
-    }
-    group_mark_kernel<<<grid, 256, 0, s>>>(ga, d_spec, d_fixl, d_merge, d_flag, d_trace);
-    BCUDA(cudaGetLastError());
+    GroupArgs ga{d_wavn.p, d_iso.p, d_inr.p, d_iown.p, n, b->wn_lo, b->odwn};
+    group_spec_kernel<<<(unsigned)((nblocks + 127) / 128), 128, 0, s>>>(ga, nblocks, d_spec.p, d_exit.p);
+    group_fix_kernel<<<1, 1, 0, s>>>(ga, nblocks, d_spec.p, d_exit.p, d_fixl.p, d_merge.p, d_flags.p);
+    CUDA_OK(cudaGetLastError());
+    CUDA_OK(cudaMemcpyAsync(&flags, d_flags.p, 4, cudaMemcpyDeviceToHost, s));
+    CUDA_OK(cudaStreamSynchronize(s));
+    if (flags) return false;                       // the walks never merged: host path
+    group_mark_kernel<<<grid, 256, 0, s>>>(ga, d_spec.p, d_fixl.p, d_merge.p, d_flag.p, d_trace.p);
+    CUDA_OK(cudaGetLastError());
     // ranks of the leaders (group numbers) and of the members (positions in the grouped line
     // arrays): exclusive sums over n + 1 flags, the last entry being the total
-    cub::TransformInputIterator<long long, FlagBit, const unsigned char *> lead(d_flag, FlagBit{0}),
-        memb(d_flag, FlagBit{1});
+    cub::TransformInputIterator<long long, FlagBit, const unsigned char *> lead(d_flag.p, FlagBit{0}),
+        memb(d_flag.p, FlagBit{1});
     size_t tmp_bytes = 0;
-    cub::DeviceScan::ExclusiveSum(nullptr, tmp_bytes, lead, d_lrank, n, s);
-    void *d_tmp = nullptr;
-    BCUDA(cudaMalloc(&d_tmp, std::max<size_t>(1, tmp_bytes)));
-    cub::DeviceScan::ExclusiveSum(d_tmp, tmp_bytes, lead, d_lrank, n, s);
-    cub::DeviceScan::ExclusiveSum(d_tmp, tmp_bytes, memb, d_mrank, n, s);
-    BCUDA(cudaGetLastError());
+    cub::DeviceScan::ExclusiveSum(nullptr, tmp_bytes, lead, d_lrank.p, n, s);
+    DevBuf<char> d_tmp(std::max<size_t>(1, tmp_bytes));
+    cub::DeviceScan::ExclusiveSum(d_tmp.p, tmp_bytes, lead, d_lrank.p, n, s);
+    cub::DeviceScan::ExclusiveSum(d_tmp.p, tmp_bytes, memb, d_mrank.p, n, s);
+    CUDA_OK(cudaGetLastError());
     long long lastr[2];
     unsigned char lastf = 0;
-    BCUDA(cudaMemcpyAsync(&lastr[0], d_lrank + (n - 1), 8, cudaMemcpyDeviceToHost, s));
-    BCUDA(cudaMemcpyAsync(&lastr[1], d_mrank + (n - 1), 8, cudaMemcpyDeviceToHost, s));
-    BCUDA(cudaMemcpyAsync(&lastf, d_flag + (n - 1), 1, cudaMemcpyDeviceToHost, s));
-    BCUDA(cudaStreamSynchronize(s));
-    cudaFree(d_tmp);
+    CUDA_OK(cudaMemcpyAsync(&lastr[0], d_lrank.p + (n - 1), 8, cudaMemcpyDeviceToHost, s));
+    CUDA_OK(cudaMemcpyAsync(&lastr[1], d_mrank.p + (n - 1), 8, cudaMemcpyDeviceToHost, s));
+    CUDA_OK(cudaMemcpyAsync(&lastf, d_flag.p + (n - 1), 1, cudaMemcpyDeviceToHost, s));
+    CUDA_OK(cudaStreamSynchronize(s));
     ngroups = lastr[0] + (lastf & 1);
     nmember = lastr[1] + ((lastf >> 1) & 1);
   }
   b->nlines = n;
   b->ngroups = ngroups;
-  BCUDA(cudaMalloc((void **)&b->d_gstart, (ngroups + 1) * 8));
-  BCUDA(cudaMalloc((void **)&b->d_giown, std::max<long long>(1, ngroups) * 4));
-  BCUDA(cudaMalloc((void **)&b->d_gidwn, std::max<long long>(1, ngroups) * 4));
-  BCUDA(cudaMalloc((void **)&b->d_giso, std::max<long long>(1, ngroups) * 2));
-  BCUDA(cudaMalloc((void **)&b->d_gwavn, std::max<long long>(1, ngroups) * 8));
-  BCUDA(cudaMalloc((void **)&b->d_c_wavn, std::max<long long>(1, nmember) * 8));
-  BCUDA(cudaMalloc((void **)&b->d_c_elow, std::max<long long>(1, nmember) * 8));
-  BCUDA(cudaMalloc((void **)&b->d_c_gf, std::max<long long>(1, nmember) * 8));
+  b->d_gstart.ensure(ngroups + 1);
+  b->d_giown.ensure(std::max<long long>(1, ngroups));
+  b->d_gidwn.ensure(std::max<long long>(1, ngroups));
+  b->d_giso.ensure(std::max<long long>(1, ngroups));
+  b->d_gwavn.ensure(std::max<long long>(1, ngroups));
+  b->d_c_wavn.ensure(std::max<long long>(1, nmember));
+  b->d_c_elow.ensure(std::max<long long>(1, nmember));
+  b->d_c_gf.ensure(std::max<long long>(1, nmember));
   if (n > 0) {
-    group_fill_kernel<<<grid, 256, 0, s>>>(d_wavn, d_elow, d_gf, d_iso, d_iown, d_idwn, d_flag, d_lrank,
-                                           d_mrank, n, b->d_gstart, b->d_giown, b->d_gidwn, b->d_giso,
-                                           b->d_gwavn, b->d_c_wavn, b->d_c_elow, b->d_c_gf);
-    BCUDA(cudaGetLastError());
+    group_fill_kernel<<<grid, 256, 0, s>>>(d_wavn.p, d_elow.p, d_gf.p, d_iso.p, d_iown.p, d_idwn.p, d_flag.p,
+                                           d_lrank.p, d_mrank.p, n, b->d_gstart.p, b->d_giown.p, b->d_gidwn.p,
+                                           b->d_giso.p, b->d_gwavn.p, b->d_c_wavn.p, b->d_c_elow.p, b->d_c_gf.p);
+    CUDA_OK(cudaGetLastError());
   }
-  BCUDA(cudaMemcpyAsync(b->d_gstart + ngroups, &nmember, 8, cudaMemcpyHostToDevice, s));
+  CUDA_OK(cudaMemcpyAsync(b->d_gstart.p + ngroups, &nmember, 8, cudaMemcpyHostToDevice, s));
   b->iso_gbeg.assign(b->niso + 1, ngroups);
   if (n > 0) {
-    long long *d_gbeg = nullptr;
-    BCUDA(cudaMalloc((void **)&d_gbeg, (b->niso + 1) * 8));
-    group_isobeg_kernel<<<1, 128, 0, s>>>(d_iso, n, b->niso, d_lrank, ngroups, d_gbeg);
-    BCUDA(cudaGetLastError());
-    BCUDA(cudaMemcpyAsync(b->iso_gbeg.data(), d_gbeg, (b->niso + 1) * 8, cudaMemcpyDeviceToHost, s));
-    BCUDA(cudaStreamSynchronize(s));
-    cudaFree(d_gbeg);
+    DevBuf<long long> d_gbeg(b->niso + 1);
+    group_isobeg_kernel<<<1, 128, 0, s>>>(d_iso.p, n, b->niso, d_lrank.p, ngroups, d_gbeg.p);
+    CUDA_OK(cudaGetLastError());
+    CUDA_OK(cudaMemcpyAsync(b->iso_gbeg.data(), d_gbeg.p, (b->niso + 1) * 8, cudaMemcpyDeviceToHost, s));
+    CUDA_OK(cudaStreamSynchronize(s));
   }
-  BCUDA(cudaStreamSynchronize(s));
+  CUDA_OK(cudaStreamSynchronize(s));
   b->h_iown.clear();
-  b->d_trace = d_trace;
-  drop({d_wl, d_elow, d_gf, d_iso, d_wavn, d_iown, d_idwn, d_inr, d_spec, d_fixl, d_flag, d_flags, d_exit,
-        d_merge, d_lrank, d_mrank});
+  b->d_trace = std::move(d_trace);
   lap("grouping_device");
   return true;
 }
@@ -1153,28 +1093,31 @@ static void load_lines(BuilderState *b, const Options &o, Tli &t, const std::vec
     from = now;
   };
   auto tl = std::chrono::steady_clock::now();
-  b->d_wl = dev_upload(t.wl); b->d_elow = dev_upload(t.elow); b->d_gf = dev_upload(t.gf);
-  b->d_isoid = dev_upload(t.isoid);
-  BCUDA(cudaMalloc((void **)&b->d_wavn, std::max<long long>(1, n) * 8));
-  BCUDA(cudaMalloc((void **)&b->d_iown, std::max<long long>(1, n) * 4));
-  BCUDA(cudaMalloc((void **)&b->d_idwn, std::max<long long>(1, n) * 4));
-  BCUDA(cudaMalloc((void **)&b->d_inrange, std::max<long long>(1, n)));
+  // the raw per-line arrays live until the grouped copies are on the device
+  DevBuf<double> d_wl, d_elow, d_gf;
+  DevBuf<short> d_isoid;
+  upload(d_wl, t.wl); upload(d_elow, t.elow); upload(d_gf, t.gf);
+  upload(d_isoid, t.isoid);
+  const long long na = std::max<long long>(1, n);
+  DevBuf<double> d_wavn(na);
+  DevBuf<int> d_iown(na), d_idwn(na);
+  DevBuf<unsigned char> d_inrange(na);
   const double own_last = b->wn_lo + (double)(b->nowns - 1) * b->odwn;
   if (n > 0) {
-    line_index_kernel<<<(unsigned)((n + 255) / 256), 256, 0, s>>>(b->d_wl, n, b->wn_lo, own_last, b->odwn,
-                                                                   b->dwn, b->d_wavn, b->d_iown, b->d_idwn,
-                                                                   b->d_inrange);
-    BCUDA(cudaGetLastError());
+    line_index_kernel<<<(unsigned)((n + 255) / 256), 256, 0, s>>>(d_wl.p, n, b->wn_lo, own_last, b->odwn,
+                                                                   b->dwn, d_wavn.p, d_iown.p, d_idwn.p,
+                                                                   d_inrange.p);
+    CUDA_OK(cudaGetLastError());
   }
   std::vector<double> wavn(n);
   std::vector<int> iown(n), idwn(n);
   std::vector<unsigned char> inr(n);
-  BCUDA(cudaStreamSynchronize(s));
+  CUDA_OK(cudaStreamSynchronize(s));
   if (n > 0) {
-    BCUDA(cudaMemcpy(wavn.data(), b->d_wavn, n * 8, cudaMemcpyDeviceToHost));
-    BCUDA(cudaMemcpy(iown.data(), b->d_iown, n * 4, cudaMemcpyDeviceToHost));
-    BCUDA(cudaMemcpy(idwn.data(), b->d_idwn, n * 4, cudaMemcpyDeviceToHost));
-    BCUDA(cudaMemcpy(inr.data(), b->d_inrange, n, cudaMemcpyDeviceToHost));
+    CUDA_OK(cudaMemcpy(wavn.data(), d_wavn.p, n * 8, cudaMemcpyDeviceToHost));
+    CUDA_OK(cudaMemcpy(iown.data(), d_iown.p, n * 4, cudaMemcpyDeviceToHost));
+    CUDA_OK(cudaMemcpy(idwn.data(), d_idwn.p, n * 4, cudaMemcpyDeviceToHost));
+    CUDA_OK(cudaMemcpy(inr.data(), d_inrange.p, n, cudaMemcpyDeviceToHost));
   }
   lap("lines_h2d_index_d2h", tl);
   // co-add grouping (extinction.c:450-462): a leader absorbs the following lines of the same
@@ -1218,41 +1161,28 @@ static void load_lines(BuilderState *b, const Options &o, Tli &t, const std::vec
   b->phase_ms["grouping_host"] += std::chrono::duration<double, std::milli>(
       std::chrono::steady_clock::now() - tg0).count();
   tl = std::chrono::steady_clock::now();
-  b->d_gstart = dev_upload(bounds);
-  b->d_giown = dev_upload(giown); b->d_gidwn = dev_upload(gidwn); b->d_giso = dev_upload(giso);
-  b->d_gwavn = dev_upload(gwavn);
-  b->d_c_wavn = dev_upload(c_wavn); b->d_c_elow = dev_upload(c_elow); b->d_c_gf = dev_upload(c_gf);
-  // the raw per-line arrays are no longer needed on the device: everything downstream works on
-  // the grouped copies
-  for (void **q : {(void **)&b->d_wl, (void **)&b->d_elow, (void **)&b->d_gf, (void **)&b->d_wavn,
-                   (void **)&b->d_isoid, (void **)&b->d_iown, (void **)&b->d_idwn, (void **)&b->d_inrange}) {
-    cudaFree(*q); *q = nullptr;
-  }
+  upload(b->d_gstart, bounds);
+  upload(b->d_giown, giown); upload(b->d_gidwn, gidwn); upload(b->d_giso, giso);
+  upload(b->d_gwavn, gwavn);
+  upload(b->d_c_wavn, c_wavn); upload(b->d_c_elow, c_elow); upload(b->d_c_gf, c_gf);
   lap("groups_h2d", tl);
   b->lines_loaded = true;
 }
 
 // ---------------------------------------------------------------------------------------
 // Plane / cell driver shared by the grid build and the line-by-line forward mode.
-struct PlaneWork {
-  DevBuf T, tq, facfull, fac2, kmax, blk, total, base, cisobeg, S;    // per plane
-  DevBuf c_idx;                                                        // compact pool
-  DevBuf cell_plane, cell_out, cellinfo;                               // per cell
-  DevBuf iso_spec, iso_out, iso_mass, spec_mass, spec_radius;          // static tables
-  bool statics = false;
-};
 
 static void upload_statics(BuilderState *b, const Molecules &mol, const Tli &t, bool total_mode,
                            cudaStream_t s) {
-  PlaneWork &w = *b->work;
+  PlaneWork &w = b->work;
   std::vector<int> iso_out = b->iso_gmol;
   if (total_mode) std::fill(iso_out.begin(), iso_out.end(), 0);      // permol = 0: m stays 0
-  BCUDA(cudaMemcpyAsync(w.iso_spec.get<int>(b->niso), b->iso_spec.data(), b->niso * 4, cudaMemcpyHostToDevice, s));
-  BCUDA(cudaMemcpyAsync(w.iso_out.get<int>(b->niso), iso_out.data(), b->niso * 4, cudaMemcpyHostToDevice, s));
-  BCUDA(cudaMemcpyAsync(w.iso_mass.get<double>(b->niso), t.iso_mass.data(), b->niso * 8, cudaMemcpyHostToDevice, s));
-  BCUDA(cudaMemcpyAsync(w.spec_mass.get<double>(b->nspec), mol.mass.data(), b->nspec * 8, cudaMemcpyHostToDevice, s));
-  BCUDA(cudaMemcpyAsync(w.spec_radius.get<double>(b->nspec), mol.radius_cm.data(), b->nspec * 8, cudaMemcpyHostToDevice, s));
-  BCUDA(cudaStreamSynchronize(s));
+  CUDA_OK(cudaMemcpyAsync(w.iso_spec.ensure_grow(b->niso), b->iso_spec.data(), b->niso * 4, cudaMemcpyHostToDevice, s));
+  CUDA_OK(cudaMemcpyAsync(w.iso_out.ensure_grow(b->niso), iso_out.data(), b->niso * 4, cudaMemcpyHostToDevice, s));
+  CUDA_OK(cudaMemcpyAsync(w.iso_mass.ensure_grow(b->niso), t.iso_mass.data(), b->niso * 8, cudaMemcpyHostToDevice, s));
+  CUDA_OK(cudaMemcpyAsync(w.spec_mass.ensure_grow(b->nspec), mol.mass.data(), b->nspec * 8, cudaMemcpyHostToDevice, s));
+  CUDA_OK(cudaMemcpyAsync(w.spec_radius.ensure_grow(b->nspec), mol.radius_cm.data(), b->nspec * 8, cudaMemcpyHostToDevice, s));
+  CUDA_OK(cudaStreamSynchronize(s));
 }
 
 // Runs nplanes planes / ncell cells.  plane_T[P]; plane_Z[P][niso] partition functions;
@@ -1264,8 +1194,7 @@ static long long run_planes(BuilderState *b, const Options &o, const Molecules &
                             const int *cell_plane, const double *d_cell_dens,
                             const long long *cell_out, double *d_out, bool total_mode,
                             cudaStream_t s) {
-  if (!b->work) b->work = new PlaneWork();
-  PlaneWork &w = *b->work;
+  PlaneWork &w = b->work;
   upload_statics(b, mol, t, total_mode, s);
   const int niso = b->niso, nout = total_mode ? 1 : b->ngmol;
   const int nblk = (int)((b->ngroups + kCompactThreads - 1) / kCompactThreads);
@@ -1278,27 +1207,28 @@ static long long run_planes(BuilderState *b, const Options &o, const Molecules &
       facfull[(size_t)p * niso + i] = t.iso_ratio[i] * kSIGCTE / t.iso_mass[i] / Z;
       fac2[(size_t)p * niso + i] = kSIGCTE * t.iso_ratio[i] / (t.iso_mass[i] * Z);
     }
-  double *d_T = w.T.get<double>(nplanes), *d_facfull = w.facfull.get<double>(facfull.size()),
-         *d_fac2 = w.fac2.get<double>(fac2.size()), *d_kmax = w.kmax.get<double>((size_t)nplanes * kMaxGridMol);
-  int *d_blk = w.blk.get<int>((size_t)nplanes * std::max(1, nblk));
-  long long *d_total = w.total.get<long long>(nplanes), *d_base = w.base.get<long long>(nplanes),
-            *d_cisobeg = w.cisobeg.get<long long>((size_t)nplanes * (niso + 1));
-  BCUDA(cudaMemcpyAsync(d_T, plane_T, nplanes * 8, cudaMemcpyHostToDevice, s));
+  double *d_T = w.T.ensure_grow(nplanes), *d_facfull = w.facfull.ensure_grow(facfull.size()),
+         *d_fac2 = w.fac2.ensure_grow(fac2.size()), *d_kmax = w.kmax.ensure_grow((size_t)nplanes * kMaxGridMol);
+  int *d_blk = w.blk.ensure_grow((size_t)nplanes * std::max(1, nblk));
+  long long *d_total = w.total.ensure_grow(nplanes), *d_base = w.base.ensure_grow(nplanes),
+            *d_cisobeg = w.cisobeg.ensure_grow((size_t)nplanes * (niso + 1));
+  CUDA_OK(cudaMemcpyAsync(d_T, plane_T, nplanes * 8, cudaMemcpyHostToDevice, s));
   std::vector<double> tq(nplanes);
   for (int p = 0; p < nplanes; p++) tq[p] = -kEXPCTE / plane_T[p];
-  double *d_tq = w.tq.get<double>(nplanes);
-  BCUDA(cudaMemcpyAsync(d_tq, tq.data(), nplanes * 8, cudaMemcpyHostToDevice, s));
-  BCUDA(cudaMemcpyAsync(d_facfull, facfull.data(), facfull.size() * 8, cudaMemcpyHostToDevice, s));
-  BCUDA(cudaMemcpyAsync(d_fac2, fac2.data(), fac2.size() * 8, cudaMemcpyHostToDevice, s));
-  BCUDA(cudaMemsetAsync(d_kmax, 0, (size_t)nplanes * kMaxGridMol * 8, s));
-  BCUDA(cudaMemsetAsync(d_cisobeg, 0, (size_t)nplanes * (niso + 1) * 8, s));
-  BCUDA(cudaMemsetAsync(d_total, 0, (size_t)nplanes * 8, s));
-  const int *d_iso_out = (const int *)w.iso_out.p;
+  double *d_tq = w.tq.ensure_grow(nplanes);
+  CUDA_OK(cudaMemcpyAsync(d_tq, tq.data(), nplanes * 8, cudaMemcpyHostToDevice, s));
+  CUDA_OK(cudaMemcpyAsync(d_facfull, facfull.data(), facfull.size() * 8, cudaMemcpyHostToDevice, s));
+  CUDA_OK(cudaMemcpyAsync(d_fac2, fac2.data(), fac2.size() * 8, cudaMemcpyHostToDevice, s));
+  CUDA_OK(cudaMemsetAsync(d_kmax, 0, (size_t)nplanes * kMaxGridMol * 8, s));
+  CUDA_OK(cudaMemsetAsync(d_cisobeg, 0, (size_t)nplanes * (niso + 1) * 8, s));
+  CUDA_OK(cudaMemsetAsync(d_total, 0, (size_t)nplanes * 8, s));
+  const int *d_iso_out = w.iso_out.p;
   PlaneArgs pa;
-  pa.gstart = b->d_gstart; pa.giso = b->d_giso; pa.wavn = b->d_c_wavn; pa.elow = b->d_c_elow; pa.gf = b->d_c_gf;
+  pa.gstart = b->d_gstart.p; pa.giso = b->d_giso.p; pa.wavn = b->d_c_wavn.p; pa.elow = b->d_c_elow.p;
+  pa.gf = b->d_c_gf.p;
   pa.ngroups = b->ngroups; pa.plane_T = d_T; pa.plane_fac2 = d_fac2; pa.plane_facfull = d_facfull;
   pa.plane_tq = d_tq;
-  pa.kmax = d_kmax; pa.S = w.S.get<double>((size_t)nplanes * std::max<long long>(1, b->ngroups));
+  pa.kmax = d_kmax; pa.S = w.S.ensure_grow((size_t)nplanes * std::max<long long>(1, b->ngroups));
   pa.iso_out = d_iso_out; pa.niso = niso; pa.nout = nout; pa.ethresh = o.ethreshold; pa.nblk = nblk;
   pa.wn_lo = b->wn_lo; pa.own_last = b->wn_lo + (double)(b->nowns - 1) * b->odwn;
   std::vector<long long> total(nplanes, 0), base(nplanes, 0);
@@ -1308,42 +1238,40 @@ static long long run_planes(BuilderState *b, const Options &o, const Molecules &
     strength_kmax_kernel<<<dim3(nblk, (nplanes + kPlanesPerThread - 1) / kPlanesPerThread), kCompactThreads, 0, s>>>(pa, nplanes);
     strength_count_kernel<<<dim3(nblk, nplanes), kCompactThreads, 0, s>>>(pa, d_blk);
     block_scan_kernel<<<nplanes, 1024, 0, s>>>(d_blk, nblk, d_total);
-    BCUDA(cudaGetLastError());
-    BCUDA(cudaMemcpyAsync(total.data(), d_total, nplanes * 8, cudaMemcpyDeviceToHost, s));
-    BCUDA(cudaStreamSynchronize(s));
+    CUDA_OK(cudaGetLastError());
+    CUDA_OK(cudaMemcpyAsync(total.data(), d_total, nplanes * 8, cudaMemcpyDeviceToHost, s));
+    CUDA_OK(cudaStreamSynchronize(s));
     for (int p = 0; p < nplanes; p++) { base[p] = pool; pool += total[p]; }
-    BCUDA(cudaMemcpyAsync(d_base, base.data(), nplanes * 8, cudaMemcpyHostToDevice, s));
-    int *ci = w.c_idx.get<int>(pool);
+    CUDA_OK(cudaMemcpyAsync(d_base, base.data(), nplanes * 8, cudaMemcpyHostToDevice, s));
+    int *ci = w.c_idx.ensure_grow(pool);
     strength_fill_kernel<<<dim3(nblk, nplanes), kCompactThreads, 0, s>>>(pa, d_blk, d_base, ci, d_cisobeg);
-    BCUDA(cudaGetLastError());
+    CUDA_OK(cudaGetLastError());
   } else {
-    BCUDA(cudaMemsetAsync(d_base, 0, nplanes * 8, s));
-    w.c_idx.get<int>(1);
+    CUDA_OK(cudaMemsetAsync(d_base, 0, nplanes * 8, s));
+    w.c_idx.ensure_grow(1);
   }
-  int *d_cell_plane = w.cell_plane.get<int>(ncell);
-  long long *d_cell_out = w.cell_out.get<long long>(ncell);
-  CellIso *cells = w.cellinfo.get<CellIso>((size_t)ncell * niso);
-  BCUDA(cudaMemcpyAsync(d_cell_plane, cell_plane, ncell * 4, cudaMemcpyHostToDevice, s));
-  BCUDA(cudaMemcpyAsync(d_cell_out, cell_out, ncell * 8, cudaMemcpyHostToDevice, s));
+  int *d_cell_plane = w.cell_plane.ensure_grow(ncell);
+  long long *d_cell_out = w.cell_out.ensure_grow(ncell);
+  CellIso *cells = w.cellinfo.ensure_grow((size_t)ncell * niso);
+  CUDA_OK(cudaMemcpyAsync(d_cell_plane, cell_plane, ncell * 4, cudaMemcpyHostToDevice, s));
+  CUDA_OK(cudaMemcpyAsync(d_cell_out, cell_out, ncell * 8, cudaMemcpyHostToDevice, s));
   CellArgs ca;
   ca.cell_plane = d_cell_plane; ca.cell_dens = d_cell_dens; ca.cell_out = d_cell_out;
   ca.plane_T = d_T; ca.plane_base = d_base; ca.cisobeg = d_cisobeg;
-  ca.c_idx = (const int *)w.c_idx.p;
-  ca.giown = b->d_giown; ca.gidwn = b->d_gidwn; ca.gwavn = b->d_gwavn;
+  ca.c_idx = w.c_idx.p;
+  ca.giown = b->d_giown.p; ca.gidwn = b->d_gidwn.p; ca.gwavn = b->d_gwavn.p;
   ca.S = pa.S; ca.ngroups = std::max<long long>(1, b->ngroups);
   ca.niso = niso; ca.nspec = b->nspec; ca.nout = nout; ca.nwave = b->nwave; ca.osamp = b->osamp;
   ca.nDop = b->nDop; ca.nLor = b->nLor;
-  ca.iso_spec = (const int *)w.iso_spec.p; ca.iso_out = d_iso_out;
-  ca.aDop = b->d_aDop; ca.aLor = b->d_aLor; ca.prof_off = b->d_prof_off; ca.prof_size = b->d_prof_size;
-  ca.pool = b->d_prof;
+  ca.iso_spec = w.iso_spec.p; ca.iso_out = d_iso_out;
+  ca.aDop = b->d_aDop.p; ca.aLor = b->d_aLor.p; ca.prof_off = b->d_prof_off.p; ca.prof_size = b->d_prof_size.p;
+  ca.pool = b->d_prof.p;
   ca.wn0 = b->wn_lo; ca.own_last = b->wn_lo + (double)(b->nowns - 1) * b->odwn; ca.dwn = b->dwn;
   ca.total_mode = total_mode ? 1 : 0;
   {
     PhaseTimer pt(b, "widths", s);
-    widths_kernel<<<ncell, std::max(32, niso), 0, s>>>(ca, cells, (const double *)w.spec_mass.p,
-                                                       (const double *)w.spec_radius.p,
-                                                       (const double *)w.iso_mass.p);
-    BCUDA(cudaGetLastError());
+    widths_kernel<<<ncell, std::max(32, niso), 0, s>>>(ca, cells, w.spec_mass.p, w.spec_radius.p, w.iso_mass.p);
+    CUDA_OK(cudaGetLastError());
   }
   {
     PhaseTimer pt(b, "accumulate", s);
@@ -1362,9 +1290,9 @@ static long long run_planes(BuilderState *b, const Options &o, const Molecules &
       else if (tile == 256) accumulate_kernel<256><<<dim3(ntile, nc), kAccCta, 0, s>>>(cb, cells + (size_t)c0 * niso, d_out, fast);
       else accumulate_kernel<128><<<dim3(ntile, nc), kAccCta, 0, s>>>(cb, cells + (size_t)c0 * niso, d_out, fast);
     }
-    BCUDA(cudaGetLastError());
+    CUDA_OK(cudaGetLastError());
   }
-  BCUDA(cudaStreamSynchronize(s));
+  CUDA_OK(cudaStreamSynchronize(s));
   long long ne = 0;
   for (int c = 0; c < ncell; c++) ne += total[cell_plane[c]];
   return ne;
@@ -1378,19 +1306,21 @@ static int planes_per_batch(const BuilderState *b) {
   return (int)std::max<size_t>(1, std::min<size_t>(16, std::min(by_out, by_S)));
 }
 
-static void ensure_builder(BuilderState *&b, const Options &o, const Atmosphere &a,
-                           const Molecules &m, Tli &t, const std::vector<double> &wn, cudaStream_t s) {
-  if (!b) b = new BuilderState();
+static BuilderState *ensure_builder(BuilderPtr &bp, const Options &o, const Atmosphere &a,
+                                    const Molecules &m, Tli &t, const std::vector<double> &wn, cudaStream_t s) {
+  if (!bp) bp.reset(new BuilderState());
+  BuilderState *b = bp.get();
   if (!t.present) fail("the line-by-line opacity calculation needs a TLI line list (linedb)");
   if (b->nwave == 0) setup_static(b, o, a, m, t, wn);
   build_profiles(b, o, s);
   load_lines(b, o, t, wn, s);
+  return b;
 }
 
-void builder_slice(BuilderState *&b, const Options &o, const Atmosphere &a, const Molecules &m,
+void builder_slice(BuilderPtr &bp, const Options &o, const Atmosphere &a, const Molecules &m,
                    Tli &t, const std::vector<double> &wn, cudaStream_t s, int t_begin, int t_end,
                    double *host_out) {
-  ensure_builder(b, o, a, m, t, wn, s);
+  BuilderState *b = ensure_builder(bp, o, a, m, t, wn, s);
   if (!b->grid_ready) setup_grid_temps(b, o, t);
   if (t_begin < 0 || t_end > b->ntemp || t_begin > t_end)
     fail("temperature slice [%d, %d) outside the grid of %d temperatures", t_begin, t_end, b->ntemp);
@@ -1417,20 +1347,20 @@ void builder_slice(BuilderState *&b, const Options &o, const Atmosphere &a, cons
         }
       }
     }
-    double *d_dens = b->dens.get<double>(dens.size());
-    double *d_out = b->out.get<double>((size_t)nc * plane);
-    BCUDA(cudaMemcpyAsync(d_dens, dens.data(), dens.size() * 8, cudaMemcpyHostToDevice, s));
-    BCUDA(cudaMemsetAsync(d_out, 0, (size_t)nc * plane * 8, s));
+    double *d_dens = b->dens.ensure_grow(dens.size());
+    double *d_out = b->out.ensure_grow((size_t)nc * plane);
+    CUDA_OK(cudaMemcpyAsync(d_dens, dens.data(), dens.size() * 8, cudaMemcpyHostToDevice, s));
+    CUDA_OK(cudaMemsetAsync(d_out, 0, (size_t)nc * plane * 8, s));
     b->neval += run_planes(b, o, m, t, np, pT.data(), pZ.data(), nc, cplane.data(), d_dens,
                            cout_.data(), d_out, false, s);
     auto td0 = std::chrono::steady_clock::now();
     // device [plane][layer][mol][wave] -> host [layer][t - t_begin][mol][wave]: one strided copy
     // per plane straight into the caller's buffer (fast when it is pinned, as the file writer's is)
     for (int p = 0; p < np; p++)
-      BCUDA(cudaMemcpy2DAsync(host_out + (size_t)(it0 + p - t_begin) * plane, (size_t)nt * plane * 8,
+      CUDA_OK(cudaMemcpy2DAsync(host_out + (size_t)(it0 + p - t_begin) * plane, (size_t)nt * plane * 8,
                               d_out + (size_t)p * nl * plane, plane * 8, plane * 8, nl,
                               cudaMemcpyDeviceToHost, s));
-    BCUDA(cudaStreamSynchronize(s));
+    CUDA_OK(cudaStreamSynchronize(s));
     b->phase_ms["d2h"] += std::chrono::duration<double, std::milli>(
         std::chrono::steady_clock::now() - td0).count();
   }
@@ -1439,11 +1369,11 @@ void builder_slice(BuilderState *&b, const Options &o, const Atmosphere &a, cons
 // Line-by-line forward mode: total molecular extinction (all isotopes collapsed, times the
 // species densities) of ncell (model, layer) cells at their own temperatures, written to
 // d_out + cell_out[c] (nwave doubles each).  tau.c:163-175,253-264 -> computemolext(permol=0).
-void builder_lbl_cells(BuilderState *&b, const Options &o, const Atmosphere &a, const Molecules &m,
+void builder_lbl_cells(BuilderPtr &bp, const Options &o, const Atmosphere &a, const Molecules &m,
                        Tli &t, const std::vector<double> &wn, cudaStream_t s, int ncell,
                        const double *cell_T, const double *d_cell_dens, const long long *cell_out,
                        double *d_out) {
-  ensure_builder(b, o, a, m, t, wn, s);
+  BuilderState *b = ensure_builder(bp, o, a, m, t, wn, s);
   if (b->zspline.empty()) {                 // second derivatives of Z_iso(T), makesample.c:534-544
     b->zspline.resize(b->niso);
     for (int i = 0; i < b->niso; i++) {
@@ -1474,10 +1404,10 @@ void builder_lbl_cells(BuilderState *&b, const Options &o, const Atmosphere &a, 
   }
 }
 
-void builder_run_and_write(BuilderState *&b, const Options &o, const Atmosphere &a,
+void builder_run_and_write(BuilderPtr &bp, const Options &o, const Atmosphere &a,
                            const Molecules &m, Tli &t, const std::vector<double> &wn,
                            cudaStream_t s, const std::string &path) {
-  ensure_builder(b, o, a, m, t, wn, s);
+  BuilderState *b = ensure_builder(bp, o, a, m, t, wn, s);
   if (!b->grid_ready) setup_grid_temps(b, o, t);
   OpacityGrid g;
   g.nmol = b->ngmol; g.ntemp = b->ntemp; g.nlayer = b->nlayer; g.nwave = b->nwave;
@@ -1502,7 +1432,7 @@ void builder_run_and_write(BuilderState *&b, const Options &o, const Atmosphere 
   // Streaming writer: the planes of a batch of temperatures are built, copied back and written in
   // place (file order o[layer][temp][mol][wave], opacity.c:418-421), so host memory holds one
   // batch (<= 2 GB) however large the grid is.  Rank 0 / the first slice writes the header.
-  int fd = open(path.c_str(), O_WRONLY | O_CREAT | (t0 == 0 && t1 == b->ntemp ? O_TRUNC : 0), 0644);
+  const Fd fd(path.c_str(), O_WRONLY | O_CREAT | (t0 == 0 && t1 == b->ntemp ? O_TRUNC : 0), 0644);
   if (fd < 0) fail("Opacity filename '%s' cannot be opened for writing.", path.c_str());
   const long long hdr = 4 * sizeof(long) + g.nmol * sizeof(int) + (g.ntemp + g.nlayer + g.nwave) * 8;
   // every slice writer sets the file to its final size: a stale, larger file of other dimensions
@@ -1521,16 +1451,16 @@ void builder_run_and_write(BuilderState *&b, const Options &o, const Atmosphere 
     if (pwrite(fd, h.data(), hdr, 0) != hdr) fail("short write on '%s'", path.c_str());
   }
   const int pb = planes_per_batch(b);
-  double *slab = nullptr;                                   // pinned staging for one batch
-  if (t1 > t0) BCUDA(cudaMallocHost((void **)&slab, (size_t)b->nlayer * std::min(pb, t1 - t0) * plane * 8));
+  PinnedBuf<double> slab;                                   // pinned staging for one batch
+  if (t1 > t0) slab.ensure((size_t)b->nlayer * std::min(pb, t1 - t0) * plane);
   for (int it0 = t0; it0 < t1; it0 += pb) {
     const int nt = std::min(pb, t1 - it0);
-    builder_slice(b, o, a, m, t, wn, s, it0, it0 + nt, slab);
+    builder_slice(bp, o, a, m, t, wn, s, it0, it0 + nt, slab.p);
     auto tw0 = std::chrono::steady_clock::now();
     for (int r = 0; r < b->nlayer; r++) {
       const long long off = hdr + ((long long)r * g.ntemp + it0) * (long long)plane * 8;
       const long long len = (long long)nt * plane * 8;
-      const char *src = (const char *)(slab + (size_t)r * nt * plane);
+      const char *src = (const char *)(slab.p + (size_t)r * nt * plane);
       for (long long done = 0; done < len;) {               // pwrite may be partial above 2 GB
         const ssize_t w = pwrite(fd, src + done, (size_t)std::min<long long>(len - done, 1LL << 30), off + done);
         if (w <= 0) fail("short write on '%s'", path.c_str());
@@ -1540,8 +1470,6 @@ void builder_run_and_write(BuilderState *&b, const Options &o, const Atmosphere 
     b->phase_ms["file_write"] += std::chrono::duration<double, std::milli>(
         std::chrono::steady_clock::now() - tw0).count();
   }
-  if (slab) cudaFreeHost(slab);
-  close(fd);
 }
 
 long long builder_stats(BuilderState *b, long long *nlines, long long *ngroups, long long *neval) {
@@ -1559,9 +1487,9 @@ double builder_phase_ms(BuilderState *b, const char *name) {
 }
 
 long long builder_line_bins(BuilderState *b, long long *iown_out, long long capacity) {
-  if (b->h_iown.empty() && b->d_trace && b->nlines > 0) {
+  if (b->h_iown.empty() && b->d_trace.p && b->nlines > 0) {
     b->h_iown.resize((size_t)b->nlines);
-    BCUDA(cudaMemcpy(b->h_iown.data(), b->d_trace, (size_t)b->nlines * 4, cudaMemcpyDeviceToHost));
+    CUDA_OK(cudaMemcpy(b->h_iown.data(), b->d_trace.p, (size_t)b->nlines * 4, cudaMemcpyDeviceToHost));
   }
   const long long n = (long long)b->h_iown.size();
   for (long long i = 0; i < n && i < capacity; i++) iown_out[i] = b->h_iown[i];
@@ -1579,28 +1507,12 @@ int builder_profile(BuilderState *b, int idop, int ilor, float *out, long long c
     if (capacity < n) fail("profile buffer too small (%lld needed)", n);
     const long long K = (n - 1) / b->osamp + 1;
     std::vector<float> tr((size_t)b->osamp * K);
-    BCUDA(cudaMemcpy(tr.data(), b->d_prof + b->prof_off[p], tr.size() * sizeof(float), cudaMemcpyDeviceToHost));
+    CUDA_OK(cudaMemcpy(tr.data(), b->d_prof.p + b->prof_off[p], tr.size() * sizeof(float), cudaMemcpyDeviceToHost));
     for (long long i = 0; i < n; i++) out[i] = tr[(size_t)(i % b->osamp) * K + i / b->osamp];
   }
   return 0;
 }
 
-void builder_free(BuilderState *b) {
-  if (!b) return;
-  void *ptrs[] = {b->d_wl, b->d_elow, b->d_gf, b->d_wavn, b->d_c_wavn, b->d_c_elow, b->d_c_gf,
-                  b->d_isoid, b->d_iown, b->d_idwn, b->d_inrange, b->d_gstart, b->d_giown,
-                  b->d_gidwn, b->d_giso, b->d_gwavn, b->d_trace, b->d_prof, b->d_aDop, b->d_aLor,
-                  b->d_prof_off, b->d_prof_size, b->dens.p, b->out.p};
-  for (void *p : ptrs) if (p) cudaFree(p);
-  if (b->work) {
-    PlaneWork &w = *b->work;
-    DevBuf *bufs[] = {&w.T, &w.tq, &w.facfull, &w.fac2, &w.kmax, &w.S, &w.blk, &w.total, &w.base, &w.cisobeg,
-                      &w.c_idx, &w.cell_plane, &w.cell_out, &w.cellinfo,
-                      &w.iso_spec, &w.iso_out, &w.iso_mass, &w.spec_mass, &w.spec_radius};
-    for (DevBuf *d : bufs) d->release();
-    delete b->work;
-  }
-  delete b;
-}
+void builder_free(BuilderState *b) { delete b; }
 
 }  // namespace bart

@@ -4,6 +4,8 @@
 #include <vector>
 #include <cstdio>
 #include <cstdint>
+#include <fcntl.h>
+#include <unistd.h>
 
 namespace bart {
 
@@ -30,6 +32,25 @@ constexpr double kSQRTLN2 = 0.83255461115769775635;
 void fail(const char *fmt, ...);          // records message; exits in mode 0 (reference behaviour)
 void warn(int level, const char *fmt, ...);
 extern int g_verb;
+
+// ---- file owners: closed when the owner goes, so a fail() that throws leaks no handle ----
+struct Fd {                               // open(); fd < 0 when that failed
+  int fd;
+  Fd(const char *path, int flags, mode_t mode = 0) : fd(open(path, flags, mode)) {}
+  ~Fd() { if (fd >= 0) close(fd); }
+  Fd(const Fd &) = delete;
+  Fd &operator=(const Fd &) = delete;
+  operator int() const { return fd; }
+};
+struct File {                             // fopen(); null when that failed
+  FILE *f;
+  File(const char *path, const char *mode) : f(fopen(path, mode)) {}
+  ~File() { if (f) fclose(f); }
+  File(File &&o) noexcept : f(o.f) { o.f = nullptr; }
+  File(const File &) = delete;
+  File &operator=(const File &) = delete;
+  operator FILE *() const { return f; }
+};
 
 // ---- options (reference: transit/src/argum.c:112-320 table, 372-739 handling) ----
 struct Options {

@@ -181,7 +181,7 @@ std::string rdstr(FILE *f) {
 void read_tli_header(const std::string &path, Tli &t) {
   t = Tli();
   if (path.empty()) { warn(1, "No TLI file set."); return; }
-  FILE *f = fopen(path.c_str(), "rb");
+  const File f(path.c_str(), "rb");
   if (!f) fail("Line info file '%s' is not found.", path.c_str());
   (void)rd<int32_t>(f);                                     // endianness magic
   unsigned short ver = rd<unsigned short>(f);
@@ -217,7 +217,6 @@ void read_tli_header(const std::string &path, Tli &t) {
   }
   t.data_offset = ftell(f);
   t.present = true;
-  fclose(f);
 }
 
 // Lines inside [wnlow, wnhigh], per isotope block, by the same boundary rule as the reference's
@@ -252,18 +251,28 @@ bool parallel_pread(int fd, void *dst, size_t bytes, long long off) {
   return ok;
 }
 
+namespace {
+struct Mapping {                          // read-only mmap of a whole file, unmapped when it goes
+  void *p;
+  size_t size;
+  Mapping(int fd, size_t n) : p(mmap(nullptr, n, PROT_READ, MAP_PRIVATE, fd, 0)), size(n) {}
+  ~Mapping() { if (p != MAP_FAILED) munmap(p, size); }
+  Mapping(const Mapping &) = delete;
+  Mapping &operator=(const Mapping &) = delete;
+};
+}  // namespace
+
 void map_tli_lines(const std::string &path, const Tli &t, double wnlow, double wnhigh, TliLineMap &m) {
-  int fd = open(path.c_str(), O_RDONLY);
+  const Fd fd(path.c_str(), O_RDONLY);
   if (fd < 0) fail("Data file '%s' not found.", path.c_str());
   struct stat st;
-  if (fstat(fd, &st) != 0) { close(fd); fail("Data file '%s': cannot stat.", path.c_str()); }
+  if (fstat(fd, &st) != 0) fail("Data file '%s': cannot stat.", path.c_str());
   const size_t fsize = (size_t)st.st_size;
-  void *mp = mmap(nullptr, fsize, PROT_READ, MAP_PRIVATE, fd, 0);
-  close(fd);
-  if (mp == MAP_FAILED) fail("Data file '%s': mmap failed.", path.c_str());
-  const char *base = (const char *)mp;
+  const Mapping map(fd, fsize);
+  if (map.p == MAP_FAILED) fail("Data file '%s': mmap failed.", path.c_str());
+  const char *base = (const char *)map.p;
   auto need = [&](long long off, long long bytes) {
-    if (off < 0 || bytes < 0 || (size_t)(off + bytes) > fsize) { munmap(mp, fsize); fail("TLI file: truncated"); }
+    if (off < 0 || bytes < 0 || (size_t)(off + bytes) > fsize) fail("TLI file: truncated");
   };
   long long pos = t.data_offset;
   need(pos, 12);
@@ -305,13 +314,12 @@ void map_tli_lines(const std::string &path, const Tli &t, double wnlow, double w
     m.total += nread;
     off += n;
   }
-  munmap(mp, fsize);
 }
 
 void read_tli_lines(const std::string &path, Tli &t, double wnlow, double wnhigh) {
   TliLineMap m;
   map_tli_lines(path, t, wnlow, wnhigh, m);
-  int fd = open(path.c_str(), O_RDONLY);
+  const Fd fd(path.c_str(), O_RDONLY);
   if (fd < 0) fail("Data file '%s' not found.", path.c_str());
   t.wl.assign((size_t)m.total, 0.0); t.elow.assign((size_t)m.total, 0.0); t.gf.assign((size_t)m.total, 0.0);
   t.isoid.assign((size_t)m.total, 0);
@@ -319,7 +327,7 @@ void read_tli_lines(const std::string &path, Tli &t, double wnlow, double wnhigh
     char *d = (char *)dst;
     while (bytes > 0) {
       const ssize_t got = pread(fd, d, (size_t)bytes, (off_t)off);
-      if (got <= 0) { close(fd); fail("TLI file: read failed"); }
+      if (got <= 0) fail("TLI file: read failed");
       d += got; off += got; bytes -= got;
     }
   };
@@ -333,7 +341,6 @@ void read_tli_lines(const std::string &path, Tli &t, double wnlow, double wnhigh
     rd(t.gf.data() + b0, m.gf_off + f * 8, n * 8);
     b0 += (size_t)n;
   }
-  close(fd);
 }
 
 // ---------------------------------------------------------------------------------------
@@ -378,27 +385,26 @@ void read_cia(const std::string &path, CiaTable &c) {
 // long Nmol, Ntemp, Nlayer, Nwave; int molID[Nmol]; double temp[Ntemp]; double press[Nlayer]
 // (barye); double wns[Nwave]; double o[Nlayer][Ntemp][Nmol][Nwave] (cm2/g), native endian.
 bool read_opacity_header(const std::string &path, OpacityGrid &g) {
-  FILE *f = fopen(path.c_str(), "rb");
+  const File f(path.c_str(), "rb");
   if (!f) return false;
   long dims[4];
-  if (fread(dims, sizeof(long), 4, f) != 4) { fclose(f); fail("Opacity file '%s' is truncated.", path.c_str()); }
+  if (fread(dims, sizeof(long), 4, f) != 4) fail("Opacity file '%s' is truncated.", path.c_str());
   g.nmol = dims[0]; g.ntemp = dims[1]; g.nlayer = dims[2]; g.nwave = dims[3];
   if (g.nmol <= 0 || g.ntemp <= 1 || g.nlayer <= 0 || g.nwave <= 0 || g.nmol > 1000 ||
       g.ntemp > 100000 || g.nlayer > 100000)
-    { fclose(f); fail("Opacity file '%s' has an invalid header.", path.c_str()); }
+    fail("Opacity file '%s' has an invalid header.", path.c_str());
   g.molid.resize(g.nmol); g.temp.resize(g.ntemp); g.press.resize(g.nlayer); g.wn.resize(g.nwave);
   bool ok = fread(g.molid.data(), sizeof(int), g.nmol, f) == (size_t)g.nmol &&
             fread(g.temp.data(), 8, g.ntemp, f) == (size_t)g.ntemp &&
             fread(g.press.data(), 8, g.nlayer, f) == (size_t)g.nlayer &&
             fread(g.wn.data(), 8, g.nwave, f) == (size_t)g.nwave;
   g.data_offset = ftell(f);
-  fclose(f);
   if (!ok) fail("Opacity file '%s' is truncated.", path.c_str());
   return true;
 }
 
 void write_opacity_file(const std::string &path, const OpacityGrid &g, const double *o) {
-  FILE *f = fopen(path.c_str(), "wb");
+  const File f(path.c_str(), "wb");
   if (!f) fail("Opacity filename '%s' cannot be opened for writing.", path.c_str());
   long dims[4] = {g.nmol, g.ntemp, g.nlayer, g.nwave};
   fwrite(dims, sizeof(long), 4, f);
@@ -407,8 +413,7 @@ void write_opacity_file(const std::string &path, const OpacityGrid &g, const dou
   fwrite(g.press.data(), 8, g.nlayer, f);
   fwrite(g.wn.data(), 8, g.nwave, f);
   size_t n = (size_t)g.nlayer * g.ntemp * g.nmol * g.nwave;
-  if (fwrite(o, 8, n, f) != n) { fclose(f); fail("Short write on opacity file '%s'.", path.c_str()); }
-  fclose(f);
+  if (fwrite(o, 8, n, f) != n) fail("Short write on opacity file '%s'.", path.c_str());
 }
 
 // ---------------------------------------------------------------------------------------

@@ -6,8 +6,11 @@
 // models, with no per-call allocation, no file output inside the MCMC loop (the reference's
 // printflux/printmod rewrite the spectrum file on every call, eclipse.c:355-380,
 // slantpath.c:510-555; see DESIGN.md "deviations") and no host round trips between stages.
+// Host resources are owned by the types of cuda_host.hpp (buffers, staging) and host.hpp (files):
+// a configuration's state is one Config value, released whole by reset_state.
 #include "../../include/bart_b200.h"
 #include "host.hpp"
+#include "cuda_host.hpp"
 #include "kernels.hpp"
 #include "column_math.cuh"
 #include "builder.hpp"
@@ -23,8 +26,7 @@
 #include <map>
 #include <algorithm>
 #include <functional>
-#include <unistd.h>
-#include <fcntl.h>
+#include <optional>
 #include <sys/stat.h>
 
 namespace bart {
@@ -69,38 +71,15 @@ static void info(int level, const char *fmt, ...) {
   va_end(ap);
 }
 
-#define CUDA_OK(call)                                                                      \
-  do {                                                                                     \
-    cudaError_t e_ = (call);                                                               \
-    if (e_ != cudaSuccess) fail("CUDA error %s at %s:%d (%s)", cudaGetErrorString(e_),     \
-                                __FILE__, __LINE__, #call);                                \
-  } while (0)
-
 // ---------------------------------------------------------------------------------------
 // profiling: per-kernel CUDA-event timing on the library stream
 struct KStat { long long launches = 0; double ms = 0; };
 struct PendingEv { std::string name; cudaEvent_t a, b; };
 
-template <class T> struct DevBuf {
-  T *p = nullptr;
-  size_t cap = 0;
-  void ensure(size_t n) {
-    if (n <= cap) return;
-    if (p) cudaFree(p);
-    p = nullptr; cap = 0;
-    cudaError_t e = cudaMalloc((void **)&p, n * sizeof(T));
-    if (e != cudaSuccess) fail("cudaMalloc of %zu bytes failed: %s", n * sizeof(T), cudaGetErrorString(e));
-    cap = n;
-  }
-  void release() { if (p) cudaFree(p); p = nullptr; cap = 0; }
-};
-
-struct State {
+// Everything one transit_init configuration owns; free_memory and the next transit_init drop it
+// whole (reset_state).
+struct Config {
   bool init = false;
-  int device = -1;
-  cudaStream_t stream = nullptr;          // compute (and default copy) stream
-  cudaStream_t s_h2d = nullptr, s_d2h = nullptr;   // copy streams of the pipelined host path
-  std::vector<cudaEvent_t> ev_pool;                // its events (created once)
   Options opt;
   Atmosphere atm;
   Molecules mol;
@@ -117,10 +96,8 @@ struct State {
   // batch buffers
   DevBuf<double> d_prof, d_tabs, d_spec, d_wts, d_tau, d_band, d_ext, d_flush;
   DevBuf<int> d_status, d_status_col, d_last;
-  int *h_status = nullptr;                 // pinned staging for per-model status
-  size_t h_status_cap = 0;
-  double *h_lean = nullptr;                // pinned staging of the small-call path (bart_run_batch)
-  size_t h_lean_cap = 0;                   // doubles
+  PinnedBuf<int> h_status;                 // pinned staging for per-model status
+  PinnedBuf<double> h_lean;                // pinned staging of the small-call path (bart_run_batch)
   DevBuf<double> d_kr0, d_kcloud, d_klogext;
   DevBuf<int> d_kflag;
   int knob_models = 0;
@@ -133,9 +110,47 @@ struct State {
   // energy-balance rejection (BARTfunc.py:366-383), applied wherever band fluxes are produced
   bool eb_on = false;
   double eb_ein = 0.0, eb_scale = 0.0;
+  int last_batch = 0;
+  BuilderPtr builder;
+  // line-by-line forward mode (no opacity file)
+  bool lbl = false;
+  DevBuf<double> d_lbl_ext, d_lbl_dens;
+  std::vector<double> h_lbl_T;
+  std::vector<int> h_lbl_status;
+  // input converter (retrieval.hpp)
+  ConvConfig conv{};
+  DevBuf<double> d_cpress, d_cbase, d_cratio, d_cparams, d_csmooth, d_cnodex;
+  DevBuf<int> d_cnodeseg;
+  DevBuf<int> d_cstatus;
+  const int *pre_status = nullptr;         // converter rejections of the batch being launched
+  // DE-MC loop: `mc` holds views of these
+  McmcDev mc{};
+  bool mc_ready = false;
+  int mc_lo = 0, mc_hi = 0, mc_pad = 0;
+  struct {
+    DevBuf<double> pmin, pmax, prior, priorlow, data, uncert, params, nextp, currchisq, nextchisq, c2,
+        bestp, bestchisq, bestmodel, numaccept, support, unif, ugamma, allparams, zbest;
+    DevBuf<int> outbounds, outflag, iter, r1, r2, zsize, noproj, slot;
+  } mcb;
+  DevBuf<double> d_mcband, d_mcgather, d_mccur, d_mcallm;
+  cudaGraphExec_t mc_graph = nullptr;      // destroyed by reset_state
+  // snooker walk: sample history Z
+  DevBuf<double> d_Z, d_Zchisq, d_snk_usn;
+  DevBuf<int> d_snk_idx, d_snk_off;
+  int mc_zsize = 0;                        // host mirror of the device row counter
+  size_t mc_zcap = 0;                      // rows allocated
+  std::vector<double> mc_ztemplate;        // [nchains][npars] what an unfilled row holds
+};
+
+// The process: the device, its streams, the communicator and peer window, profiling and debug
+// switches outlive configurations.
+struct State : Config {
+  int device = -1;
+  cudaStream_t stream = nullptr;          // compute (and default copy) stream
+  cudaStream_t s_h2d = nullptr, s_d2h = nullptr;   // copy streams of the pipelined host path
+  std::vector<cudaEvent_t> ev_pool;                // its events (created once)
   // debug
   bool keep = false;
-  int last_batch = 0;
   int use_tma = 1;
   // profiling
   bool profile = false;
@@ -155,35 +170,11 @@ struct State {
   PeerOut pw{};
   unsigned long long *pw_gen = nullptr, *pw_flags = nullptr;
   int *pw_err = nullptr;
-  // builder
-  BuilderState *builder = nullptr;
-  // line-by-line forward mode (no opacity file)
-  bool lbl = false;
-  DevBuf<double> d_lbl_ext, d_lbl_dens;
-  std::vector<double> h_lbl_T;
-  std::vector<int> h_lbl_status;
-  // input converter (retrieval.hpp)
-  ConvConfig conv{};
-  DevBuf<double> d_cpress, d_cbase, d_cratio, d_cparams, d_csmooth, d_cnodex;
-  DevBuf<int> d_cnodeseg;
-  DevBuf<int> d_cstatus;
-  const int *pre_status = nullptr;         // converter rejections of the batch being launched
-  // DE-MC loop
-  McmcDev mc{};
-  bool mc_ready = false;
-  int mc_lo = 0, mc_hi = 0, mc_pad = 0;
-  DevBuf<double> d_mcd[20];
-  DevBuf<int> d_mci[8];
-  DevBuf<double> d_mcband, d_mcgather, d_mccur, d_mcallm;
-  cudaGraphExec_t mc_graph = nullptr;
-  // snooker walk: sample history Z
-  DevBuf<double> d_Z, d_Zchisq, d_snk_usn;
-  DevBuf<int> d_snk_idx, d_snk_off;
-  int mc_zsize = 0;                        // host mirror of the device row counter
-  size_t mc_zcap = 0;                      // rows allocated
-  std::vector<double> mc_ztemplate;        // [nchains][npars] what an unfilled row holds
 };
-static State G;
+// Never destroyed: a destructor would run at exit() (error mode 0, or the normal end of the
+// process) and call cudaFree while the CUDA runtime is being torn down.  The process's device
+// memory goes with the process.
+static State &G = *new State;
 
 struct KernelScope {
   const char *name;
@@ -258,9 +249,11 @@ static void ensure_device() {
   G.use_tma = (t && atoi(t)) ? 0 : 1;
 }
 
-template <class T> static void upload(DevBuf<T> &b, const std::vector<T> &v) {
-  b.ensure(v.size() ? v.size() : 1);
-  if (!v.empty()) CUDA_OK(cudaMemcpy(b.p, v.data(), v.size() * sizeof(T), cudaMemcpyHostToDevice));
+// n elements of src -> b (at least one element), queued on the library stream
+template <class T> static const T *upload_queued(DevBuf<T> &b, const T *src, size_t n) {
+  b.ensure(std::max<size_t>(n, 1));
+  if (n) CUDA_OK(cudaMemcpyAsync(b.p, src, n * sizeof(T), cudaMemcpyHostToDevice, G.stream));
+  return b.p;
 }
 
 // ---------------------------------------------------------------------------------------
@@ -335,41 +328,27 @@ static void load_grid_to_device(const std::string &path) {
   const size_t cell_in = (size_t)g.nmol * g.nwave, cell_out = (size_t)gms * g.nwave;
   G.d_grid.ensure(ncell * cell_out + (size_t)kEclPad * gms);   // + padding (kernels.hpp kEclPad)
   CUDA_OK(cudaMemsetAsync(G.d_grid.p + ncell * cell_out, 0, (size_t)kEclPad * gms * sizeof(double), G.stream));
-  const int fd = open(path.c_str(), O_RDONLY);
+  const Fd fd(path.c_str(), O_RDONLY);
   if (fd < 0) fail("Opening opacity file '%s' failed.", path.c_str());
   long long fpos = g.data_offset;
-  // stream whole (layer, temperature) cells through two pinned staging buffers (files reach tens
-  // of GB at high resolution); each chunk is re-laid out on the device while the next is read
-  const size_t cells_per_chunk = std::max<size_t>(1, (size_t)(64u << 20) / (cell_in * 8));
-  const size_t chunk = cells_per_chunk * cell_in * 8;
-  void *stage[2] = {nullptr, nullptr};
-  DevBuf<double> d_stage[2];
-  cudaEvent_t done_ev[2];
-  for (int i = 0; i < 2; i++) {
-    CUDA_OK(cudaMallocHost(&stage[i], chunk));
-    d_stage[i].ensure(cells_per_chunk * cell_in);
-    CUDA_OK(cudaEventCreate(&done_ev[i]));
-  }
-  size_t cell = 0;
-  int which = 0;
-  bool bad = false;
-  while (cell < ncell && !bad) {
+  // stream whole (layer, temperature) cells through the pinned staging (files reach tens of GB at
+  // high resolution); each chunk is re-laid out on the device while the next is read
+  const size_t cells_per_chunk = std::max<size_t>(1, PinnedStage::kBytes / (cell_in * 8));
+  DevBuf<double> d_stage[2] = {DevBuf<double>(cells_per_chunk * cell_in), DevBuf<double>(cells_per_chunk * cell_in)};
+  PinnedStage st(cells_per_chunk * cell_in * 8);
+  for (size_t cell = 0; cell < ncell;) {
     const size_t nc = std::min(cells_per_chunk, ncell - cell);
     const size_t want = nc * cell_in * 8;
-    CUDA_OK(cudaEventSynchronize(done_ev[which]));           // staging buffer free again
-    if (!parallel_pread(fd, stage[which], want, fpos)) { bad = true; break; }
+    double *d_in = d_stage[st.next()].p;
+    if (!st.put(fd, fpos, want, d_in, G.stream, [&] {
+          launch_grid_relayout(d_in, G.d_grid.p + cell * cell_out, (int)nc, (int)g.nmol, gms, (int)g.nwave,
+                               G.stream);
+        }))
+      fail("Opacity file '%s' is truncated.", path.c_str());
     fpos += (long long)want;
-    CUDA_OK(cudaMemcpyAsync(d_stage[which].p, stage[which], want, cudaMemcpyHostToDevice, G.stream));
-    launch_grid_relayout(d_stage[which].p, G.d_grid.p + cell * cell_out, (int)nc, (int)g.nmol, gms,
-                         (int)g.nwave, G.stream);
-    CUDA_OK(cudaEventRecord(done_ev[which], G.stream));
     cell += nc;
-    which ^= 1;
   }
   cudaStreamSynchronize(G.stream);
-  for (int i = 0; i < 2; i++) { cudaFreeHost(stage[i]); d_stage[i].release(); cudaEventDestroy(done_ev[i]); }
-  close(fd);
-  if (bad) fail("Opacity file '%s' is truncated.", path.c_str());
   check_launch("grid_relayout");
 }
 
@@ -389,31 +368,8 @@ static void finish_grid_config() {
 }
 
 static void reset_state() {
-  G.d_grid.release(); G.d_gtemp.release(); G.d_wn.release(); G.d_press.release();
-  G.d_mass.release(); G.d_pol.release();
-  for (int f = 0; f < kMaxCia; f++) { G.d_ciaPQ[f].release(); G.d_ciaT[f].release(); }
-  G.d_prof.release(); G.d_tabs.release(); G.d_spec.release(); G.d_wts.release(); G.d_tau.release();
-  G.d_band.release(); G.d_ext.release(); G.d_status.release(); G.d_status_col.release();
-  G.d_last.release(); G.d_kr0.release(); G.d_kcloud.release(); G.d_klogext.release(); G.d_kflag.release();
-  G.d_fstart.release(); G.d_fcount.release(); G.d_foffset.release(); G.d_fweight.release();
-  G.d_fstar.release(); G.d_flush.release();
-  if (G.builder) { builder_free(G.builder); G.builder = nullptr; }
-  G.d_lbl_ext.release(); G.d_lbl_dens.release(); G.lbl = false;
-  G.d_cpress.release(); G.d_cbase.release(); G.d_cratio.release(); G.d_cparams.release();
-  G.d_csmooth.release(); G.d_cnodex.release(); G.d_cnodeseg.release();
-  G.d_cstatus.release(); G.d_mcband.release(); G.d_mcgather.release();
-  G.d_mccur.release(); G.d_mcallm.release();
-  for (auto &b : G.d_mcd) b.release();
-  for (auto &b : G.d_mci) b.release();
-  G.d_snk_usn.release(); G.d_snk_idx.release(); G.d_snk_off.release();
-  G.d_Z.release(); G.d_Zchisq.release(); G.mc_zsize = 0; G.mc_zcap = 0; G.mc_ztemplate.clear();
-  if (G.mc_graph) { cudaGraphExecDestroy(G.mc_graph); G.mc_graph = nullptr; }
-  if (G.h_lean) { cudaFreeHost(G.h_lean); G.h_lean = nullptr; G.h_lean_cap = 0; }
-  if (G.h_status) { cudaFreeHost(G.h_status); G.h_status = nullptr; G.h_status_cap = 0; }
-  G.conv = ConvConfig(); G.mc = McmcDev(); G.mc_ready = false; G.pre_status = nullptr;
-  G.nfilters = 0; G.knob_models = 0; G.last_batch = 0; G.eb_on = false;
-  G.cia.clear(); G.wn.clear(); G.angles.clear();
-  G.init = false;
+  if (G.mc_graph) cudaGraphExecDestroy(G.mc_graph);
+  static_cast<Config &>(G) = Config();
 }
 
 static void do_init(int argc, char **argv) {
@@ -987,16 +943,16 @@ static void write_savefiles(const double *re_input, int n_in) {
   if (bart_extinction_batch(re_input, 1, n_in, cia.data(), 2) != 0) return;
   const char *fmt = "%-20.10g";
   auto open_dump = [](const char *name, const char *header) {
-    FILE *f = fopen(name, "w");
+    File f(name, "w");
     if (!f) fail("cannot open '%s' for writing (savefiles)", name);
     fprintf(f, "\n");
     fputs(header, f);
     return f;
   };
   // per-wavenumber rows [wn][rad], rad[0] = bottom: total, cloud, scattering (save1Darray)
-  FILE *ft = open_dump("total_extion.dat", "# 2D total extinction\n# er [wn][rad]; wn[0]=min(wn), row[0]=bottom (max(p))\n");
-  FILE *fc = open_dump("cloud_extion.dat", "# 2D cloud extinction\n# e_c [wn][rad]; wn[0]=min(wn), row[0]=bottom (max(p))\n");
-  FILE *fs = open_dump("scatt_extion.dat", "# 2D scatt extinction\n# e_s [wn][rad]; wn[0]=min(wn), row[0]=bottom (max(p))\n");
+  const File ft = open_dump("total_extion.dat", "# 2D total extinction\n# er [wn][rad]; wn[0]=min(wn), row[0]=bottom (max(p))\n");
+  const File fc = open_dump("cloud_extion.dat", "# 2D cloud extinction\n# e_c [wn][rad]; wn[0]=min(wn), row[0]=bottom (max(p))\n");
+  const File fs = open_dump("scatt_extion.dat", "# 2D scatt extinction\n# e_s [wn][rad]; wn[0]=min(wn), row[0]=bottom (max(p))\n");
   for (int w = 0; w < nw; w++) {
     const double wn = G.wn[w], wn4 = (wn * wn) * (wn * wn);
     FILE *fl[3] = {ft, fc, fs};
@@ -1012,10 +968,9 @@ static void write_savefiles(const double *re_input, int n_in) {
       fprintf(fl[k], "\n");
     }
   }
-  fclose(ft); fclose(fc); fclose(fs);
   // tau.dat [wn][rad], rad[0] = top; CIA.dat [wn][rad], rad[0] = bottom (print2dArrayDouble)
-  FILE *f = open_dump("tau.dat", "# 2D optical depth\n# tau [wn][rad]; wn[0]=min(wn); rad[0]=top (min(p))\n\n");
-  FILE *g = open_dump("CIA.dat", "# 2D CIA extinction\n# e_cs [wn][rad]; wn[0]=min(wn); row[0]=bottom (max(p))\n\n");
+  const File f = open_dump("tau.dat", "# 2D optical depth\n# tau [wn][rad]; wn[0]=min(wn); rad[0]=top (min(p))\n\n");
+  const File g = open_dump("CIA.dat", "# 2D CIA extinction\n# e_cs [wn][rad]; wn[0]=min(wn); row[0]=bottom (max(p))\n\n");
   for (int w = 0; w < nw; w++) {
     FILE *fl[2] = {f, g};
     for (int k = 0; k < 2; k++) {
@@ -1026,15 +981,13 @@ static void write_savefiles(const double *re_input, int n_in) {
       fprintf(fl[k], "\n\n");
     }
   }
-  fclose(f); fclose(g);
   // mol_extion.dat [rad][wn], rad[0] = bottom (savemolExtion)
-  f = open_dump("mol_extion.dat", "# mol-line extinction\n# e [rad][wn]; rad[0]=bottom (max(p)); wn[0]=min(wn)\n\n");
+  const File m = open_dump("mol_extion.dat", "# mol-line extinction\n# e [rad][wn]; rad[0]=bottom (max(p)); wn[0]=min(wn)\n\n");
   for (int r = 0; r < nl; r++) {
-    fprintf(f, "radius: %-20.10g\n", tab[(size_t)(nl - 1 - r) * nf + TabLayout::RAD]);
-    for (int w = 0; w < nw; w++) fprintf(f, fmt, mol[(size_t)r * nw + w]);
-    fprintf(f, "\n\n");
+    fprintf(m, "radius: %-20.10g\n", tab[(size_t)(nl - 1 - r) * nf + TabLayout::RAD]);
+    for (int w = 0; w < nw; w++) fprintf(m, fmt, mol[(size_t)r * nw + w]);
+    fprintf(m, "\n\n");
   }
-  fclose(f);
 }
 
 void run_transit(double *re_input, int transint, double *transit_out, int transit_out_size) {
@@ -1160,13 +1113,7 @@ int bart_run_batch(const double *profiles, int nmodels, int n_in, double *spectr
   const size_t lean_doubles = (size_t)nmodels * ((size_t)n_in + nw + 1);
   static const bool lean_on = [] { const char *e = getenv("BART_LEAN"); return !e || atoi(e) != 0; }();
   if (lean_on && lean_doubles * 8 <= (1u << 20)) {
-    if (lean_doubles > G.h_lean_cap) {
-      if (G.h_lean) cudaFreeHost(G.h_lean);
-      G.h_lean = nullptr; G.h_lean_cap = 0;
-      CUDA_OK(cudaMallocHost((void **)&G.h_lean, lean_doubles * 8));
-      G.h_lean_cap = lean_doubles;
-    }
-    double *h_in = G.h_lean, *h_out = h_in + (size_t)nmodels * n_in;
+    double *h_in = G.h_lean.ensure(lean_doubles), *h_out = h_in + (size_t)nmodels * n_in;
     int *h_st = reinterpret_cast<int *>(h_out + (size_t)nmodels * nw);
     memcpy(h_in, profiles, (size_t)nmodels * n_in * 8);
     CUDA_OK(cudaMemcpyAsync(G.d_prof.p, h_in, (size_t)nmodels * n_in * 8, cudaMemcpyHostToDevice, G.stream));
@@ -1227,18 +1174,13 @@ int bart_run_batch(const double *profiles, int nmodels, int n_in, double *spectr
     off += cnt;
   }
   if (status) {      // one small copy through pinned staging (a pageable target would block the loop)
-    if ((size_t)nmodels > G.h_status_cap) {
-      if (G.h_status) cudaFreeHost(G.h_status);
-      CUDA_OK(cudaMallocHost((void **)&G.h_status, (size_t)nmodels * sizeof(int)));
-      G.h_status_cap = nmodels;
-    }
-    CUDA_OK(cudaMemcpyAsync(G.h_status, G.d_status.p, nmodels * sizeof(int), cudaMemcpyDeviceToHost, G.s_d2h));
+    CUDA_OK(cudaMemcpyAsync(G.h_status.ensure(nmodels), G.d_status.p, nmodels * sizeof(int), cudaMemcpyDeviceToHost, G.s_d2h));
   }
   G.last_batch = nmodels;
   cudaError_t e = cudaStreamSynchronize(G.s_d2h);
   if (e != cudaSuccess) fail("CUDA execution failed: %s", cudaGetErrorString(e));
   finish_stream();
-  if (status) memcpy(status, G.h_status, nmodels * sizeof(int));
+  if (status) memcpy(status, G.h_status.p, nmodels * sizeof(int));
   return 0;
   API_END_INT
 }
@@ -1581,16 +1523,14 @@ static void setup_peer_window() {
   Msg mine; memset(&mine, 0, sizeof(mine));
   if (ok && cudaIpcGetMemHandle(&mine.h, G.pw_base) != cudaSuccess) { cudaGetLastError(); ok = 0; }
   mine.ok = ok;
-  Msg *d_msg = nullptr, *d_all = nullptr;
-  CUDA_OK(cudaMalloc((void **)&d_msg, sizeof(Msg)));
-  CUDA_OK(cudaMalloc((void **)&d_all, sizeof(Msg) * G.world));
+  DevBuf<Msg> d_msg(1), d_all(G.world);
   std::vector<Msg> all(G.world);
   auto exchange = [&]() {
-    CUDA_OK(cudaMemcpy(d_msg, &mine, sizeof(Msg), cudaMemcpyHostToDevice));
-    int rc = ((fn_allgather)nccl_sym("ncclAllGather"))(d_msg, d_all, sizeof(Msg), 0 /*ncclInt8*/, G.nccl_comm, G.stream);
+    CUDA_OK(cudaMemcpy(d_msg.p, &mine, sizeof(Msg), cudaMemcpyHostToDevice));
+    int rc = ((fn_allgather)nccl_sym("ncclAllGather"))(d_msg.p, d_all.p, sizeof(Msg), 0 /*ncclInt8*/, G.nccl_comm, G.stream);
     if (rc != 0) fail("ncclAllGather failed: %s", ((fn_errstr)nccl_sym("ncclGetErrorString"))(rc));
     CUDA_OK(cudaStreamSynchronize(G.stream));
-    CUDA_OK(cudaMemcpy(all.data(), d_all, sizeof(Msg) * G.world, cudaMemcpyDeviceToHost));
+    CUDA_OK(cudaMemcpy(all.data(), d_all.p, sizeof(Msg) * G.world, cudaMemcpyDeviceToHost));
   };
   exchange();
   for (int r = 0; r < G.world; r++) ok = ok && all[r].ok;
@@ -1604,7 +1544,6 @@ static void setup_peer_window() {
   mine.ok = ok;
   exchange();                                                 // everyone mapped everyone?
   for (int r = 0; r < G.world; r++) ok = ok && all[r].ok;
-  cudaFree(d_msg); cudaFree(d_all);
   if (!ok) { warn(1, "peer windows unavailable (CUDA IPC); using ncclAllGather\n"); return; }
   G.pw_cap = cap;
   G.pw_flags = (unsigned long long *)(G.pw_base + win_bytes);
@@ -1927,29 +1866,30 @@ int bart_mcmc_init(int nchains, int npars, const double *params, const double *p
   }
   if (mc.nfree < 1) fail("no free parameters");
   mc.gamma = fgamma * 2.4 / sqrt(2.0 * mc.nfree);
-  auto up = [&](int slot, const double *src, size_t n) -> double * {
+  auto up = [&](DevBuf<double> &b, const double *src, size_t n) -> double * {
     std::vector<double> v(n, 0.0);
     if (src) v.assign(src, src + n);
-    upload(G.d_mcd[slot], v);
-    return G.d_mcd[slot].p;
+    upload(b, v);
+    return b.p;
   };
-  mc.pmin = up(0, pmin, npars); mc.pmax = up(1, pmax, npars);
-  mc.prior = up(2, prior, npars); mc.priorlow = up(3, priorlow, npars);
-  mc.data = up(4, data, ndata); mc.uncert = up(5, uncert, ndata);
+  auto &mb = G.mcb;
+  mc.pmin = up(mb.pmin, pmin, npars); mc.pmax = up(mb.pmax, pmax, npars);
+  mc.prior = up(mb.prior, prior, npars); mc.priorlow = up(mb.priorlow, priorlow, npars);
+  mc.data = up(mb.data, data, ndata); mc.uncert = up(mb.uncert, uncert, ndata);
   std::vector<double> p0(params, params + (size_t)nchains * npars);
   for (int c = 0; c < nchains; c++)
     for (int s = 0; s < mc.nshare; s++)
       p0[(size_t)c * npars + mc.share_dst[s]] = p0[(size_t)c * npars + mc.share_src[s]];
-  mc.params = up(6, p0.data(), p0.size());
-  mc.nextp = up(7, p0.data(), p0.size());
-  mc.currchisq = up(8, nullptr, nchains); mc.nextchisq = up(9, nullptr, nchains);
-  mc.c2 = up(10, nullptr, nchains); mc.bestp = up(11, nullptr, npars);
-  mc.bestchisq = up(12, nullptr, 1); mc.bestmodel = up(13, nullptr, ndata);
-  mc.numaccept = up(14, nullptr, nchains);
+  mc.params = up(mb.params, p0.data(), p0.size());
+  mc.nextp = up(mb.nextp, p0.data(), p0.size());
+  mc.currchisq = up(mb.currchisq, nullptr, nchains); mc.nextchisq = up(mb.nextchisq, nullptr, nchains);
+  mc.c2 = up(mb.c2, nullptr, nchains); mc.bestp = up(mb.bestp, nullptr, npars);
+  mc.bestchisq = up(mb.bestchisq, nullptr, 1); mc.bestmodel = up(mb.bestmodel, nullptr, ndata);
+  mc.numaccept = up(mb.numaccept, nullptr, nchains);
   std::vector<int> zi((size_t)nchains * mc.nfree, 0);
-  upload(G.d_mci[0], zi); mc.outbounds = G.d_mci[0].p;
-  zi.assign(nchains, 0); upload(G.d_mci[1], zi); mc.outflag = G.d_mci[1].p;
-  zi.assign(1, 0); upload(G.d_mci[2], zi); mc.iter = G.d_mci[2].p;
+  upload(mb.outbounds, zi); mc.outbounds = mb.outbounds.p;
+  zi.assign(nchains, 0); upload(mb.outflag, zi); mc.outflag = mb.outflag.p;
+  zi.assign(1, 0); upload(mb.iter, zi); mc.iter = mb.iter.p;
   G.mc = mc;
   G.mc_ztemplate = p0;
   G.mc_zsize = 0;
@@ -2004,26 +1944,12 @@ int bart_mcmc_run(int niter, const double *support, const int *r1, const int *r2
     if (r1[k] < 0 || r1[k] >= nc || r2[k] < 0 || r2[k] >= nc) fail("chain index out of range in r1/r2");
   mc.nold += mc.chainsize;               // iterations of earlier calls count towards burn-in
   mc.chainsize = niter;
-  auto upd = [&](DevBuf<double> &b, const double *src, size_t n) {
-    b.ensure(n);
-    CUDA_OK(cudaMemcpyAsync(b.p, src, n * 8, cudaMemcpyHostToDevice, G.stream));
-    return (const double *)b.p;
-  };
-  auto upi = [&](DevBuf<int> &b, const int *src, size_t n) {
-    b.ensure(n);
-    CUDA_OK(cudaMemcpyAsync(b.p, src, n * 4, cudaMemcpyHostToDevice, G.stream));
-    return (const int *)b.p;
-  };
-  DevBuf<double> &d_support = G.d_mcd[15], &d_unif = G.d_mcd[16], &d_ugamma = G.d_mcd[17],
-                 &d_trace = G.d_mcd[18];
-  DevBuf<int> &d_r1 = G.d_mci[3], &d_r2 = G.d_mci[4];
-  mc.support = upd(d_support, support, (size_t)niter * nc * mc.nfree);
-  mc.unif = upd(d_unif, unif, (size_t)niter * nc);
-  mc.ugamma = upd(d_ugamma, ugamma, (size_t)niter * nc);
-  mc.r1 = upi(d_r1, r1, (size_t)nc * niter);
-  mc.r2 = upi(d_r2, r2, (size_t)nc * niter);
-  d_trace.ensure((size_t)nc * mc.nfree * niter);
-  mc.allparams = d_trace.p;
+  mc.support = upload_queued(G.mcb.support, support, (size_t)niter * nc * mc.nfree);
+  mc.unif = upload_queued(G.mcb.unif, unif, (size_t)niter * nc);
+  mc.ugamma = upload_queued(G.mcb.ugamma, ugamma, (size_t)niter * nc);
+  mc.r1 = upload_queued(G.mcb.r1, r1, (size_t)nc * niter);
+  mc.r2 = upload_queued(G.mcb.r2, r2, (size_t)nc * niter);
+  mc.allparams = G.mcb.allparams.ensure((size_t)nc * mc.nfree * niter);
   G.d_mcallm.ensure((size_t)nc * mc.ndata * niter);
   mc.allmodel = G.d_mcallm.p;
   mc.walk = 0;
@@ -2053,8 +1979,7 @@ static void snooker_reserve_rows(size_t rows) {
     CUDA_OK(cudaMemcpyAsync(nc.p, G.d_Zchisq.p, (size_t)G.mc_zsize * mc.nchains * 8, cudaMemcpyDeviceToDevice, G.stream));
   }
   CUDA_OK(cudaStreamSynchronize(G.stream));
-  G.d_Z.release(); G.d_Zchisq.release();
-  G.d_Z = nz; G.d_Zchisq = nc;
+  G.d_Z = std::move(nz); G.d_Zchisq = std::move(nc);
   G.mc_zcap = rows;
   mc.Z = G.d_Z.p; mc.Zchisq = G.d_Zchisq.p;
 }
@@ -2090,11 +2015,11 @@ int bart_mcmc_snooker_init(int hsize, int thinning, const double *z0) {
     }
   CUDA_OK(cudaMemcpyAsync(mc.Z, rows.data(), rows.size() * 8, cudaMemcpyHostToDevice, G.stream));
   std::vector<int> zi(1, hsize);
-  upload(G.d_mci[5], zi); mc.zsize = G.d_mci[5].p;
+  upload(G.mcb.zsize, zi); mc.zsize = G.mcb.zsize.p;
   zi.assign(nc, 0);
-  upload(G.d_mci[6], zi); mc.noproj = G.d_mci[6].p;
-  upload(G.d_mci[7], zi); mc.slot = G.d_mci[7].p;
-  G.d_mcd[19].ensure(1 + np + mc.ndata); mc.zbest = G.d_mcd[19].p;
+  upload(G.mcb.noproj, zi); mc.noproj = G.mcb.noproj.p;
+  upload(G.mcb.slot, zi); mc.slot = G.mcb.slot.p;
+  mc.zbest = G.mcb.zbest.ensure(1 + np + mc.ndata);
   mc.hsize = hsize; mc.thinning = thinning; mc.walk = 1;
   ensure_params_buffers(G.mc_hi - G.mc_lo);
   ModelMap mp{G.world, nc / G.world, nc % G.world, G.mc_pad};
@@ -2150,33 +2075,20 @@ int bart_mcmc_run_snooker(int niter, const double *support, const int *i1, const
   }
   mc.nold += mc.chainsize;
   mc.chainsize = niter;
-  auto upd = [&](DevBuf<double> &b, const double *src, size_t n) {
-    b.ensure(std::max<size_t>(n, 1));
-    if (n) CUDA_OK(cudaMemcpyAsync(b.p, src, n * 8, cudaMemcpyHostToDevice, G.stream));
-    return (const double *)b.p;
-  };
-  auto upi = [&](DevBuf<int> &b, const int *src, size_t n) {
-    b.ensure(n);
-    CUDA_OK(cudaMemcpyAsync(b.p, src, n * 4, cudaMemcpyHostToDevice, G.stream));
-    return (const int *)b.p;
-  };
   // i1, i2, iz, ic packed in one buffer; usn_offset in another
-  DevBuf<int> &d_idx = G.d_snk_idx, &d_off = G.d_snk_off;
-  DevBuf<double> &d_usn = G.d_snk_usn;
   const size_t n1 = (size_t)niter * nc;
   std::vector<int> packed(4 * n1);
   std::copy(i1, i1 + n1, packed.begin()); std::copy(i2, i2 + n1, packed.begin() + n1);
   std::copy(iz, iz + n1, packed.begin() + 2 * n1); std::copy(ic, ic + n1, packed.begin() + 3 * n1);
-  const int *pk = upi(d_idx, packed.data(), packed.size());
+  const int *pk = upload_queued(G.d_snk_idx, packed.data(), packed.size());
   CUDA_OK(cudaStreamSynchronize(G.stream));
   mc.i1 = pk; mc.i2 = pk + n1; mc.iz = pk + 2 * n1; mc.ic = pk + 3 * n1;
-  mc.usn_off = upi(d_off, usn_offset, (size_t)niter + 1);
-  mc.usn = upd(d_usn, usnooker, (size_t)usn_offset[niter] * mc.nfree);
-  mc.support = upd(G.d_mcd[15], support, n1 * mc.nfree);
-  mc.unif = upd(G.d_mcd[16], unif, n1);
-  mc.ugamma = upd(G.d_mcd[17], ugamma, n1);
-  G.d_mcd[18].ensure((size_t)nc * mc.nfree * niter);
-  mc.allparams = G.d_mcd[18].p;
+  mc.usn_off = upload_queued(G.d_snk_off, usn_offset, (size_t)niter + 1);
+  mc.usn = upload_queued(G.d_snk_usn, usnooker, (size_t)usn_offset[niter] * mc.nfree);
+  mc.support = upload_queued(G.mcb.support, support, n1 * mc.nfree);
+  mc.unif = upload_queued(G.mcb.unif, unif, n1);
+  mc.ugamma = upload_queued(G.mcb.ugamma, ugamma, n1);
+  mc.allparams = G.mcb.allparams.ensure((size_t)nc * mc.nfree * niter);
   G.d_mcallm.ensure((size_t)nc * mc.ndata * niter);
   mc.allmodel = G.d_mcallm.p;
   mc.walk = 1;
@@ -2245,19 +2157,22 @@ int bart_cli_run(void) {
     for (int i = 0; i < nl; i++) in[(size_t)(j + 1) * nl + i] = G.atm.q[(size_t)j * nl + i];
   // main() runs do_transit on the atmosphere as read: the file's own radius column, no hydrostatic
   // recomputation (that is reloadatm's, i.e. run_transit's, job)
-  DevBuf<double> d_rad;
-  upload(d_rad, G.atm.radius);
-  G.knobs.radius_file = d_rad.p;
-  run_transit(in.data(), (int)in.size(), out.data(), nw);
-  G.knobs.radius_file = nullptr;
-  d_rad.release();
+  {
+    DevBuf<double> d_rad;
+    upload(d_rad, G.atm.radius);
+    G.knobs.radius_file = d_rad.p;
+    run_transit(in.data(), (int)in.size(), out.data(), nw);
+    G.knobs.radius_file = nullptr;
+  }
   if (bart_error_pending()) return -1;
   // printflux / printmod text format: eclipse.c:355-380, slantpath.c:510-555
   FILE *f = stdout;
+  std::optional<File> file;
   const std::string &name = G.opt.outspec;
   if (!name.empty() && name != "-") {
-    f = fopen(name.c_str(), "w");
-    if (!f) fail("Cannot open output file '%s'", name.c_str());
+    file.emplace(name.c_str(), "w");
+    if (!*file) fail("Cannot open output file '%s'", name.c_str());
+    f = *file;
   }
   const double wfct = 1.0;                       // wns.fct is always 1 (makesample.c:367)
   if (G.dc.eclipse) {
@@ -2267,7 +2182,6 @@ int bart_cli_run(void) {
     fprintf(f, "#wvl [um]        modulation\n");
     for (int w = 0; w < nw; w++) fprintf(f, "%-17.9g%-18.9g\n", 1e4 / (G.wn[w] / wfct), out[w]);
   }
-  if (f != stdout) fclose(f);
   return 0;
   API_END_INT
 }
@@ -2282,24 +2196,24 @@ int bart_build_opacity_slice(int t_begin, int t_end, double *host_out) {
   API_END_INT
 }
 
-double bart_builder_phase_ms(const char *name) { return builder_phase_ms(G.builder, name); }
+double bart_builder_phase_ms(const char *name) { return builder_phase_ms(G.builder.get(), name); }
 
 long long bart_builder_stats(long long *nlines, long long *ngroups, long long *neval) {
   if (!G.builder) return -1;
-  return builder_stats(G.builder, nlines, ngroups, neval);
+  return builder_stats(G.builder.get(), nlines, ngroups, neval);
 }
 
 long long bart_line_bins(long long *iown_out, long long capacity) {
   API_BEGIN
   if (!G.builder) fail("the opacity-grid builder has not run in this process");
-  return builder_line_bins(G.builder, iown_out, capacity);
+  return builder_line_bins(G.builder.get(), iown_out, capacity);
   API_END_INT
 }
 
 int bart_voigt_profile(int idop, int ilor, float *out, long long capacity, long long *halfsize) {
   API_BEGIN
   if (!G.builder) fail("the opacity-grid builder has not run in this process");
-  return builder_profile(G.builder, idop, ilor, out, capacity, halfsize);
+  return builder_profile(G.builder.get(), idop, ilor, out, capacity, halfsize);
   API_END_INT
 }
 
