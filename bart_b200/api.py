@@ -100,6 +100,9 @@ def lib():
     L.bart_chain_block.restype = None
     L.bart_mcmc_init.argtypes = [C.c_int, C.c_int, dp, dp, dp, dp, dp, dp, C.c_int, dp, dp,
                                  C.c_double, C.c_double, C.c_int]
+    L.bart_mcmc_init_ensemble.argtypes = [C.c_int, C.c_int, C.c_int, dp, dp, dp, dp, dp, dp, C.c_int,
+                                          dp, dp, C.c_double, C.c_double, C.c_int]
+    L.bart_mcmc_nretr.restype = C.c_int
     L.bart_mcmc_run.argtypes = [C.c_int, dp, ip, ip, dp, dp]
     L.bart_mcmc_resume.argtypes = [C.c_int, dp]
     L.bart_mcmc_snooker_init.argtypes = [C.c_int, C.c_int, dp]
@@ -339,14 +342,47 @@ class Transit:
                                     _d(prior), _d(priorlow), len(data), _d(data), _d(uncert),
                                     float(fgamma), float(fepsilon), int(burnin)))
         self._mc_shape = (nchains, npars, int(np.sum(stepsize > 0)), len(data))
+        self._mc_ensemble = False
+
+    def mcmc_init_ensemble(self, params, pmin, pmax, stepsize, data, uncert, prior=None,
+                           priorlow=None, fgamma=1.0, fepsilon=0.0, burnin=0):
+        """R independent retrievals in one device loop (bart_mcmc_init_ensemble): params[R][C][P]
+        starting points, data / uncert[R][D]; bounds, step sizes and priors shared.  Afterwards the
+        mcmc_* calls take and return every array behind a leading [R] axis."""
+        params = np.ascontiguousarray(params, dtype=np.float64)
+        if params.ndim != 3:
+            raise BartError("params must be [retrievals][chains][parameters]")
+        nretr, nchains, npars = params.shape
+        f = lambda a: np.ascontiguousarray(a if a is not None else np.zeros(npars), dtype=np.float64)
+        pmin, pmax, stepsize, prior, priorlow = (f(a) for a in (pmin, pmax, stepsize, prior, priorlow))
+        data = np.ascontiguousarray(data, dtype=np.float64)
+        uncert = np.ascontiguousarray(uncert, dtype=np.float64)
+        if data.ndim != 2 or data.shape[0] != nretr or uncert.shape != data.shape:
+            raise BartError("data and uncert must be [%d retrievals][data points]" % nretr)
+        _check(lib().bart_mcmc_init_ensemble(nretr, nchains, npars, _d(params), _d(pmin), _d(pmax),
+                                             _d(stepsize), _d(prior), _d(priorlow), data.shape[1],
+                                             _d(data), _d(uncert), float(fgamma), float(fepsilon),
+                                             int(burnin)))
+        self._mc_shape = (nchains, npars, int(np.sum(stepsize > 0)), data.shape[1])
+        self._mc_ensemble = True
+
+    def _mc_lead(self):
+        """Leading axis of the loop's arrays: () after mcmc_init, (R,) after mcmc_init_ensemble."""
+        return (lib().bart_mcmc_nretr(),) if getattr(self, "_mc_ensemble", False) else ()
+
+    def _mc_refuse(self, lead, what):
+        raise BartError("%s do not have MC3's shapes for %s%d chains" % (
+            what, "%d retrievals x " % lead[0] if lead else "", self._mc_shape[0]))
 
     def mcmc_resume(self, nold, curmodel=None):
         """MC3's resume=True (mcmc.py:254-269) after mcmc_init with the old run's last states."""
         if curmodel is not None:
             curmodel = np.ascontiguousarray(curmodel, dtype=np.float64)
             nchains, npars, nfree, ndata = self._mc_shape
-            if curmodel.shape != (nchains, ndata):
-                raise BartError("curmodel must be [%d chains][%d data]" % (nchains, ndata))
+            lead = self._mc_lead()
+            if curmodel.shape != lead + (nchains, ndata):
+                raise BartError("curmodel must be [%s%d chains][%d data]"
+                                % ("%d retrievals][" % lead[0] if lead else "", nchains, ndata))
         _check(lib().bart_mcmc_resume(int(nold), None if curmodel is None else _d(curmodel)))
 
     def mcmc_run(self, support, r1, r2, unif, ugamma):
@@ -355,38 +391,51 @@ class Transit:
         ugamma = np.ascontiguousarray(ugamma, dtype=np.float64)
         r1 = np.ascontiguousarray(r1, dtype=np.int32)
         r2 = np.ascontiguousarray(r2, dtype=np.int32)
-        niter = unif.shape[0]
+        lead = self._mc_lead()
+        niter = unif.shape[-2] if unif.ndim >= 2 else 0
         nchains, npars, nfree, ndata = self._mc_shape
-        if support.shape != (niter, nchains, nfree) or r1.shape != (nchains, niter) or \
-                r2.shape != (nchains, niter) or unif.shape != (niter, nchains) or \
-                ugamma.shape != (niter, nchains):
-            raise BartError("random streams do not have MC3's shapes for %d chains x %d iterations"
-                            % (nchains, niter))
+        if support.shape != lead + (niter, nchains, nfree) or r1.shape != lead + (nchains, niter) or \
+                r2.shape != lead + (nchains, niter) or unif.shape != lead + (niter, nchains) or \
+                ugamma.shape != lead + (niter, nchains):
+            if not lead:
+                raise BartError("random streams do not have MC3's shapes for %d chains x %d iterations"
+                                % (nchains, niter))
+            self._mc_refuse(lead, "random streams")
         _check(lib().bart_mcmc_run(niter, _d(support), r1.ctypes.data_as(ip), r2.ctypes.data_as(ip),
                                    _d(unif), _d(ugamma)))
         self._mc_niter = niter
 
     def mcmc_snooker_init(self, z0, thinning=1):
-        """z0[hsize][nchains][nfree]: MC3's M0 initial history samples (mcmc.py:421-424)."""
+        """z0[hsize][nchains][nfree] ([R][hsize][nchains][nfree] for an ensemble): MC3's M0 initial
+        history samples (mcmc.py:421-424)."""
         nchains, npars, nfree, ndata = self._mc_shape
+        lead = self._mc_lead()
         z0 = np.ascontiguousarray(z0, dtype=np.float64)
-        if z0.ndim != 3 or z0.shape[1:] != (nchains, nfree):
-            raise BartError("z0 must be [hsize][%d][%d]" % (nchains, nfree))
-        _check(lib().bart_mcmc_snooker_init(z0.shape[0], int(thinning), _d(z0)))
-        self._mc_zsize, self._mc_thinning = z0.shape[0], int(thinning)
+        if z0.ndim != 3 + len(lead) or z0.shape[:len(lead)] != lead or z0.shape[-2:] != (nchains, nfree):
+            raise BartError("z0 must be [%shsize][%d][%d]" % ("%d][" % lead[0] if lead else "", nchains, nfree))
+        hsize = z0.shape[len(lead)]
+        _check(lib().bart_mcmc_snooker_init(hsize, int(thinning), _d(z0)))
+        self._mc_zsize, self._mc_thinning = hsize, int(thinning)
 
     def mcmc_run_snooker(self, support, i1, i2, iz, ic, usnooker, usn_offset, unif, ugamma):
+        """Streams of run_snooker's shapes; for an ensemble each behind [R], usnooker the
+        retrievals' factor rows one after the other and usn_offset[R][niter+1] absolute rows."""
         nchains, npars, nfree, ndata = self._mc_shape
+        lead = self._mc_lead()
         support, unif, ugamma, usnooker = (np.ascontiguousarray(a, dtype=np.float64)
                                            for a in (support, unif, ugamma, usnooker))
         i1, i2, iz, ic, usn_offset = (np.ascontiguousarray(a, dtype=np.int32)
                                       for a in (i1, i2, iz, ic, usn_offset))
-        niter = unif.shape[0]
-        if support.shape != (niter, nchains, nfree) or ugamma.shape != (niter, nchains) or \
-                any(a.shape != (niter, nchains) for a in (i1, i2, iz, ic)) or \
-                usn_offset.shape != (niter + 1,) or usnooker.shape != (usn_offset[-1], nfree):
-            raise BartError("random streams do not have MC3's shapes for %d chains x %d iterations"
-                            % (nchains, niter))
+        niter = unif.shape[-2] if unif.ndim >= 2 else 0
+        if support.shape != lead + (niter, nchains, nfree) or ugamma.shape != lead + (niter, nchains) or \
+                unif.shape != lead + (niter, nchains) or \
+                any(a.shape != lead + (niter, nchains) for a in (i1, i2, iz, ic)) or \
+                usn_offset.shape != lead + (niter + 1,) or \
+                usnooker.shape != (usn_offset.flat[-1] if usn_offset.size else -1, nfree):
+            if not lead:
+                raise BartError("random streams do not have MC3's shapes for %d chains x %d iterations"
+                                % (nchains, niter))
+            self._mc_refuse(lead, "snooker streams")
         _check(lib().bart_mcmc_run_snooker(
             niter, _d(support), i1.ctypes.data_as(ip), i2.ctypes.data_as(ip), iz.ctypes.data_as(ip),
             ic.ctypes.data_as(ip), _d(usnooker), usn_offset.ctypes.data_as(ip), _d(unif), _d(ugamma)))
@@ -395,20 +444,25 @@ class Transit:
 
     def mcmc_get(self, name):
         nchains, npars, nfree, ndata = self._mc_shape
+        lead = self._mc_lead()
         if name in ("Z", "Zchisq"):
             # _mc_zsize is an upper bound (it counts thinned rows per call; the library grows Z on
             # the GLOBAL iteration number, like MC3): size the result from what the library returns
-            out = np.zeros((self._mc_zsize, nchains, npars) if name == "Z" else (self._mc_zsize, nchains))
+            tail = (nchains, npars) if name == "Z" else (nchains,)
+            out = np.zeros(lead + (getattr(self, "_mc_zsize", 0),) + tail)
             n = lib().bart_mcmc_get(name.encode(), _d(out), out.size)
             _check(0 if n >= 0 else -1)
-            rows = n // (nchains * npars if name == "Z" else nchains)
-            return out[:rows]
+            rows = n // (int(np.prod(lead + tail)))
+            if not lead:
+                return out[:rows]
+            return out.ravel()[:n].reshape(lead + (rows,) + tail).copy()
         shapes = {"allparams": (nchains, nfree, getattr(self, "_mc_niter", 0)),
                   "allmodel": (nchains, ndata, getattr(self, "_mc_niter", 0)),
                   "params": (nchains, npars), "currchisq": (nchains,), "numaccept": (nchains,),
                   "outbounds": (nchains, nfree), "bestp": (npars,), "bestchisq": (1,),
                   "bestmodel": (ndata,), "models": (nchains, ndata)}
-        out = np.zeros(shapes[name])
+        shape = lead + shapes[name] if name != "bestchisq" or not lead else lead
+        out = np.zeros(shape)
         n = lib().bart_mcmc_get(name.encode(), _d(out), out.size)
         _check(0 if n >= 0 else -1)
         return out

@@ -10,11 +10,17 @@
 //                          rejection tests, per-model radius / cloud-top / scattering knobs.
 //                          Writes the profiles buffer in run_transit's layout, so atm_prep reads it
 //                          unchanged.
-//   demc_propose_kernel    warp <-> chain, lanes over parameters: DE-MC jump from two other chains' current states,
-//                          boundary clamp, shared parameters.  Products and sums are rounded
-//                          separately (no FMA contraction) so chains are bit-identical to numpy.
-//   chisq_accept_kernel    one CTA: per-chain chi-squared with priors, Metropolis rule, state
-//                          update, trace, running best fit (first-index argmin like numpy).
+//   demc_propose_kernel    warp <-> (retrieval, chain), lanes over parameters: DE-MC jump from two
+//                          other chains' current states of the same retrieval, boundary clamp, shared
+//                          parameters.  Products and sums are rounded separately (no FMA
+//                          contraction) so chains are bit-identical to numpy.
+//   chisq_accept_kernel    one CTA per retrieval: per-chain chi-squared with priors, Metropolis rule,
+//                          state update, trace, running best fit (first-index argmin like numpy).
+//
+// An ensemble of retrievals (McmcDev::nretr) is one flattened population g = r * nchains + c for the
+// forward model; every per-retrieval step (partners, slot numbering, norm ratio, best fit, history)
+// stays inside the retrieval's own chains and keeps the lone run's arithmetic and order, so
+// retrieval r of an ensemble is bit-identical to the same retrieval run alone.
 //
 // These are latency-bound kernels over [nchains x npars] doubles: no roofline claim; they exist so
 // that the per-generation host round trip (MPI scatter/gather in the reference) disappears.
@@ -319,33 +325,36 @@ void launch_energy_balance(const double *spectra, const double *wn, int nwave, d
 
 // ---------------------------------------------------------------------------------------
 // DE-MC proposal (mcmc.py:524-575): jump = gamma1 (x_r1 - x_r2) + fepsilon * support
-// One warp per chain, lanes over the free parameters: the loads of a jump (two other chains' states,
+// One warp per (retrieval, chain), lanes over the free parameters: the loads of a jump (two other chains' states,
 // the support draw, the bounds) go out side by side instead of as one dependent round trip per
 // parameter (at MC3's population sizes the kernel's time is its chain of memory latencies).
 __global__ void __launch_bounds__(256) demc_propose_kernel(McmcDev mc) {
   const int lane = threadIdx.x & 31;
-  const int c = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
-  if (c >= mc.nchains) return;                  // whole warps
-  const int i = *mc.iter;
+  const int g = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;   // (retrieval, chain) flattened
+  const int nc = mc.nchains;
+  if (g >= mc.nretr * nc) return;               // whole warps
+  const int r = g / nc, c = g - r * nc;
+  const int i = mc.iter[r];
   const int np = mc.npars;
-  const double *cur = mc.params + (size_t)c * np;
-  double *nx = mc.nextp + (size_t)c * np;
-  const int ra = mc.r1[(size_t)c * mc.chainsize + i], rb = mc.r2[(size_t)c * mc.chainsize + i];
-  const double ug = mc.ugamma[(size_t)i * mc.nchains + c];
-  const double *a = mc.params + (size_t)ra * np;
-  const double *b = mc.params + (size_t)rb * np;
-  const double g = ug < 0.1 ? 0.98 : mc.gamma;
-  const double *sup = mc.support + ((size_t)i * mc.nchains + c) * mc.nfree;
+  const double *cur = mc.params + (size_t)g * np;
+  double *nx = mc.nextp + (size_t)g * np;
+  const int ra = mc.r1[(size_t)g * mc.chainsize + i], rb = mc.r2[(size_t)g * mc.chainsize + i];
+  const size_t k = ((size_t)r * mc.chainsize + i) * nc + c;    // this chain's entry of generation i
+  const double ug = mc.ugamma[k];
+  const double *a = mc.params + ((size_t)r * nc + ra) * np;
+  const double *b = mc.params + ((size_t)r * nc + rb) * np;
+  const double gm = ug < 0.1 ? 0.98 : mc.gamma;
+  const double *sup = mc.support + k * mc.nfree;
   int out = 0;
   for (int f = lane; f < mc.nfree; f += 32) {
     const int p = mc.ifree[f];
     const double ap = a[p], bp = b[p], cp = cur[p], sf = sup[f], lo = mc.pmin[p], hi = mc.pmax[p];
-    const int ob = mc.outbounds[(size_t)c * mc.nfree + f];
-    const double jump = __dadd_rn(__dmul_rn(g, __dsub_rn(ap, bp)), __dmul_rn(mc.fepsilon, sf));
+    const int ob = mc.outbounds[(size_t)g * mc.nfree + f];
+    const double jump = __dadd_rn(__dmul_rn(gm, __dsub_rn(ap, bp)), __dmul_rn(mc.fepsilon, sf));
     double v = __dadd_rn(cp, jump);
     const int o = (v < lo) || (v > hi);
     out |= o;
-    mc.outbounds[(size_t)c * mc.nfree + f] = ob + o;
+    mc.outbounds[(size_t)g * mc.nfree + f] = ob + o;
     if (v < lo) v = lo;
     if (v > hi) v = hi;
     nx[p] = v;
@@ -354,13 +363,14 @@ __global__ void __launch_bounds__(256) demc_propose_kernel(McmcDev mc) {
   __syncwarp();                                 // the lanes' nx[] are visible to lane 0
   if (lane == 0) {
     for (int s = 0; s < mc.nshare; s++) nx[mc.share_dst[s]] = nx[mc.share_src[s]];
-    mc.outflag[c] = out;
+    mc.outflag[g] = out;
   }
 }
 
 void launch_demc_propose(const McmcDev &mc, cudaStream_t s) {
   const int threads = 256;                      // 8 chains per CTA
-  demc_propose_kernel<<<(mc.nchains * 32 + threads - 1) / threads, threads, 0, s>>>(mc);
+  const int warps = mc.nretr * mc.nchains;
+  demc_propose_kernel<<<(warps * 32 + threads - 1) / threads, threads, 0, s>>>(mc);
 }
 
 // ---------------------------------------------------------------------------------------
@@ -390,45 +400,51 @@ __device__ double np_pairwise_sum(const double *a, int n) {
 // along x - z (zp = projections of z1, z2), or u (z2 - z1) when z coincides with the chain's
 // state.  The uniform factors u come in the reference from two calls whose sizes depend on the
 // states (unprojected chains first): `slot` reproduces that assignment.
-// One CTA (the slot numbering below is one ordered pass over the chains); a warp per chain with
+// One CTA per retrieval (the slot numbering below is one ordered pass over its chains); a warp per chain with
 // lanes over the parameters, like demc_propose_kernel: the loads of a jump go out side by side and the
 // projection's three dot products are numpy's pairwise sums (np_pairwise_sum, every lane the same
 // sequence) over the warp's products in shared memory.
 constexpr int kSnkThreads = 512;
 __global__ void __launch_bounds__(kSnkThreads) snooker_propose_kernel(McmcDev mc) {
   __shared__ double s_dz[kSnkThreads / 32][kMaxPars], s_t[3][kSnkThreads / 32][kMaxPars];
-  const int i = *mc.iter;
+  const int r = blockIdx.x;                     // retrieval
+  const int i = mc.iter[r];
   const int np = mc.npars, nc = mc.nchains;
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nwarps = blockDim.x >> 5;
-  const int *gi1 = mc.i1 + (size_t)i * nc, *gi2 = mc.i2 + (size_t)i * nc;
-  const int *giz = mc.iz + (size_t)i * nc, *gic = mc.ic + (size_t)i * nc;
-  const double *ug = mc.ugamma + (size_t)i * nc;
+  const size_t gen = ((size_t)r * mc.chainsize + i) * nc;   // generation i of retrieval r in the streams
+  const int *gi1 = mc.i1 + gen, *gi2 = mc.i2 + gen;
+  const int *giz = mc.iz + gen, *gic = mc.ic + gen;
+  const double *ug = mc.ugamma + gen;
+  int *noproj = mc.noproj + (size_t)r * nc, *slot = mc.slot + (size_t)r * nc;
+  const double *params = mc.params + (size_t)r * nc * np;
   for (int c = warp; c < nc; c += nwarps) {
-    const double *z = mc.Z + ((size_t)giz[c] * nc + gic[c]) * np;
-    const double *cur = mc.params + (size_t)c * np;
+    const double *z = mc.Z + zidx(mc, giz[c], r, gic[c]) * np;
+    const double *cur = params + (size_t)c * np;
     int same = 1;
     for (int p = lane; p < np; p += 32) same &= (z[p] == cur[p]);   // np.all(z == params, axis=1)
     same = __all_sync(0xffffffffu, same) ? 1 : 0;
-    if (lane == 0) mc.noproj[c] = same;
+    if (lane == 0) noproj[c] = same;
   }
   __syncthreads();
   if (threadIdx.x == 0) {
-    int k = mc.usn_off[i];
-    for (int c = 0; c < nc; c++) if (ug[c] < 0.1 && mc.noproj[c]) mc.slot[c] = k++;
-    for (int c = 0; c < nc; c++) if (ug[c] < 0.1 && !mc.noproj[c]) mc.slot[c] = k++;
+    int k = mc.usn_off[(size_t)r * (mc.chainsize + 1) + i];
+    for (int c = 0; c < nc; c++) if (ug[c] < 0.1 && noproj[c]) slot[c] = k++;
+    for (int c = 0; c < nc; c++) if (ug[c] < 0.1 && !noproj[c]) slot[c] = k++;
   }
   __syncthreads();
   const int nfree = mc.nfree;
   for (int c = warp; c < nc; c += nwarps) {
-    const double *cur = mc.params + (size_t)c * np;
-    double *nx = mc.nextp + (size_t)c * np;
-    const double *z1 = mc.Z + (size_t)gi1[c] * np;
-    const double *z2 = mc.Z + (size_t)gi2[c] * np;
-    const double *z = mc.Z + ((size_t)giz[c] * nc + gic[c]) * np;
+    const size_t g = (size_t)r * nc + c;
+    const double *cur = params + (size_t)c * np;
+    double *nx = mc.nextp + g * np;
+    // i1 / i2 are flat (row, chain) indices of the retrieval's own history (mcmc.py:529-535)
+    const double *z1 = mc.Z + zidx(mc, gi1[c] / nc, r, gi1[c] % nc) * np;
+    const double *z2 = mc.Z + zidx(mc, gi2[c] / nc, r, gi2[c] % nc) * np;
+    const double *z = mc.Z + zidx(mc, giz[c], r, gic[c]) * np;
     const bool sj = ug[c] < 0.1;
-    const bool proj = sj && !mc.noproj[c];
-    const double *sup = mc.support + ((size_t)i * nc + c) * nfree;
-    const double *u = sj ? mc.usn + (size_t)mc.slot[c] * nfree : nullptr;
+    const bool proj = sj && !noproj[c];
+    const double *sup = mc.support + (gen + c) * nfree;
+    const double *u = sj ? mc.usn + (size_t)slot[c] * nfree : nullptr;
     double dzp = 0.0, d2 = 1.0;
     if (proj) {
       for (int f = lane; f < nfree; f += 32) {
@@ -456,7 +472,7 @@ __global__ void __launch_bounds__(kSnkThreads) snooker_propose_kernel(McmcDev mc
       double v = __dadd_rn(cur[p], jump);
       const int o = (v < lo) || (v > hi);
       out |= o;
-      mc.outbounds[(size_t)c * nfree + f] += o;
+      mc.outbounds[g * nfree + f] += o;
       if (v < lo) v = lo;
       if (v > hi) v = hi;
       nx[p] = v;
@@ -465,13 +481,13 @@ __global__ void __launch_bounds__(kSnkThreads) snooker_propose_kernel(McmcDev mc
     __syncwarp();                               // the lanes' nx[] are visible to lane 0; s_dz / s_t free again
     if (lane == 0) {
       for (int s = 0; s < mc.nshare; s++) nx[mc.share_dst[s]] = nx[mc.share_src[s]];
-      mc.outflag[c] = out;
+      mc.outflag[g] = out;
     }
   }
 }
 
 void launch_snooker_propose(const McmcDev &mc, cudaStream_t s) {
-  snooker_propose_kernel<<<1, kSnkThreads, 0, s>>>(mc);
+  snooker_propose_kernel<<<mc.nretr, kSnkThreads, 0, s>>>(mc);
 }
 
 // ---------------------------------------------------------------------------------------
@@ -485,35 +501,34 @@ __device__ const double *chain_model(const double *models, const ModelMap &mp, i
 }
 
 // chisq.c:111-142 + stats.h:72-103: sequential sums; priorup is priorlow at the call sites
-// (mcmc.py:338-339,596-597 pass priorlow twice)
-__device__ void chain_chisq(const McmcDev &mc, const double *model, const double *p, double *chisq,
-                            double *c2) {
+// (mcmc.py:338-339,596-597 pass priorlow twice).  data / uncert: the chain's retrieval's.
+__device__ __forceinline__ void chain_chisq(const McmcDev &mc, const double *data, const double *uncert,
+                                            const double *model, const double *p, double &chisq) {
   double c = 0.0;
   for (int i = 0; i < mc.ndata; i++) {
-    const double r = (model[i] - mc.data[i]) / mc.uncert[i];
+    const double r = (model[i] - data[i]) / uncert[i];
     c = __dadd_rn(c, __dmul_rn(r, r));
   }
-  double jc = 0.0;
   for (int k = 0; k < mc.nprior; k++) {
     const int ip = mc.iprior[k];
     const double off = p[ip] - mc.prior[ip], lo = mc.priorlow[ip];
-    if (lo == -1) { const double t = 2.0 * log(off); c += t; jc += t; }
+    if (lo == -1) c += 2.0 * log(off);
     else { const double r = off / lo; c = __dadd_rn(c, __dmul_rn(r, r)); }
   }
-  *chisq = c;
-  *c2 = c - jc;
+  chisq = c;
 }
 
 // chain_chisq by a whole warp: the residuals of 32 data points at a time side by side, their squares
 // added in index order (every lane carries the same running sum), priors as in chain_chisq
-__device__ void warp_chain_chisq(const McmcDev &mc, const double *model, const double *p, int lane,
-                                 double *chisq, double *c2) {
+__device__ __forceinline__ void warp_chain_chisq(const McmcDev &mc, const double *data, const double *uncert,
+                                                 const double *model, const double *p, int lane,
+                                                 double &chisq, double &c2) {
   double c = 0.0;
   for (int base = 0; base < mc.ndata; base += 32) {
     const int idx = base + lane;
     double r2 = 0.0;
     if (idx < mc.ndata) {
-      const double r = (model[idx] - mc.data[idx]) / mc.uncert[idx];
+      const double r = (model[idx] - data[idx]) / uncert[idx];
       r2 = __dmul_rn(r, r);
     }
     const int cnt = min(32, mc.ndata - base);
@@ -526,20 +541,43 @@ __device__ void warp_chain_chisq(const McmcDev &mc, const double *model, const d
     if (lo == -1) { const double t = 2.0 * log(off); c += t; jc += t; }
     else { const double r = off / lo; c = __dadd_rn(c, __dmul_rn(r, r)); }
   }
-  *chisq = c;
-  *c2 = c - jc;
+  chisq = c;
+  c2 = c - jc;
 }
 
-// One CTA; a warp per chain with lanes over the data points / parameters, so that a chain's
-// residuals, state copy and trace stores go out side by side (thread-per-chain was ~20 dependent
-// memory round trips: 11 us at 10 chains).  The snooker norm keeps its 256-slot reduction tree.
+// first index of the minimum of v[0..n) (np.argmin) by one warp; every lane gets (best, arg)
+__device__ __forceinline__ void warp_argmin(const double *v, int n, double &best, int &arg) {
+  best = INFINITY;
+  arg = 0x7fffffff;
+  for (int c = threadIdx.x & 31; c < n; c += 32) {
+    const double x = v[c];
+    if (x < best || (x == best && c < arg)) { best = x; arg = c; }
+  }
+  for (int o = 16; o > 0; o >>= 1) {
+    const double ob = __shfl_down_sync(0xffffffffu, best, o);
+    const int oa = __shfl_down_sync(0xffffffffu, arg, o);
+    if (ob < best || (ob == best && oa < arg)) { best = ob; arg = oa; }
+  }
+  best = __shfl_sync(0xffffffffu, best, 0);
+  arg = __shfl_sync(0xffffffffu, arg, 0);
+}
+
+// One CTA per retrieval; a warp per chain with lanes over the data points / parameters, so that a
+// chain's residuals, state copy and trace stores go out side by side (thread-per-chain was ~20
+// dependent memory round trips: 11 us at 10 chains).  The snooker norm keeps its 256-slot reduction
+// tree.  The CTA advances its retrieval's generation counter (and history size) at the end; no other
+// CTA reads them.
 constexpr int kChisqThreads = 512;
 __global__ void __launch_bounds__(kChisqThreads)
 chisq_accept_kernel(McmcDev mc, const double *__restrict__ models, ModelMap mp, int first) {
-  const int np = mc.npars;
-  const int i = *mc.iter;
+  const int np = mc.npars, nc = mc.nchains;
+  const int r = blockIdx.x;                     // retrieval
+  const int g0 = r * nc;                        // its first chain in the flattened population
+  const int i = mc.iter[r];
   const bool snooker = mc.walk == 1 && !first;
-  const int zrow = snooker ? *mc.zsize : 0;
+  const int zrow = snooker ? mc.zsize[r] : 0;
+  const size_t gen = ((size_t)r * mc.chainsize + i) * nc;     // generation i of retrieval r in the streams
+  const double *data = mc.data + (size_t)r * mc.ndata, *uncert = mc.uncert + (size_t)r * mc.ndata;
   // Metropolis factor of the projected snooker jumps (mcmc.py:603-609): ONE ratio of Frobenius
   // norms over all such chains of this generation, to the power nfree-1 (the reference's
   // np.linalg.norm over the stacked rows; its BLAS summation order is not reproduced, so the
@@ -550,12 +588,11 @@ chisq_accept_kernel(McmcDev mc, const double *__restrict__ models, ModelMap mp, 
   if (snooker) {
     if (threadIdx.x < 256) {
       double a1 = 0.0, a2 = 0.0;
-      for (int c = threadIdx.x; c < mc.nchains; c += 256) {
-        const bool sj = mc.ugamma[(size_t)i * mc.nchains + c] < 0.1;
-        if (!sj || mc.noproj[c] || mc.outflag[c]) continue;
-        const double *z = mc.Z + ((size_t)mc.iz[(size_t)i * mc.nchains + c] * mc.nchains +
-                                  mc.ic[(size_t)i * mc.nchains + c]) * np;
-        const double *cur = mc.params + (size_t)c * np, *nx = mc.nextp + (size_t)c * np;
+      for (int c = threadIdx.x; c < nc; c += 256) {
+        const bool sj = mc.ugamma[gen + c] < 0.1;
+        if (!sj || mc.noproj[g0 + c] || mc.outflag[g0 + c]) continue;
+        const double *z = mc.Z + zidx(mc, mc.iz[gen + c], r, mc.ic[gen + c]) * np;
+        const double *cur = mc.params + (size_t)(g0 + c) * np, *nx = mc.nextp + (size_t)(g0 + c) * np;
         for (int f = 0; f < mc.nfree; f++) {
           const int p = mc.ifree[f];
           const double d1 = nx[p] - z[p], d2 = cur[p] - z[p];
@@ -572,137 +609,121 @@ chisq_accept_kernel(McmcDev mc, const double *__restrict__ models, ModelMap mp, 
     mrf = pow(sqrt(s_n1[0]) / sqrt(s_n2[0]), (double)(mc.nfree - 1));
   }
   const int lane = threadIdx.x & 31, nwarps = blockDim.x >> 5;
-  for (int c = threadIdx.x >> 5; c < mc.nchains; c += nwarps) {
-    const double *model = chain_model(models, mp, c, mc.ndata);
-    double *cur = mc.params + (size_t)c * np;
+  for (int c = threadIdx.x >> 5; c < nc; c += nwarps) {
+    const int g = g0 + c;
+    const double *model = chain_model(models, mp, g, mc.ndata);
+    double *cur = mc.params + (size_t)g * np;
     if (first) {
       double chisq, c2;
-      warp_chain_chisq(mc, model, cur, lane, &chisq, &c2);
-      if (lane == 0) { mc.currchisq[c] = chisq; mc.c2[c] = c2; }
+      warp_chain_chisq(mc, data, uncert, model, cur, lane, chisq, c2);
+      if (lane == 0) { mc.currchisq[g] = chisq; mc.c2[g] = c2; }
       continue;
     }
-    const double *nx = mc.nextp + (size_t)c * np;
-    const int oflag = mc.outflag[c];
-    const double currc = mc.currchisq[c];
-    const double u = mc.unif[(size_t)i * mc.nchains + c];
-    const bool proj = snooker && mc.ugamma[(size_t)i * mc.nchains + c] < 0.1 && !mc.noproj[c] && !oflag;
+    const double *nx = mc.nextp + (size_t)g * np;
+    const int oflag = mc.outflag[g];
+    const double currc = mc.currchisq[g];
+    const double u = mc.unif[gen + c];
+    const bool proj = snooker && mc.ugamma[gen + c] < 0.1 && !mc.noproj[g] && !oflag;
     double next = INFINITY, c2 = 0.0;                          // mcmc.py:598
-    if (!oflag) warp_chain_chisq(mc, model, nx, lane, &next, &c2);
+    if (!oflag) warp_chain_chisq(mc, data, uncert, model, nx, lane, next, c2);
     double accept = exp(0.5 * (currc - next));
     if (proj) accept = __dmul_rn(accept, mrf);
     const bool ok = accept >= u;
     const double *state = ok ? nx : cur;                        // the chain's state after this generation
     for (int f = lane; f < mc.nfree; f += 32)
-      mc.allparams[((size_t)c * mc.nfree + f) * mc.chainsize + i] = state[mc.ifree[f]];
+      mc.allparams[((size_t)g * mc.nfree + f) * mc.chainsize + i] = state[mc.ifree[f]];
     if (snooker && (mc.nold + i) % mc.thinning == 0) {         // mcmc.py:653-660
-      double *zr = mc.Z + ((size_t)zrow * mc.nchains + c) * np;
+      const size_t zk = zidx(mc, zrow, r, c);
+      double *zr = mc.Z + zk * np;
       for (int f = lane; f < mc.nfree; f += 32) zr[mc.ifree[f]] = state[mc.ifree[f]];
-      if (lane == 0) mc.Zchisq[(size_t)zrow * mc.nchains + c] = ok ? next : currc;
+      if (lane == 0) mc.Zchisq[zk] = ok ? next : currc;
     }
     {                                                          // mcmc.py:636-651
-      double *cm = mc.curmodel + (size_t)c * mc.ndata;
+      double *cm = mc.curmodel + (size_t)g * mc.ndata;
       for (int d = lane; d < mc.ndata; d += 32) {
         const double v = ok ? model[d] : cm[d];
         if (ok) cm[d] = v;
-        mc.allmodel[((size_t)c * mc.ndata + d) * mc.chainsize + i] = v;
+        mc.allmodel[((size_t)g * mc.ndata + d) * mc.chainsize + i] = v;
       }
     }
     __syncwarp();                                              // every lane has read `state` = cur when !ok
     if (ok)
       for (int p = lane; p < np; p += 32) cur[p] = nx[p];
     if (lane == 0) {
-      if (!oflag) mc.c2[c] = c2;
-      mc.nextchisq[c] = next;
+      if (!oflag) mc.c2[g] = c2;
+      mc.nextchisq[g] = next;
       if (ok) {
-        mc.currchisq[c] = next;
-        if (mc.nold + i >= mc.burnin) mc.numaccept[c] += 1.0;
+        mc.currchisq[g] = next;
+        if (mc.nold + i >= mc.burnin) mc.numaccept[g] += 1.0;
       }
     }
   }
   __syncthreads();
   // running best fit: first index of the minimum no-Jeffreys chi-squared (np.argmin)
   if (threadIdx.x < 32) {
-    double best = INFINITY;
-    int arg = 0x7fffffff;
-    for (int c = threadIdx.x; c < mc.nchains; c += 32) {
-      const double v = mc.c2[c];
-      if (v < best || (v == best && c < arg)) { best = v; arg = c; }
-    }
-    for (int o = 16; o > 0; o >>= 1) {
-      const double ob = __shfl_down_sync(0xffffffffu, best, o);
-      const int oa = __shfl_down_sync(0xffffffffu, arg, o);
-      if (ob < best || (ob == best && oa < arg)) { best = ob; arg = oa; }
-    }
-    best = __shfl_sync(0xffffffffu, best, 0);
-    arg = __shfl_sync(0xffffffffu, arg, 0);
-    const bool take = arg < mc.nchains && (first || best < *mc.bestchisq);
+    double best;
+    int arg;
+    warp_argmin(mc.c2 + g0, nc, best, arg);
+    const bool take = arg < nc && (first || best < mc.bestchisq[r]);
     if (take) {
-      const double *model = chain_model(models, mp, arg, mc.ndata);
-      for (int p = threadIdx.x; p < np; p += 32) mc.bestp[p] = mc.params[(size_t)arg * np + p];
-      for (int d = threadIdx.x; d < mc.ndata; d += 32) mc.bestmodel[d] = model[d];
+      const double *model = chain_model(models, mp, g0 + arg, mc.ndata);
+      for (int p = threadIdx.x; p < np; p += 32) mc.bestp[(size_t)r * np + p] = mc.params[(size_t)(g0 + arg) * np + p];
+      for (int d = threadIdx.x; d < mc.ndata; d += 32) mc.bestmodel[(size_t)r * mc.ndata + d] = model[d];
     }
     __syncwarp();
     if (threadIdx.x == 0) {
-      if (take) *mc.bestchisq = best;
-      if (!first) *mc.iter = i + 1;
-      if (snooker && (mc.nold + i) % mc.thinning == 0) *mc.zsize = zrow + 1;
+      if (take) mc.bestchisq[r] = best;
+      if (!first) mc.iter[r] = i + 1;
+      if (snooker && (mc.nold + i) % mc.thinning == 0) mc.zsize[r] = zrow + 1;
     }
   }
 }
 
 // chi-squared of the initial Z samples of row `row` and the running best over rows in flattened
 // (row, chain) order, first minimum wins like np.argmin (mcmc.py:441-460); Zchisq keeps the value
-// WITH the Jeffreys term, which is also what the reference compares to the chains' best (462-470)
+// WITH the Jeffreys term, which is also what the reference compares to the chains' best (462-470).
+// One CTA per retrieval.
 __global__ void __launch_bounds__(256)
 zrow_chisq_kernel(McmcDev mc, const double *__restrict__ models, ModelMap mp, int row, int last) {
-  const int np = mc.npars;
-  double *zc = mc.Zchisq + (size_t)row * mc.nchains;
-  for (int c = threadIdx.x; c < mc.nchains; c += blockDim.x) {
-    double unused;
-    chain_chisq(mc, chain_model(models, mp, c, mc.ndata), mc.Z + ((size_t)row * mc.nchains + c) * np,
-                &zc[c], &unused);
-  }
+  const int np = mc.npars, nc = mc.nchains, nd = mc.ndata;
+  const int r = blockIdx.x, g0 = r * nc;
+  const double *data = mc.data + (size_t)r * nd, *uncert = mc.uncert + (size_t)r * nd;
+  double *zc = mc.Zchisq + zidx(mc, row, r, 0);
+  const double *zs = mc.Z + zidx(mc, row, r, 0) * np;
+  double *zbest = mc.zbest + (size_t)r * (1 + np + nd);
+  for (int c = threadIdx.x; c < nc; c += blockDim.x)
+    chain_chisq(mc, data, uncert, chain_model(models, mp, g0 + c, nd), zs + (size_t)c * np, zc[c]);
   __syncthreads();
   if (threadIdx.x < 32) {
-    double best = INFINITY;
-    int arg = 0x7fffffff;
-    for (int c = threadIdx.x; c < mc.nchains; c += 32) {
-      const double v = zc[c];
-      if (v < best || (v == best && c < arg)) { best = v; arg = c; }
-    }
-    for (int o = 16; o > 0; o >>= 1) {
-      const double ob = __shfl_down_sync(0xffffffffu, best, o);
-      const int oa = __shfl_down_sync(0xffffffffu, arg, o);
-      if (ob < best || (ob == best && oa < arg)) { best = ob; arg = oa; }
-    }
-    best = __shfl_sync(0xffffffffu, best, 0);
-    arg = __shfl_sync(0xffffffffu, arg, 0);
-    const bool take = arg < mc.nchains && (row == 0 || best < mc.zbest[0]);
+    double best;
+    int arg;
+    warp_argmin(zc, nc, best, arg);
+    const bool take = arg < nc && (row == 0 || best < zbest[0]);
     if (take) {
-      const double *model = chain_model(models, mp, arg, mc.ndata);
-      for (int p = threadIdx.x; p < np; p += 32) mc.zbest[1 + p] = mc.Z[((size_t)row * mc.nchains + arg) * np + p];
-      for (int d = threadIdx.x; d < mc.ndata; d += 32) mc.zbest[1 + np + d] = model[d];
+      const double *model = chain_model(models, mp, g0 + arg, nd);
+      for (int p = threadIdx.x; p < np; p += 32) zbest[1 + p] = zs[(size_t)arg * np + p];
+      for (int d = threadIdx.x; d < nd; d += 32) zbest[1 + np + d] = model[d];
     }
     __syncwarp();
-    if (threadIdx.x == 0 && take) mc.zbest[0] = best;
+    if (threadIdx.x == 0 && take) zbest[0] = best;
     __syncwarp();
-    if (last && mc.zbest[0] < *mc.bestchisq) {
-      for (int p = threadIdx.x; p < np; p += 32) mc.bestp[p] = mc.zbest[1 + p];
-      for (int d = threadIdx.x; d < mc.ndata; d += 32) mc.bestmodel[d] = mc.zbest[1 + np + d];
+    if (last && zbest[0] < mc.bestchisq[r]) {
+      for (int p = threadIdx.x; p < np; p += 32) mc.bestp[(size_t)r * np + p] = zbest[1 + p];
+      for (int d = threadIdx.x; d < nd; d += 32) mc.bestmodel[(size_t)r * nd + d] = zbest[1 + np + d];
       __syncwarp();
-      if (threadIdx.x == 0) *mc.bestchisq = mc.zbest[0];
+      if (threadIdx.x == 0) mc.bestchisq[r] = zbest[0];
     }
   }
 }
 
 void launch_zrow_chisq(const McmcDev &mc, const double *models, ModelMap map, int row, int last,
                        cudaStream_t s) {
-  zrow_chisq_kernel<<<1, 256, 0, s>>>(mc, models, map, row, last);
+  zrow_chisq_kernel<<<mc.nretr, 256, 0, s>>>(mc, models, map, row, last);
 }
 
 void launch_chisq_accept(const McmcDev &mc, const double *models, ModelMap map, int first,
                          cudaStream_t s) {
-  chisq_accept_kernel<<<1, kChisqThreads, 0, s>>>(mc, models, map, first);
+  chisq_accept_kernel<<<mc.nretr, kChisqThreads, 0, s>>>(mc, models, map, first);
 }
 
 }  // namespace bart

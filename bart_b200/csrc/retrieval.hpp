@@ -54,47 +54,65 @@ void launch_convert_params(const ConvConfig &cc, const double *params, int npars
 void launch_energy_balance(const double *spectra, const double *wn, int nwave, double out_scale,
                            double e_in, int *status, int nmodels, cudaStream_t s);
 
-// DE-MC state (device pointers), one population of `nchains` chains
+// DE-MC state (device pointers): an ensemble of `nretr` independent retrievals of `nchains` chains
+// each, sharing the forward model, bounds, step sizes and priors.  The population is the flattened
+// nretr x nchains models, g = r * nchains + c; arrays "per chain" below have that leading axis
+// ([nretr][nchains]...), arrays "per retrieval" a leading [nretr].  nretr = 1 is one retrieval.
 struct McmcDev {
-  int nchains, npars, nfree, ndata, nprior, chainsize, burnin, nold;
+  int nretr, nchains, npars, nfree, ndata, nprior, chainsize, burnin, nold;
   double gamma, fepsilon;
   int ifree[kMaxPars];
   int share_dst[kMaxPars], share_src[kMaxPars], nshare;
   int iprior[kMaxPars];
-  const double *pmin, *pmax, *prior, *priorlow, *data, *uncert;
-  double *params, *nextp, *currchisq, *nextchisq, *c2, *bestp, *bestchisq, *bestmodel;
-  double *numaccept, *allparams;
+  const double *pmin, *pmax, *prior, *priorlow;   // shared, [npars]
+  const double *data, *uncert;                    // per retrieval, [nretr][ndata]
+  double *params, *nextp, *currchisq, *nextchisq, *c2;   // per chain
+  double *bestp, *bestchisq, *bestmodel;          // per retrieval: [nretr][npars], [nretr], [nretr][ndata]
+  double *numaccept, *allparams;                  // per chain; allparams[g][nfree][chainsize]
   // MC3's `savemodel` trace (mcmc.py:636-651): the model of every chain's CURRENT state after each
-  // generation, allmodel[chain][datum][iteration].  curmodel starts as zeros, like the reference's
+  // generation, allmodel[g][datum][iteration].  curmodel starts as zeros, like the reference's
   // `allmodel[~accepted,:,i+nold-1]` with i + nold - 1 = -1 at the first generation.
   double *curmodel, *allmodel;
-  int *outbounds, *outflag, *iter;
-  // random streams of this run, MC3's shapes (mcmc.py:484-507)
-  const double *support;   // [chainsize][nchains][nfree]
-  const int *r1, *r2;      // [nchains][chainsize]
-  const double *unif;      // [chainsize][nchains]
-  const double *ugamma;    // [chainsize][nchains]
+  int *outbounds, *outflag;
+  // generation counter of each retrieval [nretr], advanced by that retrieval's chi-squared CTA (the
+  // only reader while it advances): generations replay as one captured graph
+  int *iter;
+  // random streams of this run, MC3's shapes (mcmc.py:484-507) behind a leading [nretr]
+  const double *support;   // [nretr][chainsize][nchains][nfree]
+  const int *r1, *r2;      // [nretr][nchains][chainsize], chain indices within the retrieval
+  const double *unif;      // [nretr][chainsize][nchains]
+  const double *ugamma;    // [nretr][chainsize][nchains]
   // walk = 1: snooker (mcmc.py:357-460,527-561,603-609,653-660)
   int walk, hsize, thinning;
-  double *Z;               // [zcap][nchains][npars] sample history; rows carry the chains'
-                           // initial non-free columns like the reference's (mcmc.py:419,425)
-  double *Zchisq;          // [zcap][nchains]
-  int *zsize;              // rows filled so far (device counter, advances with the generations)
-  double *zbest;           // [1 + npars + ndata] best initial Z sample: chisq, params, model
-  const int *i1, *i2;      // [chainsize][nchains] flat (row, chain) indices into Z
-  const int *iz, *ic;      // [chainsize][nchains]
-  const double *usn;       // [sum of snooker chains][nfree] uniform(1.2, 2.2) factors
-  const int *usn_off;      // [chainsize + 1] first row of generation i in usn
-  int *noproj;             // [nchains] scratch: z == current state (mcmc.py:543)
-  int *slot;               // [nchains] scratch: row of the chain's factors in usn
+  double *Z;               // [zcap][nretr][nchains][npars] sample history (zidx); rows carry the
+                           // chains' initial non-free columns like the reference's (mcmc.py:419,425)
+  double *Zchisq;          // [zcap][nretr][nchains]
+  int *zsize;              // [nretr] rows filled so far (advance with the generations, all equal)
+  double *zbest;           // [nretr][1 + npars + ndata] best initial Z sample: chisq, params, model
+  const int *i1, *i2;      // [nretr][chainsize][nchains] flat (row, chain) indices into the retrieval's Z
+  const int *iz, *ic;      // [nretr][chainsize][nchains]
+  const double *usn;       // [sum of snooker chains][nfree] uniform(1.2, 2.2) factors, by retrieval
+  const int *usn_off;      // [nretr][chainsize + 1] first row of generation i in usn
+  int *noproj;             // per chain scratch: z == current state (mcmc.py:543)
+  int *slot;               // per chain scratch: row of the chain's factors in usn
 };
 
-// where chain c's model sits in the gathered band-flux buffer: rank blocks of `pad` rows
+// row `row`, chain c of retrieval r in the history: one row holds every retrieval's chains, so a
+// larger history is a prefix copy of a smaller one
+BART_HD size_t zidx(const McmcDev &mc, int row, int r, int c) {
+  return ((size_t)row * mc.nretr + r) * mc.nchains + c;
+}
+
+// where model g (of the flattened population) sits in the gathered band-flux buffer: rank blocks of
+// `pad` rows
 struct ModelMap { int world, base, extra, pad; };
 
+// one warp per (retrieval, chain)
 void launch_demc_propose(const McmcDev &mc, cudaStream_t s);
+// the launches below run one CTA per retrieval
 void launch_snooker_propose(const McmcDev &mc, cudaStream_t s);
-// chi-squared of Z row `row` (models of its nchains samples); keeps the running best in mc.zbest.
+// chi-squared of Z row `row` (models of its nretr x nchains samples); keeps each retrieval's running
+// best in mc.zbest.
 // last != 0: afterwards adopt zbest as the best fit when it beats the chains' (mcmc.py:462-470)
 void launch_zrow_chisq(const McmcDev &mc, const double *models, ModelMap map, int row, int last,
                        cudaStream_t s);

@@ -139,7 +139,7 @@ struct Config {
   DevBuf<int> d_snk_idx, d_snk_off;
   int mc_zsize = 0;                        // host mirror of the device row counter
   size_t mc_zcap = 0;                      // rows allocated
-  std::vector<double> mc_ztemplate;        // [nchains][npars] what an unfilled row holds
+  std::vector<double> mc_ztemplate;        // [nretr][nchains][npars] what an unfilled row holds
 };
 
 // The process: the device, its streams, the communicator and peer window, profiling and debug
@@ -775,7 +775,8 @@ static void mcmc_generation_queued(int first) {
     check_launch("demc_propose");
   }
   const double *models = mcmc_evaluate_queued(first ? mc.params : mc.nextp);
-  ModelMap mp{G.world, mc.nchains / G.world, mc.nchains % G.world, G.mc_pad};
+  const int ntot = mc.nretr * mc.nchains;
+  ModelMap mp{G.world, ntot / G.world, ntot % G.world, G.mc_pad};
   {
     KernelScope ks("chisq_accept");
     launch_chisq_accept(mc, models, mp, first, G.stream);
@@ -783,7 +784,7 @@ static void mcmc_generation_queued(int first) {
   }
 }
 
-// band fluxes of one population `d_params` [nchains][npars] (device): this rank's block of chains
+// band fluxes of one population `d_params` [nretr * nchains][npars] (device): this rank's block of chains
 // through the forward model, then the all-gather; returns the buffer chain_model() indexes
 static const double *mcmc_evaluate_queued(const double *d_params) {
   McmcDev &mc = G.mc;
@@ -845,7 +846,7 @@ static void rank_barrier() {
 // niter generations of the walk set up in G.mc, queued and awaited
 static void mcmc_run_generations(int niter) {
   McmcDev &mc = G.mc;
-  CUDA_OK(cudaMemsetAsync(mc.iter, 0, sizeof(int), G.stream));
+  CUDA_OK(cudaMemsetAsync(mc.iter, 0, (size_t)mc.nretr * sizeof(int), G.stream));
   if (G.mc_graph) { cudaGraphExecDestroy(G.mc_graph); G.mc_graph = nullptr; }
   ensure_params_buffers(G.mc_hi - G.mc_lo);
   // One generation is a fixed sequence of launches whose only varying input, the iteration
@@ -1840,18 +1841,24 @@ void bart_chain_block(int nchains, int world, int rank, int *lo, int *hi) {
   chain_block(nchains, world, rank, lo, hi);
 }
 
-// replaces the set-up and initial evaluation of MCcubed.mc.mcmc (mcmc.py:196-345) for walk='demc'
-int bart_mcmc_init(int nchains, int npars, const double *params, const double *pmin,
-                   const double *pmax, const double *stepsize, const double *prior,
-                   const double *priorlow, int ndata, const double *data, const double *uncert,
-                   double fgamma, double fepsilon, int burnin) {
+// replaces the set-up and initial evaluation of MCcubed.mc.mcmc (mcmc.py:196-345) for walk='demc',
+// for `nretr` independent retrievals in one loop: params[nretr][nchains][npars],
+// data / uncert[nretr][ndata]; bounds, step sizes and priors shared
+int bart_mcmc_init_ensemble(int nretr, int nchains, int npars, const double *params,
+                            const double *pmin, const double *pmax, const double *stepsize,
+                            const double *prior, const double *priorlow, int ndata,
+                            const double *data, const double *uncert, double fgamma,
+                            double fepsilon, int burnin) {
   API_BEGIN
   if (!G.conv.ready) fail("bart_converter_init has not been called");
+  if (nretr < 1) fail("bart_mcmc_init: %d retrievals (need at least 1)", nretr);
   if (npars != G.conv.npars) fail("bart_mcmc_init: %d parameters, the converter expects %d", npars, G.conv.npars);
   if (ndata != G.nfilters) fail("bart_mcmc_init: %d data points but %d filters", ndata, G.nfilters);
   if (nchains < 3) fail("DE-MC needs at least 3 chains (got %d)", nchains);
+  const int ntot = nretr * nchains;              // the flattened population
   McmcDev mc{};
-  mc.nchains = nchains; mc.npars = npars; mc.ndata = ndata; mc.burnin = burnin; mc.nold = 0;
+  mc.nretr = nretr; mc.nchains = nchains; mc.npars = npars; mc.ndata = ndata; mc.burnin = burnin;
+  mc.nold = 0;
   mc.fepsilon = fepsilon;
   for (int p = 0; p < npars; p++) {
     if (stepsize[p] > 0) mc.ifree[mc.nfree++] = p;
@@ -1875,33 +1882,34 @@ int bart_mcmc_init(int nchains, int npars, const double *params, const double *p
   auto &mb = G.mcb;
   mc.pmin = up(mb.pmin, pmin, npars); mc.pmax = up(mb.pmax, pmax, npars);
   mc.prior = up(mb.prior, prior, npars); mc.priorlow = up(mb.priorlow, priorlow, npars);
-  mc.data = up(mb.data, data, ndata); mc.uncert = up(mb.uncert, uncert, ndata);
-  std::vector<double> p0(params, params + (size_t)nchains * npars);
-  for (int c = 0; c < nchains; c++)
+  mc.data = up(mb.data, data, (size_t)nretr * ndata); mc.uncert = up(mb.uncert, uncert, (size_t)nretr * ndata);
+  std::vector<double> p0(params, params + (size_t)ntot * npars);
+  for (int g = 0; g < ntot; g++)
     for (int s = 0; s < mc.nshare; s++)
-      p0[(size_t)c * npars + mc.share_dst[s]] = p0[(size_t)c * npars + mc.share_src[s]];
+      p0[(size_t)g * npars + mc.share_dst[s]] = p0[(size_t)g * npars + mc.share_src[s]];
   mc.params = up(mb.params, p0.data(), p0.size());
   mc.nextp = up(mb.nextp, p0.data(), p0.size());
-  mc.currchisq = up(mb.currchisq, nullptr, nchains); mc.nextchisq = up(mb.nextchisq, nullptr, nchains);
-  mc.c2 = up(mb.c2, nullptr, nchains); mc.bestp = up(mb.bestp, nullptr, npars);
-  mc.bestchisq = up(mb.bestchisq, nullptr, 1); mc.bestmodel = up(mb.bestmodel, nullptr, ndata);
-  mc.numaccept = up(mb.numaccept, nullptr, nchains);
-  std::vector<int> zi((size_t)nchains * mc.nfree, 0);
+  mc.currchisq = up(mb.currchisq, nullptr, ntot); mc.nextchisq = up(mb.nextchisq, nullptr, ntot);
+  mc.c2 = up(mb.c2, nullptr, ntot); mc.bestp = up(mb.bestp, nullptr, (size_t)nretr * npars);
+  mc.bestchisq = up(mb.bestchisq, nullptr, nretr);
+  mc.bestmodel = up(mb.bestmodel, nullptr, (size_t)nretr * ndata);
+  mc.numaccept = up(mb.numaccept, nullptr, ntot);
+  std::vector<int> zi((size_t)ntot * mc.nfree, 0);
   upload(mb.outbounds, zi); mc.outbounds = mb.outbounds.p;
-  zi.assign(nchains, 0); upload(mb.outflag, zi); mc.outflag = mb.outflag.p;
-  zi.assign(1, 0); upload(mb.iter, zi); mc.iter = mb.iter.p;
+  zi.assign(ntot, 0); upload(mb.outflag, zi); mc.outflag = mb.outflag.p;
+  zi.assign(nretr, 0); upload(mb.iter, zi); mc.iter = mb.iter.p;
   G.mc = mc;
   G.mc_ztemplate = p0;
   G.mc_zsize = 0;
-  chain_block(nchains, G.world, G.rank, &G.mc_lo, &G.mc_hi);
-  G.mc_pad = nchains / G.world + (nchains % G.world ? 1 : 0);
+  chain_block(ntot, G.world, G.rank, &G.mc_lo, &G.mc_hi);
+  G.mc_pad = ntot / G.world + (ntot % G.world ? 1 : 0);
   G.d_mcband.ensure((size_t)G.mc_pad * ndata);
   G.d_mcgather.ensure((size_t)G.mc_pad * ndata * G.world);
   CUDA_OK(cudaMemsetAsync(G.d_mcband.p, 0, (size_t)G.mc_pad * ndata * 8, G.stream));
-  G.d_mccur.ensure((size_t)nchains * ndata);
-  CUDA_OK(cudaMemsetAsync(G.d_mccur.p, 0, (size_t)nchains * ndata * 8, G.stream));
+  G.d_mccur.ensure((size_t)ntot * ndata);
+  CUDA_OK(cudaMemsetAsync(G.d_mccur.p, 0, (size_t)ntot * ndata * 8, G.stream));
   G.mc.curmodel = G.d_mccur.p;
-  G.d_mcallm.ensure((size_t)nchains * ndata);              // the initial evaluation writes no trace
+  G.d_mcallm.ensure((size_t)ntot * ndata);                 // the initial evaluation writes no trace
   G.mc.allmodel = G.d_mcallm.p;
   if (G.mc_graph) { cudaGraphExecDestroy(G.mc_graph); G.mc_graph = nullptr; }
   ensure_params_buffers(G.mc_hi - G.mc_lo);
@@ -1914,6 +1922,18 @@ int bart_mcmc_init(int nchains, int npars, const double *params, const double *p
   API_END_INT
 }
 
+// replaces the set-up and initial evaluation of MCcubed.mc.mcmc (mcmc.py:196-345) for walk='demc':
+// an ensemble of one
+int bart_mcmc_init(int nchains, int npars, const double *params, const double *pmin,
+                   const double *pmax, const double *stepsize, const double *prior,
+                   const double *priorlow, int ndata, const double *data, const double *uncert,
+                   double fgamma, double fepsilon, int burnin) {
+  return bart_mcmc_init_ensemble(1, nchains, npars, params, pmin, pmax, stepsize, prior, priorlow,
+                                 ndata, data, uncert, fgamma, fepsilon, burnin);
+}
+
+int bart_mcmc_nretr(void) { return G.mc_ready ? G.mc.nretr : 0; }
+
 // MC3's resume=True for walk='demc' (mcmc.py:254-269): iterations of the previous run count towards
 // burn-in and the savemodel trace continues from the previous run's last column
 int bart_mcmc_resume(int nold, const double *curmodel) {
@@ -1924,7 +1944,7 @@ int bart_mcmc_resume(int nold, const double *curmodel) {
   if (nold < 0) fail("bart_mcmc_resume: nold = %d", nold);
   mc.nold = nold;
   if (curmodel)
-    CUDA_OK(cudaMemcpyAsync(G.d_mccur.p, curmodel, (size_t)mc.nchains * mc.ndata * 8,
+    CUDA_OK(cudaMemcpyAsync(G.d_mccur.p, curmodel, (size_t)mc.nretr * mc.nchains * mc.ndata * 8,
                             cudaMemcpyHostToDevice, G.stream));
   finish_stream();
   return 0;
@@ -1940,17 +1960,24 @@ int bart_mcmc_run(int niter, const double *support, const int *r1, const int *r2
   if (niter <= 0) return 0;
   McmcDev &mc = G.mc;
   const int nc = mc.nchains;
-  for (size_t k = 0; k < (size_t)nc * niter; k++)
-    if (r1[k] < 0 || r1[k] >= nc || r2[k] < 0 || r2[k] >= nc) fail("chain index out of range in r1/r2");
+  const size_t n1 = (size_t)mc.nretr * nc * niter;       // every stream has nretr x niter x nchains entries
+  for (int r = 0; r < mc.nretr; r++)
+    for (int c = 0; c < nc; c++)
+      for (int i = 0; i < niter; i++) {
+        const size_t k = ((size_t)r * nc + c) * niter + i;
+        if (r1[k] < 0 || r1[k] >= nc || r2[k] < 0 || r2[k] >= nc)
+          fail("chain index out of range in r1/r2: retrieval %d, generation %d, chain %d (r1 %d, r2 %d, "
+               "%d chains)", r, i, c, r1[k], r2[k], nc);
+      }
   mc.nold += mc.chainsize;               // iterations of earlier calls count towards burn-in
   mc.chainsize = niter;
-  mc.support = upload_queued(G.mcb.support, support, (size_t)niter * nc * mc.nfree);
-  mc.unif = upload_queued(G.mcb.unif, unif, (size_t)niter * nc);
-  mc.ugamma = upload_queued(G.mcb.ugamma, ugamma, (size_t)niter * nc);
-  mc.r1 = upload_queued(G.mcb.r1, r1, (size_t)nc * niter);
-  mc.r2 = upload_queued(G.mcb.r2, r2, (size_t)nc * niter);
-  mc.allparams = G.mcb.allparams.ensure((size_t)nc * mc.nfree * niter);
-  G.d_mcallm.ensure((size_t)nc * mc.ndata * niter);
+  mc.support = upload_queued(G.mcb.support, support, n1 * mc.nfree);
+  mc.unif = upload_queued(G.mcb.unif, unif, n1);
+  mc.ugamma = upload_queued(G.mcb.ugamma, ugamma, n1);
+  mc.r1 = upload_queued(G.mcb.r1, r1, n1);
+  mc.r2 = upload_queued(G.mcb.r2, r2, n1);
+  mc.allparams = G.mcb.allparams.ensure(n1 * mc.nfree);
+  G.d_mcallm.ensure(n1 * mc.ndata);
   mc.allmodel = G.d_mcallm.p;
   mc.walk = 0;
   mcmc_run_generations(niter);
@@ -1966,17 +1993,18 @@ int bart_mcmc_run(int niter, const double *support, const int *r1, const int *r2
 static void snooker_reserve_rows(size_t rows) {
   McmcDev &mc = G.mc;
   if (rows <= G.mc_zcap) return;
-  const size_t rowlen = (size_t)mc.nchains * mc.npars;
+  const size_t rowchains = (size_t)mc.nretr * mc.nchains;    // a row holds every retrieval's chains
+  const size_t rowlen = rowchains * mc.npars;
   rows += rows / 2 + 16;
   DevBuf<double> nz, nc;
-  nz.ensure(rows * rowlen); nc.ensure(rows * mc.nchains);
+  nz.ensure(rows * rowlen); nc.ensure(rows * rowchains);
   std::vector<double> fill(rows * rowlen);
   for (size_t r = 0; r < rows; r++) std::copy(G.mc_ztemplate.begin(), G.mc_ztemplate.end(), fill.begin() + r * rowlen);
   CUDA_OK(cudaMemcpyAsync(nz.p, fill.data(), fill.size() * 8, cudaMemcpyHostToDevice, G.stream));
-  CUDA_OK(cudaMemsetAsync(nc.p, 0, rows * mc.nchains * 8, G.stream));
+  CUDA_OK(cudaMemsetAsync(nc.p, 0, rows * rowchains * 8, G.stream));
   if (G.mc_zsize > 0) {
     CUDA_OK(cudaMemcpyAsync(nz.p, G.d_Z.p, (size_t)G.mc_zsize * rowlen * 8, cudaMemcpyDeviceToDevice, G.stream));
-    CUDA_OK(cudaMemcpyAsync(nc.p, G.d_Zchisq.p, (size_t)G.mc_zsize * mc.nchains * 8, cudaMemcpyDeviceToDevice, G.stream));
+    CUDA_OK(cudaMemcpyAsync(nc.p, G.d_Zchisq.p, (size_t)G.mc_zsize * rowchains * 8, cudaMemcpyDeviceToDevice, G.stream));
   }
   CUDA_OK(cudaStreamSynchronize(G.stream));
   G.d_Z = std::move(nz); G.d_Zchisq = std::move(nc);
@@ -1995,38 +2023,42 @@ int bart_mcmc_snooker_init(int hsize, int thinning, const double *z0) {
   McmcDev &mc = G.mc;
   if (hsize < 2) fail("snooker needs hsize >= 2 (got %d)", hsize);
   if (thinning < 1) fail("thinning must be >= 1 (got %d)", thinning);
-  const int nc = mc.nchains, np = mc.npars;
-  // fixed parameters of every Z sample are chain 0's (mcmc.py:425)
-  for (int c = 0; c < nc; c++)
+  const int nc = mc.nchains, np = mc.npars, nr = mc.nretr, ntot = nr * nc;
+  // fixed parameters of every Z sample are chain 0's of its retrieval (mcmc.py:425)
+  for (int g = 0; g < ntot; g++)
     for (int p = 0; p < np; p++) {
       bool fixed = true;
       for (int f = 0; f < mc.nfree; f++) fixed &= mc.ifree[f] != p;
       for (int k = 0; k < mc.nshare; k++) fixed &= mc.share_dst[k] != p;
-      if (fixed) G.mc_ztemplate[(size_t)c * np + p] = G.mc_ztemplate[p];
+      if (fixed) G.mc_ztemplate[(size_t)g * np + p] = G.mc_ztemplate[(size_t)(g / nc) * nc * np + p];
     }
   G.mc_zsize = 0; G.mc_zcap = 0;
   snooker_reserve_rows((size_t)hsize + 64);
-  std::vector<double> rows((size_t)hsize * nc * np);
-  for (int r = 0; r < hsize; r++)
-    for (int c = 0; c < nc; c++) {
-      double *dst = &rows[((size_t)r * nc + c) * np];
-      std::copy(&G.mc_ztemplate[(size_t)c * np], &G.mc_ztemplate[(size_t)c * np] + np, dst);
-      for (int f = 0; f < mc.nfree; f++) dst[mc.ifree[f]] = z0[((size_t)r * nc + c) * mc.nfree + f];
-    }
+  // z0[nretr][hsize][nchains][nfree] -> rows [hsize][nretr][nchains][npars]
+  std::vector<double> rows((size_t)hsize * ntot * np);
+  for (int r = 0; r < nr; r++)
+    for (int row = 0; row < hsize; row++)
+      for (int c = 0; c < nc; c++) {
+        const size_t g = (size_t)r * nc + c;
+        double *dst = &rows[zidx(mc, row, r, c) * np];
+        std::copy(&G.mc_ztemplate[g * np], &G.mc_ztemplate[g * np] + np, dst);
+        const double *src = z0 + (((size_t)r * hsize + row) * nc + c) * mc.nfree;
+        for (int f = 0; f < mc.nfree; f++) dst[mc.ifree[f]] = src[f];
+      }
   CUDA_OK(cudaMemcpyAsync(mc.Z, rows.data(), rows.size() * 8, cudaMemcpyHostToDevice, G.stream));
-  std::vector<int> zi(1, hsize);
+  std::vector<int> zi(nr, hsize);
   upload(G.mcb.zsize, zi); mc.zsize = G.mcb.zsize.p;
-  zi.assign(nc, 0);
+  zi.assign(ntot, 0);
   upload(G.mcb.noproj, zi); mc.noproj = G.mcb.noproj.p;
   upload(G.mcb.slot, zi); mc.slot = G.mcb.slot.p;
-  mc.zbest = G.mcb.zbest.ensure(1 + np + mc.ndata);
+  mc.zbest = G.mcb.zbest.ensure((size_t)nr * (1 + np + mc.ndata));
   mc.hsize = hsize; mc.thinning = thinning; mc.walk = 1;
   ensure_params_buffers(G.mc_hi - G.mc_lo);
-  ModelMap mp{G.world, nc / G.world, nc % G.world, G.mc_pad};
-  for (int r = 0; r < hsize; r++) {
-    const double *models = mcmc_evaluate_queued(mc.Z + (size_t)r * nc * np);
+  ModelMap mp{G.world, ntot / G.world, ntot % G.world, G.mc_pad};
+  for (int row = 0; row < hsize; row++) {
+    const double *models = mcmc_evaluate_queued(mc.Z + zidx(mc, row, 0, 0) * np);
     KernelScope ks("zrow_chisq");
-    launch_zrow_chisq(mc, models, mp, r, r == hsize - 1, G.stream);
+    launch_zrow_chisq(mc, models, mp, row, row == hsize - 1, G.stream);
     check_launch("zrow_chisq");
   }
   finish_stream();
@@ -2051,45 +2083,53 @@ int bart_mcmc_run_snooker(int niter, const double *support, const int *i1, const
   if (!G.mc_ready || G.mc_zsize < 2) fail("bart_mcmc_snooker_init has not been called");
   if (niter <= 0) return 0;
   McmcDev &mc = G.mc;
-  const int nc = mc.nchains;
-  // validate the indices against the history size each generation will see
-  {
-    int zs = G.mc_zsize;
+  const int nc = mc.nchains, nr = mc.nretr;
+  // validate the indices against the history size each generation will see (every retrieval's
+  // history grows on the same schedule); usn_offset[nretr][niter + 1] are absolute rows of usnooker,
+  // the retrievals' factors one after the other
+  int zs = G.mc_zsize;
+  for (int r = 0; r < nr; r++) {
+    zs = G.mc_zsize;
+    const int *off = usn_offset + (size_t)r * (niter + 1);
+    if (r > 0 && off[0] != off[-1])
+      fail("usn_offset: retrieval %d starts at row %d, retrieval %d ended at row %d", r, off[0], r - 1, off[-1]);
     for (int i = 0; i < niter; i++) {
       int nsj = 0;
       for (int c = 0; c < nc; c++) {
-        const size_t k = (size_t)i * nc + c;
+        const size_t k = ((size_t)r * niter + i) * nc + c;
         const long long lim = (long long)(zs - 1) * nc;
         if (i1[k] < 0 || i1[k] >= lim || i2[k] < 0 || i2[k] >= lim || iz[k] < 0 || iz[k] >= zs - 1 ||
             ic[k] < 0 || ic[k] >= nc)
-          fail("snooker index out of range at generation %d, chain %d (history rows %d)", i, c, zs);
+          fail("snooker index out of range: retrieval %d, generation %d, chain %d (history rows %d)", r,
+               i, c, zs);
         nsj += ugamma[k] < 0.1;
       }
-      if (usn_offset[i + 1] - usn_offset[i] != nsj || usn_offset[i] < 0)
-        fail("usn_offset: generation %d has %d snooker chains but %d rows of factors", i, nsj,
-             usn_offset[i + 1] - usn_offset[i]);
+      if (off[i + 1] - off[i] != nsj || off[i] < 0)
+        fail("usn_offset: retrieval %d, generation %d has %d snooker chains but %d rows of factors", r,
+             i, nsj, off[i + 1] - off[i]);
       if ((mc.nold + mc.chainsize + i) % mc.thinning == 0) zs++;   // global iteration number
     }
-    snooker_reserve_rows((size_t)zs + 1);
-    G.mc_zsize = zs;
   }
+  snooker_reserve_rows((size_t)zs + 1);
+  G.mc_zsize = zs;
   mc.nold += mc.chainsize;
   mc.chainsize = niter;
   // i1, i2, iz, ic packed in one buffer; usn_offset in another
-  const size_t n1 = (size_t)niter * nc;
+  const size_t n1 = (size_t)nr * niter * nc;
   std::vector<int> packed(4 * n1);
   std::copy(i1, i1 + n1, packed.begin()); std::copy(i2, i2 + n1, packed.begin() + n1);
   std::copy(iz, iz + n1, packed.begin() + 2 * n1); std::copy(ic, ic + n1, packed.begin() + 3 * n1);
   const int *pk = upload_queued(G.d_snk_idx, packed.data(), packed.size());
   CUDA_OK(cudaStreamSynchronize(G.stream));
   mc.i1 = pk; mc.i2 = pk + n1; mc.iz = pk + 2 * n1; mc.ic = pk + 3 * n1;
-  mc.usn_off = upload_queued(G.d_snk_off, usn_offset, (size_t)niter + 1);
-  mc.usn = upload_queued(G.d_snk_usn, usnooker, (size_t)usn_offset[niter] * mc.nfree);
+  const size_t noff = (size_t)nr * (niter + 1);
+  mc.usn_off = upload_queued(G.d_snk_off, usn_offset, noff);
+  mc.usn = upload_queued(G.d_snk_usn, usnooker, (size_t)usn_offset[noff - 1] * mc.nfree);
   mc.support = upload_queued(G.mcb.support, support, n1 * mc.nfree);
   mc.unif = upload_queued(G.mcb.unif, unif, n1);
   mc.ugamma = upload_queued(G.mcb.ugamma, ugamma, n1);
-  mc.allparams = G.mcb.allparams.ensure((size_t)nc * mc.nfree * niter);
-  G.d_mcallm.ensure((size_t)nc * mc.ndata * niter);
+  mc.allparams = G.mcb.allparams.ensure(n1 * mc.nfree);
+  G.d_mcallm.ensure(n1 * mc.ndata);
   mc.allmodel = G.d_mcallm.p;
   mc.walk = 1;
   mcmc_run_generations(niter);
@@ -2100,38 +2140,52 @@ int bart_mcmc_run_snooker(int niter, const double *support, const int *i1, const
 // results of the DE-MC loop: "allparams" [nchains][nfree][niter of the last run] (MC3's trace
 // layout), "params" [nchains][npars], "currchisq", "numaccept" [nchains], "outbounds"
 // [nchains][nfree], "bestp" [npars], "bestchisq" [1], "bestmodel" [ndata], "models" (band fluxes of
-// the last generation, [nchains][ndata]).  Returns the number of doubles written, or < 0.
+// the last generation, [nchains][ndata]), each behind a leading [nretr]; "Z" [nretr][Zsize]
+// [nchains][npars], "Zchisq" [nretr][Zsize][nchains].  Returns the number of doubles written, or < 0.
 long long bart_mcmc_get(const char *name, double *out, long long capacity) {
   API_BEGIN
   if (!G.mc_ready) fail("bart_mcmc_init has not been called");
   const McmcDev &mc = G.mc;
+  const long long ntot = (long long)mc.nretr * mc.nchains;
   std::string n(name);
   const double *src = nullptr;
   long long cnt = 0;
-  if (n == "allparams") { src = mc.allparams; cnt = (long long)mc.nchains * mc.nfree * mc.chainsize; }
-  else if (n == "allmodel") { src = mc.allmodel; cnt = (long long)mc.nchains * mc.ndata * mc.chainsize; }
-  else if (n == "params") { src = mc.params; cnt = (long long)mc.nchains * mc.npars; }
-  else if (n == "currchisq") { src = mc.currchisq; cnt = mc.nchains; }
-  else if (n == "numaccept") { src = mc.numaccept; cnt = mc.nchains; }
-  else if (n == "bestp") { src = mc.bestp; cnt = mc.npars; }
-  else if (n == "bestchisq") { src = mc.bestchisq; cnt = 1; }
-  else if (n == "bestmodel") { src = mc.bestmodel; cnt = mc.ndata; }
-  else if (n == "Z") { src = mc.Z; cnt = (long long)G.mc_zsize * mc.nchains * mc.npars; }
-  else if (n == "Zchisq") { src = mc.Zchisq; cnt = (long long)G.mc_zsize * mc.nchains; }
+  if (n == "allparams") { src = mc.allparams; cnt = ntot * mc.nfree * mc.chainsize; }
+  else if (n == "allmodel") { src = mc.allmodel; cnt = ntot * mc.ndata * mc.chainsize; }
+  else if (n == "params") { src = mc.params; cnt = ntot * mc.npars; }
+  else if (n == "currchisq") { src = mc.currchisq; cnt = ntot; }
+  else if (n == "numaccept") { src = mc.numaccept; cnt = ntot; }
+  else if (n == "bestp") { src = mc.bestp; cnt = (long long)mc.nretr * mc.npars; }
+  else if (n == "bestchisq") { src = mc.bestchisq; cnt = mc.nretr; }
+  else if (n == "bestmodel") { src = mc.bestmodel; cnt = (long long)mc.nretr * mc.ndata; }
+  else if (n == "Z" || n == "Zchisq") {
+    // device rows [Zsize][nretr][nchains](...) -> retrieval-major [nretr][Zsize][nchains](...)
+    if (!mc.Z) return 0;
+    const long long w = n == "Z" ? mc.npars : 1, rowlen = ntot * w, blk = (long long)mc.nchains * w;
+    cnt = (long long)G.mc_zsize * rowlen;
+    if (cnt > capacity) fail("bart_mcmc_get(%s): capacity %lld < %lld", name, capacity, cnt);
+    std::vector<double> tmp(cnt);
+    if (cnt) CUDA_OK(cudaMemcpy(tmp.data(), n == "Z" ? mc.Z : mc.Zchisq, cnt * 8, cudaMemcpyDeviceToHost));
+    for (int r = 0; r < mc.nretr; r++)
+      for (int row = 0; row < G.mc_zsize; row++)
+        std::copy(&tmp[row * rowlen + r * blk], &tmp[row * rowlen + r * blk] + blk,
+                  out + ((long long)r * G.mc_zsize + row) * blk);
+    return cnt;
+  }
   else if (n == "outbounds") {
-    cnt = (long long)mc.nchains * mc.nfree;
+    cnt = ntot * mc.nfree;
     if (cnt > capacity) fail("bart_mcmc_get(%s): capacity %lld < %lld", name, capacity, cnt);
     std::vector<int> tmp(cnt);
     CUDA_OK(cudaMemcpy(tmp.data(), mc.outbounds, cnt * 4, cudaMemcpyDeviceToHost));
     for (long long i = 0; i < cnt; i++) out[i] = tmp[i];
     return cnt;
   } else if (n == "models") {
-    cnt = (long long)mc.nchains * mc.ndata;
+    cnt = ntot * mc.ndata;
     if (cnt > capacity) fail("bart_mcmc_get(%s): capacity %lld < %lld", name, capacity, cnt);
     const double *base = G.world > 1 ? G.d_mcgather.p : G.d_mcband.p;
     for (int r = 0; r < G.world; r++) {
       int lo, hi;
-      chain_block(mc.nchains, G.world, r, &lo, &hi);
+      chain_block((int)ntot, G.world, r, &lo, &hi);
       if (hi > lo)
         CUDA_OK(cudaMemcpy(out + (size_t)lo * mc.ndata, base + (size_t)r * G.mc_pad * mc.ndata,
                            (size_t)(hi - lo) * mc.ndata * 8, cudaMemcpyDeviceToHost));

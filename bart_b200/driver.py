@@ -259,6 +259,20 @@ def demc_draws(rng, nchains, chainsize, step_free):
     return dict(support=support, r1=r1, r2=r2, unif=unif, ugamma=ugamma)
 
 
+def start_points(params, nchains, stepsize, pmin, pmax, rng):
+    """The chains' starting points (mcmc.py:296-306): `params` as given when it has a row per chain,
+    else chain 0 at params[0] and the others scattered around it by normal(0, stepsize) draws from
+    `rng`, clipped to [pmin, pmax]."""
+    params = np.atleast_2d(np.array(params, dtype=float))
+    if params.shape[0] != nchains:
+        params = np.repeat(params, nchains, 0)
+        for p in np.where(stepsize > 0)[0]:
+            params[1:, p] = rng.normal(params[0, p], stepsize[p], nchains - 1)
+            params[np.where(params[:, p] < pmin[p]), p] = pmin[p]
+            params[np.where(params[:, p] > pmax[p]), p] = pmax[p]
+    return params
+
+
 def run_demc(transit, data, uncert, params, pmin, pmax, stepsize, numit, nchains, prior=None,
              priorlow=None, burnin=0, fgamma=1.0, fepsilon=0.0, rng=np.random, draws=None,
              savefile=None, savemodel=None, grtest=False, grexit=False, thinning=1, resume=False):
@@ -282,12 +296,7 @@ def run_demc(transit, data, uncert, params, pmin, pmax, stepsize, numit, nchains
             oldmodel = np.load(savemodel)
         params = np.repeat(params[:1], nchains, 0)
         params[:, ifree] = oldparams[:, :, -1]
-    if params.shape[0] != nchains:                                   # mcmc.py:296-306
-        params = np.repeat(params, nchains, 0)
-        for p in ifree:
-            params[1:, p] = rng.normal(params[0, p], stepsize[p], nchains - 1)
-            params[np.where(params[:, p] < pmin[p]), p] = pmin[p]
-            params[np.where(params[:, p] > pmax[p]), p] = pmax[p]
+    params = start_points(params, nchains, stepsize, pmin, pmax, rng)
     transit.mcmc_init(params, pmin, pmax, stepsize, data, uncert, prior=prior, priorlow=priorlow,
                       fgamma=fgamma, fepsilon=fepsilon, burnin=burnin)
     if resume:
@@ -333,14 +342,17 @@ def gr_checkpoints(chainsize):
 
 
 def run_segments(run, fetch, chainsize, burnin=0, thinning=1, grtest=False, grexit=False, nold=0,
-                 old=None):
+                 old=None, max_segment=None):
     """Drive a device-resident walk in the segments MC3's loop is observable in (mcmc.py:662-690).
     `run(lo, hi)` advances generations [lo, hi) (state stays on the device); `fetch()` returns that
-    call's allparams / allmodel pieces.  Without grtest it is one segment.  `old` = (allparams,
-    allmodel) of the run being resumed (nold iterations).  Returns (allparams, allmodel, psrf
+    call's allparams / allmodel pieces.  Without grtest it is one segment; `max_segment` caps the
+    generations of one call (the host arrays of a call stay bounded).  `old` = (allparams,
+    allmodel) of the run being resumed (nold iterations).  Traces of an ensemble carry a leading
+    retrieval axis, and its psrf is [retrieval][nfree].  Returns (allparams, allmodel, psrf
     history [(iteration, psrf)], number of iterations in the traces)."""
     cuts = gr_checkpoints(chainsize) if grtest else []
-    edges = sorted(set([c + 1 for c in cuts] + [chainsize]))
+    bounds = list(range(max_segment, chainsize, max_segment)) if max_segment else []
+    edges = sorted(set([c + 1 for c in cuts] + bounds + [chainsize]))
     pieces_p, pieces_m, history = [], [], []
     if old is not None:
         pieces_p.append(old[0]); pieces_m.append(old[1])
@@ -352,8 +364,11 @@ def run_segments(run, fetch, chainsize, burnin=0, thinning=1, grtest=False, grex
         lo = hi
         i = hi - 1
         if grtest and i in cuts and (i + nold) > burnin:
-            allp = np.concatenate(pieces_p, axis=2)
-            psrf = gelman_rubin(allp[:, :, burnin:i + nold + 1:thinning])
+            allp = np.concatenate(pieces_p, axis=-1)
+            if allp.ndim == 4:
+                psrf = np.array([gelman_rubin(a[:, :, burnin:i + nold + 1:thinning]) for a in allp])
+            else:
+                psrf = gelman_rubin(allp[:, :, burnin:i + nold + 1:thinning])
             history.append((i, psrf))
             if np.all(psrf < 1.01):
                 if grexit and grflag:                        # two consecutive passes (mcmc.py:676-683)
@@ -361,7 +376,7 @@ def run_segments(run, fetch, chainsize, burnin=0, thinning=1, grtest=False, grex
                 grflag = True
             else:
                 grflag = False
-    return np.concatenate(pieces_p, axis=2), np.concatenate(pieces_m, axis=2), history, nold + lo
+    return np.concatenate(pieces_p, axis=-1), np.concatenate(pieces_m, axis=-1), history, nold + lo
 
 
 def _save_mc3_files(out, savefile, savemodel):
@@ -423,12 +438,7 @@ def run_snooker(transit, data, uncert, params, pmin, pmax, stepsize, numit, ncha
     chainsize = int(np.ceil(numit / nchains))
     if hsize < nchains:                                              # mcmc.py:233-235
         hsize = nchains + 1
-    if params.shape[0] != nchains:                                   # mcmc.py:296-306
-        params = np.repeat(params, nchains, 0)
-        for p in ifree:
-            params[1:, p] = rng.normal(params[0, p], stepsize[p], nchains - 1)
-            params[np.where(params[:, p] < pmin[p]), p] = pmin[p]
-            params[np.where(params[:, p] > pmax[p]), p] = pmax[p]
+    params = start_points(params, nchains, stepsize, pmin, pmax, rng)
     transit.mcmc_init(params, pmin, pmax, stepsize, data, uncert, prior=prior, priorlow=priorlow,
                       fgamma=fgamma, fepsilon=fepsilon, burnin=burnin)
     if draws is None:
@@ -451,3 +461,150 @@ def run_snooker(transit, data, uncert, params, pmin, pmax, stepsize, numit, ncha
     out["allstack"] = np.hstack([allp[c, :, burnin:chainlen] for c in range(nchains)])
     _save_mc3_files(out, savefile, savemodel)
     return out
+
+
+# ---------------------------------------------------------------------------------------------
+# Ensembles: R independent retrievals of the same configuration in one device loop
+# (Transit.mcmc_init_ensemble); every generation evaluates R x nchains models as one batch.
+# Long runs go through the device in segments of at most _segment_cap generations, so the stacked
+# stream and trace arrays of one device call stay under ENSEMBLE_CALL_BYTES.  Total host memory is
+# not bounded: every retrieval's streams are drawn up front in MC3's order (what makes its chains
+# MC3's), and the returned traces hold every generation -- at R = 64, 10 chains, 9 free parameters
+# and 1e5 generations the `support` draws alone are 4.6 GB.
+ENSEMBLE_CALL_BYTES = 1 << 28          # host stream + trace arrays of one device call
+
+
+def stack_demc_draws(draws, lo, hi):
+    """Transit.mcmc_run's arguments for generations [lo, hi) of R retrievals' demc_draws."""
+    h = slice(lo, hi)
+    st = lambda k, cols: np.stack([d[k][:, h] if cols else d[k][h] for d in draws])
+    return st("support", 0), st("r1", 1), st("r2", 1), st("unif", 0), st("ugamma", 0)
+
+
+def stack_snooker_draws(draws, lo, hi):
+    """Transit.mcmc_run_snooker's arguments for generations [lo, hi) of R retrievals'
+    snooker_draws: each retrieval's factor rows one after the other, usn_offset[R][hi-lo+1] rebased
+    to absolute rows of the concatenation."""
+    h = slice(lo, hi)
+    usn, offs, base = [], [], 0
+    for d in draws:
+        off = np.asarray(d["usn_offset"])[lo:hi + 1]
+        usn.append(d["usnooker"][off[0]:off[-1]])
+        offs.append(off - off[0] + base)
+        base += off[-1] - off[0]
+    st = lambda k: np.stack([d[k][h] for d in draws])
+    return (st("support"), st("i1"), st("i2"), st("iz"), st("ic"), np.concatenate(usn),
+            np.stack(offs), st("unif"), st("ugamma"))
+
+
+def _ensemble_setup(data, uncert, params, pmin, pmax, stepsize, nchains, rngs, draws):
+    data = np.asarray(data, dtype=float)
+    uncert = np.asarray(uncert, dtype=float)
+    nretr = data.shape[0]
+    if nretr < 1 or data.ndim != 2 or uncert.shape != data.shape or len(params) != nretr:
+        raise ValueError("data, uncert and params need one entry per retrieval")
+    for name, v in (("rngs", rngs), ("draws", draws)):
+        if v is not None and len(v) != nretr:
+            raise ValueError("%s needs one entry per retrieval (%d)" % (name, nretr))
+    pmin, pmax, stepsize = (np.asarray(a, dtype=float) for a in (pmin, pmax, stepsize))
+    starts = []
+    for r in range(nretr):
+        rng = rngs[r] if rngs is not None else None
+        if rng is None and (np.atleast_2d(params[r]).shape[0] != nchains or draws is None):
+            raise ValueError("retrieval %d needs an rng (its start points or random streams are "
+                             "drawn)" % r)
+        starts.append(start_points(params[r], nchains, stepsize, pmin, pmax, rng))
+    return data, uncert, np.array(starts), pmin, pmax, stepsize
+
+
+def _segment_cap(nretr, nchains, nfree, ndata, extra=0):
+    """Generations of one device call so that its host arrays stay under ENSEMBLE_CALL_BYTES."""
+    per_gen = nretr * nchains * (8 * (2 * nfree + ndata + 2 + extra) + 2 * 4)
+    return max(1, int(ENSEMBLE_CALL_BYTES // per_gen))
+
+
+def _ensemble_results(transit, keys, allp, allm, history, chainlen, burnin, nchains, savefile,
+                      savemodel):
+    got = {k: transit.mcmc_get(k) for k in keys}
+    bestchisq = transit.mcmc_get("bestchisq")
+    outs = []
+    for r in range(allp.shape[0]):
+        out = {k: v[r] for k, v in got.items()}
+        out["allparams"], out["allmodel"] = allp[r], allm[r]
+        out["psrf"] = [(i, psrf[r]) for i, psrf in history]
+        out["bestchisq"] = float(bestchisq[r])
+        out["allstack"] = np.hstack([allp[r, c, :, burnin:chainlen] for c in range(nchains)])
+        _save_mc3_files(out, savefile[r] if savefile is not None else None,
+                        savemodel[r] if savemodel is not None else None)
+        outs.append(out)
+    return outs
+
+
+def run_demc_ensemble(transit, data, uncert, params, pmin, pmax, stepsize, numit, nchains,
+                      prior=None, priorlow=None, burnin=0, fgamma=1.0, fepsilon=0.0, rngs=None,
+                      draws=None, savefile=None, savemodel=None, grtest=False, grexit=False,
+                      thinning=1):
+    """`run_demc` for R retrievals of the same configuration in one device loop: data /
+    uncert[R][ndata], params[R] (each what run_demc takes: one start point, scattered with that
+    retrieval's rng as mcmc.py:296-306 does, or one row per chain), rngs / draws one per retrieval
+    (draws as demc_draws returns them), savefile / savemodel one path per retrieval.  Returns a list
+    of R dicts with run_demc's keys; retrieval r equals run_demc on its own data and streams.
+    grexit is refused: the retrievals would stop at different iterations.  One device call's host
+    arrays are bounded, the whole run's are not (see ENSEMBLE_CALL_BYTES)."""
+    if grexit:
+        raise ValueError("grexit is not offered for ensembles: the retrievals would stop at "
+                         "different iterations")
+    data, uncert, starts, pmin, pmax, stepsize = _ensemble_setup(
+        data, uncert, params, pmin, pmax, stepsize, nchains, rngs, draws)
+    nretr = data.shape[0]
+    ifree = np.where(stepsize > 0)[0]
+    chainsize = int(np.ceil(numit / nchains))
+    transit.mcmc_init_ensemble(starts, pmin, pmax, stepsize, data, uncert, prior=prior,
+                               priorlow=priorlow, fgamma=fgamma, fepsilon=fepsilon, burnin=burnin)
+    if draws is None:
+        draws = [demc_draws(rngs[r], nchains, chainsize, stepsize[ifree]) for r in range(nretr)]
+
+    def run(lo, hi):
+        transit.mcmc_run(*stack_demc_draws(draws, lo, hi))
+    allp, allm, history, chainlen = run_segments(
+        run, lambda: (transit.mcmc_get("allparams"), transit.mcmc_get("allmodel")), chainsize,
+        burnin=burnin, thinning=thinning, grtest=grtest,
+        max_segment=_segment_cap(nretr, nchains, len(ifree), data.shape[1]))
+    return _ensemble_results(transit, ("params", "currchisq", "numaccept", "outbounds", "bestp",
+                                       "bestmodel", "models"),
+                             allp, allm, history, chainlen, burnin, nchains, savefile, savemodel)
+
+
+def run_snooker_ensemble(transit, data, uncert, params, pmin, pmax, stepsize, numit, nchains,
+                         prior=None, priorlow=None, burnin=0, thinning=1, fgamma=1.0, fepsilon=0.0,
+                         hsize=1, rngs=None, draws=None, savefile=None, savemodel=None,
+                         grtest=False, grexit=False):
+    """`run_snooker` for R retrievals in one device loop (arguments as run_demc_ensemble; draws as
+    snooker_draws returns them).  hsize and thinning are shared, so every retrieval's history grows
+    on the same schedule.  Returns a list of R dicts with run_snooker's keys."""
+    if grexit:
+        raise ValueError("grexit is not offered for ensembles: the retrievals would stop at "
+                         "different iterations")
+    data, uncert, starts, pmin, pmax, stepsize = _ensemble_setup(
+        data, uncert, params, pmin, pmax, stepsize, nchains, rngs, draws)
+    nretr = data.shape[0]
+    ifree = np.where(stepsize > 0)[0]
+    chainsize = int(np.ceil(numit / nchains))
+    if hsize < nchains:                                              # mcmc.py:233-235
+        hsize = nchains + 1
+    transit.mcmc_init_ensemble(starts, pmin, pmax, stepsize, data, uncert, prior=prior,
+                               priorlow=priorlow, fgamma=fgamma, fepsilon=fepsilon, burnin=burnin)
+    if draws is None:
+        draws = [snooker_draws(rngs[r], nchains, len(ifree), chainsize, hsize, thinning,
+                               stepsize[ifree], pmin[ifree], pmax[ifree]) for r in range(nretr)]
+    transit.mcmc_snooker_init(np.stack([d["z0"] for d in draws]), thinning)
+
+    def run(lo, hi):
+        transit.mcmc_run_snooker(*stack_snooker_draws(draws, lo, hi))
+    allp, allm, history, chainlen = run_segments(
+        run, lambda: (transit.mcmc_get("allparams"), transit.mcmc_get("allmodel")), chainsize,
+        burnin=burnin, thinning=thinning, grtest=grtest,
+        max_segment=_segment_cap(nretr, nchains, len(ifree), data.shape[1], extra=len(ifree) / 5 + 2))
+    return _ensemble_results(transit, ("params", "currchisq", "numaccept", "outbounds", "bestp",
+                                       "bestmodel", "models", "Z", "Zchisq"),
+                             allp, allm, history, chainlen, burnin, nchains, savefile, savemodel)

@@ -256,22 +256,40 @@ void bart_chain_block(int nchains, int world, int rank, int *lo, int *hi);
  * are the chains' starting points; stepsize > 0 free, 0 fixed, < 0 shared with parameter
  * -stepsize (1-based).  ndata must equal the number of filters.  With a communicator
  * (bart_comm_init) every rank evaluates its block of chains and one all-gather per generation
- * shares the band fluxes; the proposal and Metropolis steps run redundantly on every rank.       */
+ * shares the band fluxes; the proposal and Metropolis steps run redundantly on every rank.
+ * Same as bart_mcmc_init_ensemble with nretr = 1.                                               */
 int  bart_mcmc_init(int nchains, int npars, const double *params, const double *pmin,
                     const double *pmax, const double *stepsize, const double *prior,
                     const double *priorlow, int ndata, const double *data, const double *uncert,
                     double fgamma, double fepsilon, int burnin);
+/* An ensemble of nretr >= 1 independent retrievals of the same planet in one loop: each has its
+ * own starting points params[nretr][nchains][npars], data and uncert[nretr][ndata]; the forward
+ * model, filters, converter, bounds, step sizes, priors, fgamma, fepsilon and burnin are shared.
+ * Every generation evaluates the nretr x nchains models (model g = r * nchains + c) as one batch
+ * (split over the ranks like the chains of one retrieval); proposals, Metropolis steps, best fits
+ * and snooker histories stay within each retrieval, so retrieval r comes out bit-identical to the
+ * same retrieval run alone.  After it, every call below takes and returns its arrays behind a
+ * leading [nretr] axis, each retrieval's slice shaped as documented for one retrieval.           */
+int  bart_mcmc_init_ensemble(int nretr, int nchains, int npars, const double *params,
+                             const double *pmin, const double *pmax, const double *stepsize,
+                             const double *prior, const double *priorlow, int ndata,
+                             const double *data, const double *uncert, double fgamma,
+                             double fepsilon, int burnin);
+/* retrievals of the current loop: 1 after bart_mcmc_init, 0 before any init                     */
+int  bart_mcmc_nretr(void);
 /* MC3's `resume` (mcmc.py:254-269) for walk='demc': call bart_mcmc_init with the chains' last
  * states of the previous run (oldparams[:, :, -1] in the free columns), then this with nold = the
  * previous run's iterations per chain (they count towards burn-in, mcmc.py:616) and curmodel
- * [nchains][ndata] = the last column of the previous run's `savemodel` array (a chain whose proposals
- * are rejected keeps showing it, mcmc.py:649-651; NULL: zeros, as without savemodel).  Before the
- * first bart_mcmc_run.  (The reference's snooker resume rebuilds its history from the log file's
- * text and is not offered.)                                                                       */
+ * [nretr][nchains][ndata] = the last column of the previous run's `savemodel` array (a chain whose
+ * proposals are rejected keeps showing it, mcmc.py:649-651; NULL: zeros, as without savemodel).
+ * nold is shared by the retrievals.  Before the first bart_mcmc_run.  (The reference's snooker
+ * resume rebuilds its history from the log file's text and is not offered.)                     */
 int  bart_mcmc_resume(int nold, const double *curmodel);
 /* niter generations without a host round trip.  The random streams are the caller's, in MC3's
- * shapes with chainsize = niter (mcmc.py:484-507): support[niter][nchains][nfree],
- * r1/r2[nchains][niter], unif/ugamma[niter][nchains].                                            */
+ * shapes with chainsize = niter (mcmc.py:484-507) behind the retrieval axis:
+ * support[nretr][niter][nchains][nfree], r1/r2[nretr][nchains][niter] (chain indices within the
+ * retrieval), unif/ugamma[nretr][niter][nchains].  An out-of-range r1/r2 is refused with the
+ * retrieval, generation and chain named.                                                          */
 int  bart_mcmc_run(int niter, const double *support, const int *r1, const int *r2,
                    const double *unif, const double *ugamma);
 /* replaces MCcubed.mc.mcmc for walk='snooker' -- the walk every BART example configures
@@ -279,15 +297,19 @@ int  bart_mcmc_run(int niter, const double *support, const int *r1, const int *r
  * (ter Braak & Vrugt 2008): Z set-up and evaluation of the hsize*nchains initial samples
  * (mcmc.py:357-470), proposals (527-561), Metropolis factor of projected jumps (603-609), Z
  * update every `thinning` generations (653-660).  Call after bart_mcmc_init.
- * z0[hsize][nchains][nfree]: initial samples of the free parameters (the reference draws them
- * uniformly in [pmin, pmax]); hsize > nchains as mcmc.py:233-235 enforces is the caller's job.   */
+ * z0[nretr][hsize][nchains][nfree]: initial samples of the free parameters (the reference draws
+ * them uniformly in [pmin, pmax]); hsize > nchains as mcmc.py:233-235 enforces is the caller's
+ * job.  hsize and thinning are shared: every retrieval's history grows on the same schedule.     */
 int  bart_mcmc_snooker_init(int hsize, int thinning, const double *z0);
 /* niter snooker generations without a host round trip.  Random streams in the order mcmc.py
- * consumes them: support[niter][nchains][nfree], unif/ugamma[niter][nchains] (490-497); per
- * generation i1, i2 (flat indices into Z's first Zsize-1 rows x nchains), iz (row), ic (chain),
- * each [niter][nchains] (529-539); usnooker[usn_offset[niter]][nfree]: the uniform(1.2, 2.2)
- * factors of the chains with ugamma < 0.1, generation i owning rows usn_offset[i] ..
- * usn_offset[i+1] in the reference's draw order (545-556).                                       */
+ * consumes them, behind the retrieval axis: support[nretr][niter][nchains][nfree],
+ * unif/ugamma[nretr][niter][nchains] (490-497); per generation i1, i2 (flat indices into the
+ * retrieval's own history, its first Zsize-1 rows x nchains), iz (row), ic (chain), each
+ * [nretr][niter][nchains] (529-539); usnooker[rows][nfree]: the uniform(1.2, 2.2) factors of the
+ * chains with ugamma < 0.1 in the reference's draw order (545-556), all retrievals' rows one
+ * retrieval after the other; usn_offset[nretr][niter+1] their absolute first rows, generation i
+ * of retrieval r owning rows usn_offset[r][i] .. usn_offset[r][i+1] (so usn_offset[r][0] ==
+ * usn_offset[r-1][niter] and rows = usn_offset[nretr-1][niter]).                                 */
 int  bart_mcmc_run_snooker(int niter, const double *support, const int *i1, const int *i2,
                            const int *iz, const int *ic, const double *usnooker,
                            const int *usn_offset, const double *unif, const double *ugamma);
@@ -295,8 +317,9 @@ int  bart_mcmc_run_snooker(int niter, const double *support, const int *i1, cons
  * [nchains][ndata][niter] (MC3's `savemodel` array, mcmc.py:636-651,849-850: the model of every
  * chain's current state, zeros until its first acceptance like the reference), "params",
  * "currchisq", "numaccept", "outbounds", "bestp", "bestchisq", "bestmodel", "models", and for
- * snooker "Z" [Zsize][nchains][npars], "Zchisq" [Zsize][nchains]; returns the number of doubles
- * written or < 0.                                                                               */
+ * snooker "Z" [Zsize][nchains][npars], "Zchisq" [Zsize][nchains]; each behind a leading [nretr]
+ * (bestp [nretr][npars], bestchisq [nretr], bestmodel [nretr][ndata]), retrieval-major; with
+ * nretr = 1 the layouts are those of one retrieval.  Returns the number of doubles written or < 0. */
 long long bart_mcmc_get(const char *name, double *out, long long capacity);
 
 #ifdef __cplusplus
