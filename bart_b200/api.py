@@ -98,8 +98,6 @@ def lib():
     L.bart_bandflux_from_params_device.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p]
     L.bart_chain_block.argtypes = [C.c_int, C.c_int, C.c_int, ip, ip]
     L.bart_chain_block.restype = None
-    L.bart_mcmc_init.argtypes = [C.c_int, C.c_int, dp, dp, dp, dp, dp, dp, C.c_int, dp, dp,
-                                 C.c_double, C.c_double, C.c_int]
     L.bart_mcmc_init_ensemble.argtypes = [C.c_int, C.c_int, C.c_int, dp, dp, dp, dp, dp, dp, C.c_int,
                                           dp, dp, C.c_double, C.c_double, C.c_int]
     L.bart_mcmc_nretr.restype = C.c_int
@@ -332,17 +330,13 @@ class Transit:
 
     def mcmc_init(self, params, pmin, pmax, stepsize, data, uncert, prior=None, priorlow=None,
                   fgamma=1.0, fepsilon=0.0, burnin=0):
-        params = np.ascontiguousarray(np.atleast_2d(params), dtype=np.float64)
-        nchains, npars = params.shape
-        f = lambda a: np.ascontiguousarray(a if a is not None else np.zeros(npars), dtype=np.float64)
-        pmin, pmax, stepsize, prior, priorlow = (f(a) for a in (pmin, pmax, stepsize, prior, priorlow))
-        data = np.ascontiguousarray(data, dtype=np.float64)
-        uncert = np.ascontiguousarray(uncert, dtype=np.float64)
-        _check(lib().bart_mcmc_init(nchains, npars, _d(params), _d(pmin), _d(pmax), _d(stepsize),
-                                    _d(prior), _d(priorlow), len(data), _d(data), _d(uncert),
-                                    float(fgamma), float(fepsilon), int(burnin)))
-        self._mc_shape = (nchains, npars, int(np.sum(stepsize > 0)), len(data))
-        self._mc_ensemble = False
+        """One retrieval: params[C][P] starting points, data / uncert[D].  It is an ensemble of one
+        whose caller uses lone shapes: the mcmc_* calls take and return every array without the
+        leading [R] axis, except bestchisq, which keeps its shape (1,)."""
+        self.mcmc_init_ensemble(np.atleast_2d(params)[None], pmin, pmax, stepsize,
+                                np.asarray(data)[None], np.asarray(uncert)[None], prior, priorlow,
+                                fgamma, fepsilon, burnin)
+        self._mc_lone = True
 
     def mcmc_init_ensemble(self, params, pmin, pmax, stepsize, data, uncert, prior=None,
                            priorlow=None, fgamma=1.0, fepsilon=0.0, burnin=0):
@@ -363,44 +357,39 @@ class Transit:
                                              _d(stepsize), _d(prior), _d(priorlow), data.shape[1],
                                              _d(data), _d(uncert), float(fgamma), float(fepsilon),
                                              int(burnin)))
-        self._mc_shape = (nchains, npars, int(np.sum(stepsize > 0)), data.shape[1])
-        self._mc_ensemble = True
+        self._mc_shape = (nretr, nchains, npars, int(np.sum(stepsize > 0)), data.shape[1])
+        self._mc_lone, self._mc_niter, self._mc_zsize = False, 0, 0
 
-    def _mc_lead(self):
-        """Leading axis of the loop's arrays: () after mcmc_init, (R,) after mcmc_init_ensemble."""
-        return (lib().bart_mcmc_nretr(),) if getattr(self, "_mc_ensemble", False) else ()
+    def _mc_in(self, a, dtype):
+        """An mcmc_* argument as a contiguous array behind the [R] axis (added for a lone caller)."""
+        a = np.ascontiguousarray(a, dtype=dtype)
+        return a[None] if self._mc_lone else a
 
-    def _mc_refuse(self, lead, what):
-        raise BartError("%s do not have MC3's shapes for %s%d chains" % (
-            what, "%d retrievals x " % lead[0] if lead else "", self._mc_shape[0]))
+    def _mc_dims(self, *dims):
+        """The dimensions an mcmc_* argument must have, for its error message."""
+        lead = () if self._mc_lone else ("%d retrievals" % self._mc_shape[0],)
+        return "[%s]" % "][".join(lead + dims)
 
     def mcmc_resume(self, nold, curmodel=None):
         """MC3's resume=True (mcmc.py:254-269) after mcmc_init with the old run's last states."""
         if curmodel is not None:
-            curmodel = np.ascontiguousarray(curmodel, dtype=np.float64)
-            nchains, npars, nfree, ndata = self._mc_shape
-            lead = self._mc_lead()
-            if curmodel.shape != lead + (nchains, ndata):
-                raise BartError("curmodel must be [%s%d chains][%d data]"
-                                % ("%d retrievals][" % lead[0] if lead else "", nchains, ndata))
+            curmodel = self._mc_in(curmodel, np.float64)
+            nretr, nchains, npars, nfree, ndata = self._mc_shape
+            if curmodel.shape != (nretr, nchains, ndata):
+                raise BartError("curmodel must be %s" % self._mc_dims("%d chains" % nchains,
+                                                                       "%d data" % ndata))
         _check(lib().bart_mcmc_resume(int(nold), None if curmodel is None else _d(curmodel)))
 
     def mcmc_run(self, support, r1, r2, unif, ugamma):
-        support = np.ascontiguousarray(support, dtype=np.float64)
-        unif = np.ascontiguousarray(unif, dtype=np.float64)
-        ugamma = np.ascontiguousarray(ugamma, dtype=np.float64)
-        r1 = np.ascontiguousarray(r1, dtype=np.int32)
-        r2 = np.ascontiguousarray(r2, dtype=np.int32)
-        lead = self._mc_lead()
+        support, unif, ugamma = (self._mc_in(a, np.float64) for a in (support, unif, ugamma))
+        r1, r2 = (self._mc_in(a, np.int32) for a in (r1, r2))
+        nretr, nchains, npars, nfree, ndata = self._mc_shape
         niter = unif.shape[-2] if unif.ndim >= 2 else 0
-        nchains, npars, nfree, ndata = self._mc_shape
-        if support.shape != lead + (niter, nchains, nfree) or r1.shape != lead + (nchains, niter) or \
-                r2.shape != lead + (nchains, niter) or unif.shape != lead + (niter, nchains) or \
-                ugamma.shape != lead + (niter, nchains):
-            if not lead:
-                raise BartError("random streams do not have MC3's shapes for %d chains x %d iterations"
-                                % (nchains, niter))
-            self._mc_refuse(lead, "random streams")
+        if support.shape != (nretr, niter, nchains, nfree) or r1.shape != (nretr, nchains, niter) or \
+                r2.shape != (nretr, nchains, niter) or unif.shape != (nretr, niter, nchains) or \
+                ugamma.shape != (nretr, niter, nchains):
+            raise BartError("random streams must have MC3's shapes for %s" % self._mc_dims(
+                "%d chains" % nchains, "%d iterations" % niter))
         _check(lib().bart_mcmc_run(niter, _d(support), r1.ctypes.data_as(ip), r2.ctypes.data_as(ip),
                                    _d(unif), _d(ugamma)))
         self._mc_niter = niter
@@ -408,34 +397,28 @@ class Transit:
     def mcmc_snooker_init(self, z0, thinning=1):
         """z0[hsize][nchains][nfree] ([R][hsize][nchains][nfree] for an ensemble): MC3's M0 initial
         history samples (mcmc.py:421-424)."""
-        nchains, npars, nfree, ndata = self._mc_shape
-        lead = self._mc_lead()
-        z0 = np.ascontiguousarray(z0, dtype=np.float64)
-        if z0.ndim != 3 + len(lead) or z0.shape[:len(lead)] != lead or z0.shape[-2:] != (nchains, nfree):
-            raise BartError("z0 must be [%shsize][%d][%d]" % ("%d][" % lead[0] if lead else "", nchains, nfree))
-        hsize = z0.shape[len(lead)]
-        _check(lib().bart_mcmc_snooker_init(hsize, int(thinning), _d(z0)))
-        self._mc_zsize, self._mc_thinning = hsize, int(thinning)
+        nretr, nchains, npars, nfree, ndata = self._mc_shape
+        z0 = self._mc_in(z0, np.float64)
+        if z0.ndim != 4 or z0.shape[0] != nretr or z0.shape[2:] != (nchains, nfree):
+            raise BartError("z0 must be %s" % self._mc_dims("hsize", "%d chains" % nchains,
+                                                             "%d free parameters" % nfree))
+        _check(lib().bart_mcmc_snooker_init(z0.shape[1], int(thinning), _d(z0)))
+        self._mc_zsize, self._mc_thinning = z0.shape[1], int(thinning)
 
     def mcmc_run_snooker(self, support, i1, i2, iz, ic, usnooker, usn_offset, unif, ugamma):
         """Streams of run_snooker's shapes; for an ensemble each behind [R], usnooker the
         retrievals' factor rows one after the other and usn_offset[R][niter+1] absolute rows."""
-        nchains, npars, nfree, ndata = self._mc_shape
-        lead = self._mc_lead()
-        support, unif, ugamma, usnooker = (np.ascontiguousarray(a, dtype=np.float64)
-                                           for a in (support, unif, ugamma, usnooker))
-        i1, i2, iz, ic, usn_offset = (np.ascontiguousarray(a, dtype=np.int32)
-                                      for a in (i1, i2, iz, ic, usn_offset))
+        nretr, nchains, npars, nfree, ndata = self._mc_shape
+        support, unif, ugamma = (self._mc_in(a, np.float64) for a in (support, unif, ugamma))
+        usnooker = np.ascontiguousarray(usnooker, dtype=np.float64)
+        i1, i2, iz, ic, usn_offset = (self._mc_in(a, np.int32) for a in (i1, i2, iz, ic, usn_offset))
         niter = unif.shape[-2] if unif.ndim >= 2 else 0
-        if support.shape != lead + (niter, nchains, nfree) or ugamma.shape != lead + (niter, nchains) or \
-                unif.shape != lead + (niter, nchains) or \
-                any(a.shape != lead + (niter, nchains) for a in (i1, i2, iz, ic)) or \
-                usn_offset.shape != lead + (niter + 1,) or \
+        if support.shape != (nretr, niter, nchains, nfree) or \
+                any(a.shape != (nretr, niter, nchains) for a in (unif, ugamma, i1, i2, iz, ic)) or \
+                usn_offset.shape != (nretr, niter + 1) or \
                 usnooker.shape != (usn_offset.flat[-1] if usn_offset.size else -1, nfree):
-            if not lead:
-                raise BartError("random streams do not have MC3's shapes for %d chains x %d iterations"
-                                % (nchains, niter))
-            self._mc_refuse(lead, "snooker streams")
+            raise BartError("snooker streams must have MC3's shapes for %s" % self._mc_dims(
+                "%d chains" % nchains, "%d iterations" % niter))
         _check(lib().bart_mcmc_run_snooker(
             niter, _d(support), i1.ctypes.data_as(ip), i2.ctypes.data_as(ip), iz.ctypes.data_as(ip),
             ic.ctypes.data_as(ip), _d(usnooker), usn_offset.ctypes.data_as(ip), _d(unif), _d(ugamma)))
@@ -443,29 +426,26 @@ class Transit:
         self._mc_zsize += len(range(0, niter, self._mc_thinning)) + 1     # upper bound, see mcmc_get
 
     def mcmc_get(self, name):
-        nchains, npars, nfree, ndata = self._mc_shape
-        lead = self._mc_lead()
+        nretr, nchains, npars, nfree, ndata = self._mc_shape
         if name in ("Z", "Zchisq"):
             # _mc_zsize is an upper bound (it counts thinned rows per call; the library grows Z on
             # the GLOBAL iteration number, like MC3): size the result from what the library returns
             tail = (nchains, npars) if name == "Z" else (nchains,)
-            out = np.zeros(lead + (getattr(self, "_mc_zsize", 0),) + tail)
+            out = np.zeros((nretr, self._mc_zsize) + tail)
             n = lib().bart_mcmc_get(name.encode(), _d(out), out.size)
             _check(0 if n >= 0 else -1)
-            rows = n // (int(np.prod(lead + tail)))
-            if not lead:
-                return out[:rows]
-            return out.ravel()[:n].reshape(lead + (rows,) + tail).copy()
-        shapes = {"allparams": (nchains, nfree, getattr(self, "_mc_niter", 0)),
-                  "allmodel": (nchains, ndata, getattr(self, "_mc_niter", 0)),
-                  "params": (nchains, npars), "currchisq": (nchains,), "numaccept": (nchains,),
-                  "outbounds": (nchains, nfree), "bestp": (npars,), "bestchisq": (1,),
-                  "bestmodel": (ndata,), "models": (nchains, ndata)}
-        shape = lead + shapes[name] if name != "bestchisq" or not lead else lead
-        out = np.zeros(shape)
-        n = lib().bart_mcmc_get(name.encode(), _d(out), out.size)
-        _check(0 if n >= 0 else -1)
-        return out
+            rows = n // (nretr * int(np.prod(tail)))
+            out = out.ravel()[:n].reshape((nretr, rows) + tail).copy()
+        else:
+            shapes = {"allparams": (nchains, nfree, self._mc_niter),
+                      "allmodel": (nchains, ndata, self._mc_niter),
+                      "params": (nchains, npars), "currchisq": (nchains,), "numaccept": (nchains,),
+                      "outbounds": (nchains, nfree), "bestp": (npars,), "bestchisq": (),
+                      "bestmodel": (ndata,), "models": (nchains, ndata)}
+            out = np.zeros((nretr,) + shapes[name])
+            n = lib().bart_mcmc_get(name.encode(), _d(out), out.size)
+            _check(0 if n >= 0 else -1)
+        return out[0] if self._mc_lone and name != "bestchisq" else out
 
     def debug_keep(self, on=True):
         lib().bart_debug_keep(1 if on else 0)

@@ -283,42 +283,21 @@ def run_demc(transit, data, uncert, params, pmin, pmax, stepsize, numit, nchains
     [nchains][nfree][chainsize], the stacked posterior after burn-in, bestp, numaccept, ...
     resume=True continues the run whose `savefile` (and `savemodel`) are on disk, like
     mcmc.py:254-269: chains restart from their last states, the new iterations are appended to the
-    old traces, burn-in and the convergence test count from the old run's first iteration."""
-    params = np.atleast_2d(np.array(params, dtype=float))
-    pmin, pmax, stepsize = (np.asarray(a, dtype=float) for a in (pmin, pmax, stepsize))
-    ifree = np.where(stepsize > 0)[0]
-    chainsize = int(np.ceil(numit / nchains))
-    nold, oldparams, oldmodel = 0, None, None
+    old traces, burn-in and the convergence test count from the old run's first iteration.
+    The run is an ensemble of one (see _retrieve)."""
+    old = None
     if resume:
         oldparams = np.load(savefile)
-        nold = oldparams.shape[2]
-        if savemodel is not None:
-            oldmodel = np.load(savemodel)
-        params = np.repeat(params[:1], nchains, 0)
-        params[:, ifree] = oldparams[:, :, -1]
-    params = start_points(params, nchains, stepsize, pmin, pmax, rng)
-    transit.mcmc_init(params, pmin, pmax, stepsize, data, uncert, prior=prior, priorlow=priorlow,
-                      fgamma=fgamma, fepsilon=fepsilon, burnin=burnin)
-    if resume:
-        transit.mcmc_resume(nold, None if oldmodel is None else oldmodel[:, :, -1])
-    if draws is None:
-        draws = demc_draws(rng, nchains, chainsize, stepsize[ifree])
-    def run(lo, hi):
-        h = slice(lo, hi)
-        transit.mcmc_run(draws["support"][h], draws["r1"][:, h], draws["r2"][:, h], draws["unif"][h],
-                         draws["ugamma"][h])
-    allp, allm, history, chainlen = run_segments(
-        run, lambda: (transit.mcmc_get("allparams"), transit.mcmc_get("allmodel")), chainsize,
-        burnin=burnin, thinning=thinning, grtest=grtest, grexit=grexit, nold=nold,
-        old=None if not resume else (oldparams, oldmodel if oldmodel is not None
-                                     else np.zeros((nchains, len(data), nold))))
-    out = {k: transit.mcmc_get(k) for k in ("params", "currchisq", "numaccept",
-                                            "outbounds", "bestp", "bestmodel", "models")}
-    out["allparams"], out["allmodel"], out["psrf"] = allp, allm, history
-    out["bestchisq"] = float(transit.mcmc_get("bestchisq")[0])
-    out["allstack"] = np.hstack([allp[c, :, burnin:chainlen] for c in range(nchains)])  # mcmc.py:692-695
-    _save_mc3_files(out, savefile, savemodel)
-    return out
+        oldmodel = np.load(savemodel) if savemodel is not None else None
+        params = np.repeat(np.atleast_2d(np.array(params, dtype=float))[:1], nchains, 0)
+        params[:, np.asarray(stepsize, dtype=float) > 0] = oldparams[:, :, -1]
+        allmodel = oldmodel if oldmodel is not None else np.zeros((nchains, len(data), oldparams.shape[2]))
+        old = (oldparams[None], allmodel[None], None if oldmodel is None else oldmodel[None, :, :, -1])
+    return _retrieve(transit, "demc", np.asarray(data, dtype=float)[None],
+                     np.asarray(uncert, dtype=float)[None], [params], pmin, pmax, stepsize, numit,
+                     nchains, [rng], None if draws is None else [draws], [savefile], [savemodel],
+                     prior=prior, priorlow=priorlow, burnin=burnin, fgamma=fgamma, fepsilon=fepsilon,
+                     thinning=thinning, grtest=grtest, grexit=grexit, old=old)[0]
 
 
 def gelman_rubin(chains):
@@ -345,11 +324,12 @@ def run_segments(run, fetch, chainsize, burnin=0, thinning=1, grtest=False, grex
                  old=None, max_segment=None):
     """Drive a device-resident walk in the segments MC3's loop is observable in (mcmc.py:662-690).
     `run(lo, hi)` advances generations [lo, hi) (state stays on the device); `fetch()` returns that
-    call's allparams / allmodel pieces.  Without grtest it is one segment; `max_segment` caps the
-    generations of one call (the host arrays of a call stay bounded).  `old` = (allparams,
-    allmodel) of the run being resumed (nold iterations).  Traces of an ensemble carry a leading
-    retrieval axis, and its psrf is [retrieval][nfree].  Returns (allparams, allmodel, psrf
-    history [(iteration, psrf)], number of iterations in the traces)."""
+    call's allparams / allmodel pieces, [nchains][...][hi - lo] behind any leading axes (the
+    driver's traces carry one retrieval axis).  Without grtest it is one segment; `max_segment`
+    caps the generations of one call (the host arrays of a call stay bounded).  `old` =
+    (allparams, allmodel) of the runs being resumed (nold iterations).  Returns (allparams,
+    allmodel, psrf history [(iteration, psrf[leading axes...][nfree])], number of iterations in
+    the traces)."""
     cuts = gr_checkpoints(chainsize) if grtest else []
     bounds = list(range(max_segment, chainsize, max_segment)) if max_segment else []
     edges = sorted(set([c + 1 for c in cuts] + bounds + [chainsize]))
@@ -364,11 +344,10 @@ def run_segments(run, fetch, chainsize, burnin=0, thinning=1, grtest=False, grex
         lo = hi
         i = hi - 1
         if grtest and i in cuts and (i + nold) > burnin:
-            allp = np.concatenate(pieces_p, axis=-1)
-            if allp.ndim == 4:
-                psrf = np.array([gelman_rubin(a[:, :, burnin:i + nold + 1:thinning]) for a in allp])
-            else:
-                psrf = gelman_rubin(allp[:, :, burnin:i + nold + 1:thinning])
+            allp = np.concatenate(pieces_p, axis=-1)[..., burnin:i + nold + 1:thinning]
+            lead = allp.shape[:-3]
+            psrf = np.array([gelman_rubin(a) for a in allp.reshape((-1,) + allp.shape[-3:])])
+            psrf = psrf.reshape(lead + psrf.shape[-1:])
             history.append((i, psrf))
             if np.all(psrf < 1.01):
                 if grexit and grflag:                        # two consecutive passes (mcmc.py:676-683)
@@ -431,46 +410,24 @@ def run_snooker(transit, data, uncert, params, pmin, pmax, stepsize, numit, ncha
                 rng=np.random, draws=None, savefile=None, savemodel=None, grtest=False, grexit=False):
     """`MCcubed.mc.mcmc(..., walk='snooker', leastsq=False)` -- the walk BART's examples configure
     -- with the sample history Z, the proposals, the Metropolis rule and the forward models all on
-    the GPU.  Returns MC3's arrays (see run_demc) plus Z and Zchisq."""
-    params = np.atleast_2d(np.array(params, dtype=float))
-    pmin, pmax, stepsize = (np.asarray(a, dtype=float) for a in (pmin, pmax, stepsize))
-    ifree = np.where(stepsize > 0)[0]
-    chainsize = int(np.ceil(numit / nchains))
-    if hsize < nchains:                                              # mcmc.py:233-235
-        hsize = nchains + 1
-    params = start_points(params, nchains, stepsize, pmin, pmax, rng)
-    transit.mcmc_init(params, pmin, pmax, stepsize, data, uncert, prior=prior, priorlow=priorlow,
-                      fgamma=fgamma, fepsilon=fepsilon, burnin=burnin)
-    if draws is None:
-        draws = snooker_draws(rng, nchains, len(ifree), chainsize, hsize, thinning, stepsize[ifree],
-                              pmin[ifree], pmax[ifree])
-    transit.mcmc_snooker_init(draws["z0"], thinning)
-    def run(lo, hi):
-        h = slice(lo, hi)
-        off = np.asarray(draws["usn_offset"])[lo:hi + 1]
-        transit.mcmc_run_snooker(draws["support"][h], draws["i1"][h], draws["i2"][h], draws["iz"][h],
-                                 draws["ic"][h], draws["usnooker"][off[0]:off[-1]], off - off[0],
-                                 draws["unif"][h], draws["ugamma"][h])
-    allp, allm, history, chainlen = run_segments(
-        run, lambda: (transit.mcmc_get("allparams"), transit.mcmc_get("allmodel")), chainsize,
-        burnin=burnin, thinning=thinning, grtest=grtest, grexit=grexit)
-    out = {k: transit.mcmc_get(k) for k in ("params", "currchisq", "numaccept",
-                                            "outbounds", "bestp", "bestmodel", "models", "Z", "Zchisq")}
-    out["allparams"], out["allmodel"], out["psrf"] = allp, allm, history
-    out["bestchisq"] = float(transit.mcmc_get("bestchisq")[0])
-    out["allstack"] = np.hstack([allp[c, :, burnin:chainlen] for c in range(nchains)])
-    _save_mc3_files(out, savefile, savemodel)
-    return out
+    the GPU.  Returns MC3's arrays (see run_demc) plus Z and Zchisq.  The run is an ensemble of
+    one (see _retrieve)."""
+    return _retrieve(transit, "snooker", np.asarray(data, dtype=float)[None],
+                     np.asarray(uncert, dtype=float)[None], [params], pmin, pmax, stepsize, numit,
+                     nchains, [rng], None if draws is None else [draws], [savefile], [savemodel],
+                     prior=prior, priorlow=priorlow, burnin=burnin, fgamma=fgamma, fepsilon=fepsilon,
+                     thinning=thinning, hsize=hsize, grtest=grtest, grexit=grexit)[0]
 
 
 # ---------------------------------------------------------------------------------------------
-# Ensembles: R independent retrievals of the same configuration in one device loop
-# (Transit.mcmc_init_ensemble); every generation evaluates R x nchains models as one batch.
-# Long runs go through the device in segments of at most _segment_cap generations, so the stacked
-# stream and trace arrays of one device call stay under ENSEMBLE_CALL_BYTES.  Total host memory is
-# not bounded: every retrieval's streams are drawn up front in MC3's order (what makes its chains
-# MC3's), and the returned traces hold every generation -- at R = 64, 10 chains, 9 free parameters
-# and 1e5 generations the `support` draws alone are 4.6 GB.
+# Every run is an ensemble: R independent retrievals of the same configuration in one device loop
+# (Transit.mcmc_init_ensemble), a lone run_demc / run_snooker being R = 1.  Every generation
+# evaluates R x nchains models as one batch.  Long runs go through the device in segments of at most
+# _segment_cap generations, so the stacked stream and trace arrays of one device call stay under
+# ENSEMBLE_CALL_BYTES.  Total host memory is not bounded: every retrieval's streams are drawn up
+# front in MC3's order (what makes its chains MC3's), and the returned traces hold every
+# generation -- at R = 64, 10 chains, 9 free parameters and 1e5 generations the `support` draws
+# alone are 4.6 GB.
 ENSEMBLE_CALL_BYTES = 1 << 28          # host stream + trace arrays of one device call
 
 
@@ -497,7 +454,21 @@ def stack_snooker_draws(draws, lo, hi):
             np.stack(offs), st("unif"), st("ugamma"))
 
 
-def _ensemble_setup(data, uncert, params, pmin, pmax, stepsize, nchains, rngs, draws):
+def _segment_cap(nretr, nchains, nfree, ndata, extra=0):
+    """Generations of one device call so that its host arrays stay under ENSEMBLE_CALL_BYTES."""
+    per_gen = nretr * nchains * (8 * (2 * nfree + ndata + 2 + extra) + 2 * 4)
+    return max(1, int(ENSEMBLE_CALL_BYTES // per_gen))
+
+
+def _retrieve(transit, walk, data, uncert, params, pmin, pmax, stepsize, numit, nchains, rngs, draws,
+              savefile, savemodel, prior=None, priorlow=None, burnin=0, fgamma=1.0, fepsilon=0.0,
+              thinning=1, hsize=1, grtest=False, grexit=False, old=None):
+    """R retrievals of `walk` ('demc' or 'snooker') in one device loop.  data / uncert[R][ndata];
+    params, rngs, draws, savefile and savemodel one entry per retrieval (rngs, draws, savefile and
+    savemodel may also be None); draws that are not given are drawn from the rngs after the start
+    points.  `old` = (allparams[R][C][F][nold], allmodel[R][C][D][nold], last model column[R][C][D]
+    or None) of the runs being resumed.  Returns R dicts of MC3's arrays, each also written to its
+    savefile / savemodel."""
     data = np.asarray(data, dtype=float)
     uncert = np.asarray(uncert, dtype=float)
     nretr = data.shape[0]
@@ -507,6 +478,8 @@ def _ensemble_setup(data, uncert, params, pmin, pmax, stepsize, nchains, rngs, d
         if v is not None and len(v) != nretr:
             raise ValueError("%s needs one entry per retrieval (%d)" % (name, nretr))
     pmin, pmax, stepsize = (np.asarray(a, dtype=float) for a in (pmin, pmax, stepsize))
+    ifree = np.where(stepsize > 0)[0]
+    chainsize = int(np.ceil(numit / nchains))
     starts = []
     for r in range(nretr):
         rng = rngs[r] if rngs is not None else None
@@ -514,26 +487,40 @@ def _ensemble_setup(data, uncert, params, pmin, pmax, stepsize, nchains, rngs, d
             raise ValueError("retrieval %d needs an rng (its start points or random streams are "
                              "drawn)" % r)
         starts.append(start_points(params[r], nchains, stepsize, pmin, pmax, rng))
-    return data, uncert, np.array(starts), pmin, pmax, stepsize
-
-
-def _segment_cap(nretr, nchains, nfree, ndata, extra=0):
-    """Generations of one device call so that its host arrays stay under ENSEMBLE_CALL_BYTES."""
-    per_gen = nretr * nchains * (8 * (2 * nfree + ndata + 2 + extra) + 2 * 4)
-    return max(1, int(ENSEMBLE_CALL_BYTES // per_gen))
-
-
-def _ensemble_results(transit, keys, allp, allm, history, chainlen, burnin, nchains, savefile,
-                      savemodel):
-    got = {k: transit.mcmc_get(k) for k in keys}
+    transit.mcmc_init_ensemble(np.array(starts), pmin, pmax, stepsize, data, uncert, prior=prior,
+                               priorlow=priorlow, fgamma=fgamma, fepsilon=fepsilon, burnin=burnin)
+    nold = 0 if old is None else old[0].shape[-1]
+    if old is not None:
+        transit.mcmc_resume(nold, old[2])
+    if walk == "demc":
+        if draws is None:
+            draws = [demc_draws(rng, nchains, chainsize, stepsize[ifree]) for rng in rngs]
+        run = lambda lo, hi: transit.mcmc_run(*stack_demc_draws(draws, lo, hi))
+        keys, extra = (), 0
+    else:
+        if hsize < nchains:                                          # mcmc.py:233-235
+            hsize = nchains + 1
+        if draws is None:
+            draws = [snooker_draws(rng, nchains, len(ifree), chainsize, hsize, thinning,
+                                   stepsize[ifree], pmin[ifree], pmax[ifree]) for rng in rngs]
+        transit.mcmc_snooker_init(np.stack([d["z0"] for d in draws]), thinning)
+        run = lambda lo, hi: transit.mcmc_run_snooker(*stack_snooker_draws(draws, lo, hi))
+        keys, extra = ("Z", "Zchisq"), len(ifree) / 5 + 2
+    allp, allm, history, chainlen = run_segments(
+        run, lambda: (transit.mcmc_get("allparams"), transit.mcmc_get("allmodel")), chainsize,
+        burnin=burnin, thinning=thinning, grtest=grtest, grexit=grexit, nold=nold,
+        old=None if old is None else old[:2],
+        max_segment=_segment_cap(nretr, nchains, len(ifree), data.shape[1], extra))
+    got = {k: transit.mcmc_get(k) for k in ("params", "currchisq", "numaccept", "outbounds", "bestp",
+                                            "bestmodel", "models") + keys}
     bestchisq = transit.mcmc_get("bestchisq")
     outs = []
-    for r in range(allp.shape[0]):
+    for r in range(nretr):
         out = {k: v[r] for k, v in got.items()}
         out["allparams"], out["allmodel"] = allp[r], allm[r]
         out["psrf"] = [(i, psrf[r]) for i, psrf in history]
         out["bestchisq"] = float(bestchisq[r])
-        out["allstack"] = np.hstack([allp[r, c, :, burnin:chainlen] for c in range(nchains)])
+        out["allstack"] = np.hstack([allp[r, c, :, burnin:chainlen] for c in range(nchains)])  # mcmc.py:692-695
         _save_mc3_files(out, savefile[r] if savefile is not None else None,
                         savemodel[r] if savemodel is not None else None)
         outs.append(out)
@@ -554,25 +541,9 @@ def run_demc_ensemble(transit, data, uncert, params, pmin, pmax, stepsize, numit
     if grexit:
         raise ValueError("grexit is not offered for ensembles: the retrievals would stop at "
                          "different iterations")
-    data, uncert, starts, pmin, pmax, stepsize = _ensemble_setup(
-        data, uncert, params, pmin, pmax, stepsize, nchains, rngs, draws)
-    nretr = data.shape[0]
-    ifree = np.where(stepsize > 0)[0]
-    chainsize = int(np.ceil(numit / nchains))
-    transit.mcmc_init_ensemble(starts, pmin, pmax, stepsize, data, uncert, prior=prior,
-                               priorlow=priorlow, fgamma=fgamma, fepsilon=fepsilon, burnin=burnin)
-    if draws is None:
-        draws = [demc_draws(rngs[r], nchains, chainsize, stepsize[ifree]) for r in range(nretr)]
-
-    def run(lo, hi):
-        transit.mcmc_run(*stack_demc_draws(draws, lo, hi))
-    allp, allm, history, chainlen = run_segments(
-        run, lambda: (transit.mcmc_get("allparams"), transit.mcmc_get("allmodel")), chainsize,
-        burnin=burnin, thinning=thinning, grtest=grtest,
-        max_segment=_segment_cap(nretr, nchains, len(ifree), data.shape[1]))
-    return _ensemble_results(transit, ("params", "currchisq", "numaccept", "outbounds", "bestp",
-                                       "bestmodel", "models"),
-                             allp, allm, history, chainlen, burnin, nchains, savefile, savemodel)
+    return _retrieve(transit, "demc", data, uncert, params, pmin, pmax, stepsize, numit, nchains,
+                     rngs, draws, savefile, savemodel, prior=prior, priorlow=priorlow, burnin=burnin,
+                     fgamma=fgamma, fepsilon=fepsilon, thinning=thinning, grtest=grtest)
 
 
 def run_snooker_ensemble(transit, data, uncert, params, pmin, pmax, stepsize, numit, nchains,
@@ -585,26 +556,6 @@ def run_snooker_ensemble(transit, data, uncert, params, pmin, pmax, stepsize, nu
     if grexit:
         raise ValueError("grexit is not offered for ensembles: the retrievals would stop at "
                          "different iterations")
-    data, uncert, starts, pmin, pmax, stepsize = _ensemble_setup(
-        data, uncert, params, pmin, pmax, stepsize, nchains, rngs, draws)
-    nretr = data.shape[0]
-    ifree = np.where(stepsize > 0)[0]
-    chainsize = int(np.ceil(numit / nchains))
-    if hsize < nchains:                                              # mcmc.py:233-235
-        hsize = nchains + 1
-    transit.mcmc_init_ensemble(starts, pmin, pmax, stepsize, data, uncert, prior=prior,
-                               priorlow=priorlow, fgamma=fgamma, fepsilon=fepsilon, burnin=burnin)
-    if draws is None:
-        draws = [snooker_draws(rngs[r], nchains, len(ifree), chainsize, hsize, thinning,
-                               stepsize[ifree], pmin[ifree], pmax[ifree]) for r in range(nretr)]
-    transit.mcmc_snooker_init(np.stack([d["z0"] for d in draws]), thinning)
-
-    def run(lo, hi):
-        transit.mcmc_run_snooker(*stack_snooker_draws(draws, lo, hi))
-    allp, allm, history, chainlen = run_segments(
-        run, lambda: (transit.mcmc_get("allparams"), transit.mcmc_get("allmodel")), chainsize,
-        burnin=burnin, thinning=thinning, grtest=grtest,
-        max_segment=_segment_cap(nretr, nchains, len(ifree), data.shape[1], extra=len(ifree) / 5 + 2))
-    return _ensemble_results(transit, ("params", "currchisq", "numaccept", "outbounds", "bestp",
-                                       "bestmodel", "models", "Z", "Zchisq"),
-                             allp, allm, history, chainlen, burnin, nchains, savefile, savemodel)
+    return _retrieve(transit, "snooker", data, uncert, params, pmin, pmax, stepsize, numit, nchains,
+                     rngs, draws, savefile, savemodel, prior=prior, priorlow=priorlow, burnin=burnin,
+                     fgamma=fgamma, fepsilon=fepsilon, thinning=thinning, hsize=hsize, grtest=grtest)
