@@ -105,6 +105,8 @@ def lib():
     L.bart_mcmc_resume.argtypes = [C.c_int, dp]
     L.bart_mcmc_snooker_init.argtypes = [C.c_int, C.c_int, dp]
     L.bart_mcmc_run_snooker.argtypes = [C.c_int, dp, ip, ip, ip, ip, dp, ip, dp, dp]
+    L.bart_mcmc_seed.argtypes = [C.POINTER(C.c_ulonglong)]
+    L.bart_mcmc_run_seeded.argtypes = [C.c_int]
     L.bart_mcmc_get.restype = C.c_longlong
     L.bart_mcmc_get.argtypes = [C.c_char_p, dp, C.c_longlong]
     L.bart_set_error_mode(1)
@@ -359,6 +361,7 @@ class Transit:
                                              int(burnin)))
         self._mc_shape = (nretr, nchains, npars, int(np.sum(stepsize > 0)), data.shape[1])
         self._mc_lone, self._mc_niter, self._mc_zsize = False, 0, 0
+        self._mc_walk = "demc"
 
     def _mc_in(self, a, dtype):
         """An mcmc_* argument as a contiguous array behind the [R] axis (added for a lone caller)."""
@@ -392,7 +395,7 @@ class Transit:
                 "%d chains" % nchains, "%d iterations" % niter))
         _check(lib().bart_mcmc_run(niter, _d(support), r1.ctypes.data_as(ip), r2.ctypes.data_as(ip),
                                    _d(unif), _d(ugamma)))
-        self._mc_niter = niter
+        self._mc_niter, self._mc_walk = niter, "demc"
 
     def mcmc_snooker_init(self, z0, thinning=1):
         """z0[hsize][nchains][nfree] ([R][hsize][nchains][nfree] for an ensemble): MC3's M0 initial
@@ -404,6 +407,7 @@ class Transit:
                                                              "%d free parameters" % nfree))
         _check(lib().bart_mcmc_snooker_init(z0.shape[1], int(thinning), _d(z0)))
         self._mc_zsize, self._mc_thinning = z0.shape[1], int(thinning)
+        self._mc_walk = "snooker"
 
     def mcmc_run_snooker(self, support, i1, i2, iz, ic, usnooker, usn_offset, unif, ugamma):
         """Streams of run_snooker's shapes; for an ensemble each behind [R], usnooker the
@@ -425,8 +429,47 @@ class Transit:
         self._mc_niter = niter
         self._mc_zsize += len(range(0, niter, self._mc_thinning)) + 1     # upper bound, see mcmc_get
 
+    def mcmc_seed(self, keys):
+        """Philox keys of a seeded run (bart_mcmc_seed): keys[R][2] uint64 for an ensemble, [2]
+        after mcmc_init.  Retrieval r then draws what a lone run with keys[r] draws."""
+        keys = self._mc_in(keys, np.uint64)
+        if keys.shape != (self._mc_shape[0], 2):
+            raise BartError("keys must be %s" % self._mc_dims("2 uint64 words"))
+        _check(lib().bart_mcmc_seed(keys.ctypes.data_as(C.POINTER(C.c_ulonglong))))
+
+    def mcmc_run_seeded(self, niter):
+        """niter generations of the initialised walk (DE-MC, or snooker after mcmc_snooker_init) with
+        random streams drawn on the device from the mcmc_seed keys; mcmc_get returns the streams."""
+        niter = int(niter)
+        _check(lib().bart_mcmc_run_seeded(niter))
+        if niter > 0:
+            self._mc_niter = niter
+            if self._mc_walk == "snooker":
+                self._mc_zsize += len(range(0, niter, self._mc_thinning)) + 1
+
+    # the last run call's random streams: shape behind [R] and dtype
+    _STREAMS = {"support": (("n", "c", "f"), np.float64), "unif": (("n", "c"), np.float64),
+                "ugamma": (("n", "c"), np.float64), "r1": (("c", "n"), np.int64),
+                "r2": (("c", "n"), np.int64), "i1": (("n", "c"), np.int64), "i2": (("n", "c"), np.int64),
+                "iz": (("n", "c"), np.int64), "ic": (("n", "c"), np.int64),
+                "usn_offset": (("n+1",), np.int64)}
+
     def mcmc_get(self, name):
         nretr, nchains, npars, nfree, ndata = self._mc_shape
+        if name in self._STREAMS:
+            dims, dtype = self._STREAMS[name]
+            size = {"n": self._mc_niter, "c": nchains, "f": nfree, "n+1": self._mc_niter + 1}
+            out = np.zeros((nretr,) + tuple(size[d] for d in dims))
+            n = lib().bart_mcmc_get(name.encode(), _d(out), out.size)
+            _check(0 if n >= 0 else -1)
+            out = out.astype(dtype)
+            return out[0] if self._mc_lone else out
+        if name == "usnooker":                           # every retrieval's rows, no [R] axis
+            rows = int(np.asarray(self.mcmc_get("usn_offset")).ravel()[-1]) if self._mc_niter else 0
+            out = np.zeros((rows, nfree))
+            n = lib().bart_mcmc_get(name.encode(), _d(out), out.size)
+            _check(0 if n >= 0 else -1)
+            return out
         if name in ("Z", "Zchisq"):
             # _mc_zsize is an upper bound (it counts thinned rows per call; the library grows Z on
             # the GLOBAL iteration number, like MC3): size the result from what the library returns

@@ -16,6 +16,8 @@
 //                          contraction) so chains are bit-identical to numpy.
 //   chisq_accept_kernel    one CTA per retrieval: per-chain chi-squared with priors, Metropolis rule,
 //                          state update, trace, running best fit (first-index argmin like numpy).
+//   mcmc_draw_kernel       seeded runs only: the random streams of a call from per-retrieval Philox
+//   (+ usn_scan, usn_rows) keys (philox.cuh), written where host streams are uploaded to.
 //
 // An ensemble of retrievals (McmcDev::nretr) is one flattened population g = r * nchains + c for the
 // forward model; every per-retrieval step (partners, slot numbering, norm ratio, best fit, history)
@@ -26,6 +28,7 @@
 // that the per-generation host round trip (MPI scatter/gather in the reference) disappears.
 #include "retrieval.hpp"
 #include "dyn_smem.hpp"
+#include "philox.cuh"
 #include <cmath>
 
 namespace bart {
@@ -724,6 +727,125 @@ void launch_zrow_chisq(const McmcDev &mc, const double *models, ModelMap map, in
 void launch_chisq_accept(const McmcDev &mc, const double *models, ModelMap map, int first,
                          cudaStream_t s) {
   chisq_accept_kernel<<<mc.nretr, kChisqThreads, 0, s>>>(mc, models, map, first);
+}
+
+// ---------------------------------------------------------------------------------------
+// Random streams of a seeded call (philox.cuh for the generator and the counter layout).  The
+// constructions are MC3's (mcmc.py:484-507 for DE-MC, 529-556 for snooker), so the proposal
+// distribution is MC3's; only the random numbers differ.
+
+// numpy's legacy polar method (separately rounded, so acceptance decisions are numpy's); a
+// rejected pair is followed by the next attempt's
+__device__ double polar_normal(unsigned long long k0, unsigned long long k1, long long it, int c, int f) {
+  for (int a = 0;; a++) {
+    const Philox4 b = draw_block(k0, k1, DRAW_SUPPORT, it, c, f, a);
+    const double u = __dsub_rn(__dmul_rn(2.0, u01(b.x[0])), 1.0);
+    const double v = __dsub_rn(__dmul_rn(2.0, u01(b.x[1])), 1.0);
+    const double s = __dadd_rn(__dmul_rn(u, u), __dmul_rn(v, v));
+    if (s > 0.0 && s < 1.0) return __dmul_rn(u, sqrt(__ddiv_rn(__dmul_rn(-2.0, log(s)), s)));
+  }
+}
+
+// rows of the snooker history at generation i of the call: Z grows after every generation whose
+// global iteration is a multiple of the thinning (chisq_accept_kernel)
+__device__ __forceinline__ int history_rows(const DrawArgs &d, int i) {
+  const long long th = d.thinning, a = d.it0, b = d.it0 + i;
+  return d.zs0 + (int)((b + th - 1) / th - (a + th - 1) / th);
+}
+
+// one thread per (retrieval, generation, chain): everything but the snooker factor rows
+__global__ void __launch_bounds__(256) mcmc_draw_kernel(DrawArgs d) {
+  const long long g = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  const int nc = d.nchains;
+  if (g >= (long long)d.nretr * d.niter * nc) return;
+  const int c = (int)(g % nc);
+  const long long ri = g / nc;                 // r * niter + i
+  const int i = (int)(ri % d.niter), r = (int)(ri / d.niter);
+  const unsigned long long k0 = d.keys[2 * r], k1 = d.keys[2 * r + 1];
+  const long long it = d.it0 + i;
+  for (int f = 0; f < d.nfree; f++)
+    d.support[g * d.nfree + f] = __dmul_rn(d.step[f], polar_normal(k0, k1, it, c, f));
+  d.unif[g] = u01(draw_block(k0, k1, DRAW_UNIF, it, c, 0, 0).x[0]);
+  d.ugamma[g] = u01(draw_block(k0, k1, DRAW_UGAMMA, it, c, 0, 0).x[0]);
+  if (d.walk == 0) {                           // mcmc.py:498-505; r1 / r2 are [nretr][nchains][niter]
+    int a = randint(draw_block(k0, k1, DRAW_R1, it, c, 0, 0).x[0], 0, nc - 1);
+    if (a == c) a = nc - 1;
+    int b = (c + randint(draw_block(k0, k1, DRAW_R2, it, c, 0, 0).x[0], 1, nc - 1)) % nc;
+    if (b == a) b = (c - 1 + nc) % nc;
+    const size_t k = ((size_t)r * nc + c) * d.niter + i;
+    d.r1[k] = a;
+    d.r2[k] = b;
+    return;
+  }
+  const int zs = history_rows(d, i);           // mcmc.py:529-539
+  const long long lim = (long long)(zs - 1) * nc;
+  const int a = randint(draw_block(k0, k1, DRAW_I1, it, c, 0, 0).x[0], 0, lim);
+  int b, t = 0;
+  do b = randint(draw_block(k0, k1, DRAW_I2, it, c, 0, t++).x[0], 0, lim);
+  while (b == a);
+  d.i1[g] = a;
+  d.i2[g] = b;
+  d.iz[g] = randint(draw_block(k0, k1, DRAW_IZ, it, c, 0, 0).x[0], 0, zs - 1);
+  d.ic[g] = randint(draw_block(k0, k1, DRAW_IC, it, c, 0, 0).x[0], 0, nc);
+}
+
+// usn_off[r][i]: first factor row of generation i of retrieval r, rows of the whole call counted
+// in (retrieval, generation) order, usn_off[r][niter] = usn_off[r + 1][0].  One CTA: a thread
+// counts a contiguous run of generations, the runs' counts are scanned in shared memory.
+constexpr int kScanThreads = 1024;
+__global__ void __launch_bounds__(kScanThreads) usn_scan_kernel(DrawArgs d) {
+  __shared__ int s[kScanThreads];
+  const int t = threadIdx.x, nc = d.nchains, n = d.niter;
+  const long long E = (long long)d.nretr * n, per = (E + kScanThreads - 1) / kScanThreads;
+  const long long lo = min(E, t * per), hi = min(E, lo + per);
+  int sum = 0;
+  for (long long e = lo; e < hi; e++)
+    for (int c = 0; c < nc; c++) sum += d.ugamma[e * nc + c] < 0.1;
+  s[t] = sum;
+  __syncthreads();
+  for (int o = 1; o < kScanThreads; o <<= 1) {
+    const int v = t >= o ? s[t - o] : 0;
+    __syncthreads();
+    s[t] += v;
+    __syncthreads();
+  }
+  int run = s[t] - sum;
+  for (long long e = lo; e < hi; e++) {
+    const int r = (int)(e / n), i = (int)(e - (long long)r * n);
+    d.usn_off[(size_t)r * (n + 1) + i] = run;
+    for (int c = 0; c < nc; c++) run += d.ugamma[e * nc + c] < 0.1;
+    if (i == n - 1) d.usn_off[(size_t)r * (n + 1) + n] = run;
+  }
+}
+
+// uniform(1.2, 2.2) factors of the chains with ugamma < 0.1 (mcmc.py:545-556), one row each in chain
+// order within a generation; one thread per (retrieval, generation, chain)
+__global__ void __launch_bounds__(256) usn_rows_kernel(DrawArgs d) {
+  const long long g = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  const int nc = d.nchains;
+  if (g >= (long long)d.nretr * d.niter * nc) return;
+  const int c = (int)(g % nc);
+  const long long ri = g / nc;
+  const int i = (int)(ri % d.niter), r = (int)(ri / d.niter);
+  const double *ug = d.ugamma + ri * nc;
+  if (!(ug[c] < 0.1)) return;
+  int row = d.usn_off[(size_t)r * (d.niter + 1) + i];
+  for (int k = 0; k < c; k++) row += ug[k] < 0.1;
+  const unsigned long long k0 = d.keys[2 * r], k1 = d.keys[2 * r + 1];
+  const double w = 2.2 - 1.2;                  // numpy's uniform(low, high): low + (high - low) u
+  for (int f = 0; f < d.nfree; f++)
+    d.usn[(size_t)row * d.nfree + f] =
+        __dadd_rn(1.2, __dmul_rn(w, u01(draw_block(k0, k1, DRAW_USN, d.it0 + i, c, f, 0).x[0])));
+}
+
+void launch_mcmc_draws(const DrawArgs &d, cudaStream_t s) {
+  const long long n = (long long)d.nretr * d.niter * d.nchains;
+  if (n <= 0) return;
+  const int blocks = (int)((n + 255) / 256);
+  mcmc_draw_kernel<<<blocks, 256, 0, s>>>(d);
+  if (d.walk == 0) return;
+  usn_scan_kernel<<<1, kScanThreads, 0, s>>>(d);
+  usn_rows_kernel<<<blocks, 256, 0, s>>>(d);
 }
 
 }  // namespace bart

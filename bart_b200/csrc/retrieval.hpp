@@ -7,6 +7,9 @@
 //   K9  snooker_propose_kernel  DE-MC-with-snooker proposal from the sample history Z
 //                               (ter Braak & Vrugt 2008; mcmc.py:527-561)
 //   K10 zrow_chisq_kernel       chi-squared of the initial Z samples (mcmc.py:426-460)
+//   K11 mcmc_draw_kernel,       the random streams of a seeded call from per-retrieval Philox
+//       usn_scan_kernel,        keys (philox.cuh): MC3's constructions (mcmc.py:484-507,529-556),
+//       usn_rows_kernel         other random numbers
 #pragma once
 #include "device.cuh"
 #include <cuda_runtime.h>
@@ -106,6 +109,22 @@ BART_HD size_t zidx(const McmcDev &mc, int row, int r, int c) {
 // where model g (of the flattened population) sits in the gathered band-flux buffer: rank blocks of
 // `pad` rows
 struct ModelMap { int world, base, extra, pad; };
+
+// Random streams of a seeded call (bart_mcmc_run_seeded, philox.cuh), written into the buffers a
+// host-stream call uploads into, in McmcDev's layouts.  DE-MC fills support / unif / ugamma / r1 / r2,
+// snooker support / unif / ugamma / i1 / i2 / iz / ic / usn_off / usn (usn sized for every chain).
+struct DrawArgs {
+  const unsigned long long *keys;          // [nretr][2]
+  const double *step;                      // [nfree] step sizes of the free parameters
+  int nretr, nchains, nfree, niter, walk;
+  long long it0;                           // global iteration of the call's generation 0
+  int zs0, thinning;                       // snooker: history rows at generation 0, thinning
+  double *support, *unif, *ugamma;
+  int *r1, *r2, *i1, *i2, *iz, *ic, *usn_off;
+  double *usn;
+};
+// draw kernel, then (snooker) the usn_off scan and the factor rows
+void launch_mcmc_draws(const DrawArgs &d, cudaStream_t s);
 
 // one warp per (retrieval, chain)
 void launch_demc_propose(const McmcDev &mc, cudaStream_t s);

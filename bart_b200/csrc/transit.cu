@@ -140,6 +140,11 @@ struct Config {
   int mc_zsize = 0;                        // host mirror of the device row counter
   size_t mc_zcap = 0;                      // rows allocated
   std::vector<double> mc_ztemplate;        // [nretr][nchains][npars] what an unfilled row holds
+  // seeded runs (bart_mcmc_seed / bart_mcmc_run_seeded): per-retrieval Philox keys and the free
+  // parameters' step sizes
+  DevBuf<unsigned long long> d_mckeys;
+  DevBuf<double> d_mcstep;
+  bool mc_seeded = false;
 };
 
 // The process: the device, its streams, the communicator and peer window, profiling and debug
@@ -1898,6 +1903,10 @@ int bart_mcmc_init_ensemble(int nretr, int nchains, int npars, const double *par
   upload(mb.outbounds, zi); mc.outbounds = mb.outbounds.p;
   zi.assign(ntot, 0); upload(mb.outflag, zi); mc.outflag = mb.outflag.p;
   zi.assign(nretr, 0); upload(mb.iter, zi); mc.iter = mb.iter.p;
+  std::vector<double> step;
+  for (int f = 0; f < mc.nfree; f++) step.push_back(stepsize[mc.ifree[f]]);
+  upload(G.d_mcstep, step);
+  G.mc_seeded = false;
   G.mc = mc;
   G.mc_ztemplate = p0;
   G.mc_zsize = 0;
@@ -2137,6 +2146,118 @@ int bart_mcmc_run_snooker(int niter, const double *support, const int *i1, const
   API_END_INT
 }
 
+// keys[nretr][2]: the 128-bit Philox key of every retrieval of the loop set up by the last
+// bart_mcmc_init(_ensemble); retrieval r of an ensemble then draws what a lone run with r's key draws
+int bart_mcmc_seed(const unsigned long long *keys) {
+  API_BEGIN
+  if (!G.mc_ready) fail("bart_mcmc_init has not been called");
+  if (!keys) fail("bart_mcmc_seed: no keys");
+  std::vector<unsigned long long> k(keys, keys + 2 * (size_t)G.mc.nretr);
+  upload(G.d_mckeys, k);
+  G.mc_seeded = true;
+  return 0;
+  API_END_INT
+}
+
+// niter generations of the walk set up (DE-MC, or snooker after bart_mcmc_snooker_init) with random
+// streams drawn on the device from the retrievals' keys (philox.cuh): one draw launch (snooker: plus
+// the factor-row scan) fills the buffers bart_mcmc_run / bart_mcmc_run_snooker upload into, then
+// the generations run as they do there.  Counters are global iterations, so seeded and host-stream
+// calls may alternate.
+int bart_mcmc_run_seeded(int niter) {
+  API_BEGIN
+  if (!G.mc_ready) fail("bart_mcmc_init has not been called");
+  if (!G.mc_seeded) fail("bart_mcmc_run_seeded: no keys (bart_mcmc_seed must follow bart_mcmc_init)");
+  if (niter <= 0) return 0;
+  McmcDev &mc = G.mc;
+  const int nc = mc.nchains, nr = mc.nretr;
+  if (nc < 3) fail("DE-MC needs at least 3 chains (got %d)", nc);
+  const bool snooker = mc.walk == 1;
+  DrawArgs d{};
+  d.keys = G.d_mckeys.p; d.step = G.d_mcstep.p;
+  d.nretr = nr; d.nchains = nc; d.nfree = mc.nfree; d.niter = niter; d.walk = mc.walk;
+  d.it0 = (long long)mc.nold + mc.chainsize;
+  if (snooker) {
+    const long long th = mc.thinning, a = d.it0, b = d.it0 + niter;
+    const int zs = G.mc_zsize + (int)((b + th - 1) / th - (a + th - 1) / th);
+    snooker_reserve_rows((size_t)zs + 1);
+    d.zs0 = G.mc_zsize; d.thinning = mc.thinning;
+    G.mc_zsize = zs;
+  }
+  mc.nold += mc.chainsize;
+  mc.chainsize = niter;
+  const size_t n1 = (size_t)nr * niter * nc;
+  d.support = G.mcb.support.ensure(n1 * mc.nfree);
+  d.unif = G.mcb.unif.ensure(n1);
+  d.ugamma = G.mcb.ugamma.ensure(n1);
+  if (snooker) {
+    int *pk = G.d_snk_idx.ensure(4 * n1);
+    d.i1 = pk; d.i2 = pk + n1; d.iz = pk + 2 * n1; d.ic = pk + 3 * n1;
+    d.usn_off = G.d_snk_off.ensure((size_t)nr * (niter + 1));
+    d.usn = G.d_snk_usn.ensure(n1 * mc.nfree);         // row count known on the device only
+    mc.i1 = d.i1; mc.i2 = d.i2; mc.iz = d.iz; mc.ic = d.ic;
+    mc.usn_off = d.usn_off; mc.usn = d.usn;
+  } else {
+    d.r1 = G.mcb.r1.ensure(n1);
+    d.r2 = G.mcb.r2.ensure(n1);
+    mc.r1 = d.r1; mc.r2 = d.r2;
+  }
+  mc.support = d.support; mc.unif = d.unif; mc.ugamma = d.ugamma;
+  {
+    KernelScope ks("mcmc_draws");
+    launch_mcmc_draws(d, G.stream);
+    check_launch("mcmc_draws");
+  }
+  mc.allparams = G.mcb.allparams.ensure(n1 * mc.nfree);
+  G.d_mcallm.ensure(n1 * mc.ndata);
+  mc.allmodel = G.d_mcallm.p;
+  mcmc_run_generations(niter);
+  return 0;
+  API_END_INT
+}
+
+// the last run call's random streams as doubles, in the layouts bart_mcmc_run (support, r1, r2,
+// unif, ugamma) / bart_mcmc_run_snooker (support, i1, i2, iz, ic, usnooker, usn_offset, unif,
+// ugamma) take them; 0 before the first run
+static long long get_stream(const std::string &n, double *out, long long capacity) {
+  const McmcDev &mc = G.mc;
+  const long long n1 = (long long)mc.nretr * mc.nchains * mc.chainsize;
+  if (mc.chainsize == 0 || !mc.support) return 0;
+  const bool demc_name = n == "r1" || n == "r2";
+  const bool snk_name = n == "i1" || n == "i2" || n == "iz" || n == "ic" || n == "usnooker" || n == "usn_offset";
+  if ((demc_name && mc.walk != 0) || (snk_name && mc.walk != 1))
+    fail("bart_mcmc_get(%s): the last run was a %s run", n.c_str(), mc.walk ? "snooker" : "DE-MC");
+  const double *dsrc = nullptr;
+  const int *isrc = nullptr;
+  long long cnt = n1;
+  if (n == "support") { dsrc = mc.support; cnt = n1 * mc.nfree; }
+  else if (n == "unif") dsrc = mc.unif;
+  else if (n == "ugamma") dsrc = mc.ugamma;
+  else if (n == "r1") isrc = mc.r1;
+  else if (n == "r2") isrc = mc.r2;
+  else if (n == "i1") isrc = mc.i1;
+  else if (n == "i2") isrc = mc.i2;
+  else if (n == "iz") isrc = mc.iz;
+  else if (n == "ic") isrc = mc.ic;
+  else if (n == "usn_offset") { isrc = mc.usn_off; cnt = (long long)mc.nretr * (mc.chainsize + 1); }
+  else {                                                   // usnooker
+    int rows = 0;
+    CUDA_OK(cudaMemcpy(&rows, mc.usn_off + (size_t)mc.nretr * (mc.chainsize + 1) - 1, sizeof(int),
+                       cudaMemcpyDeviceToHost));
+    dsrc = mc.usn; cnt = (long long)rows * mc.nfree;
+  }
+  if (cnt > capacity) fail("bart_mcmc_get(%s): capacity %lld < %lld", n.c_str(), capacity, cnt);
+  if (!cnt) return 0;
+  if (dsrc) {
+    CUDA_OK(cudaMemcpy(out, dsrc, cnt * 8, cudaMemcpyDeviceToHost));
+  } else {
+    std::vector<int> tmp(cnt);
+    CUDA_OK(cudaMemcpy(tmp.data(), isrc, cnt * 4, cudaMemcpyDeviceToHost));
+    for (long long i = 0; i < cnt; i++) out[i] = tmp[i];
+  }
+  return cnt;
+}
+
 // results of the DE-MC loop: "allparams" [nchains][nfree][niter of the last run] (MC3's trace
 // layout), "params" [nchains][npars], "currchisq", "numaccept" [nchains], "outbounds"
 // [nchains][nfree], "bestp" [npars], "bestchisq" [1], "bestmodel" [ndata], "models" (band fluxes of
@@ -2191,6 +2312,9 @@ long long bart_mcmc_get(const char *name, double *out, long long capacity) {
                            (size_t)(hi - lo) * mc.ndata * 8, cudaMemcpyDeviceToHost));
     }
     return cnt;
+  } else if (n == "support" || n == "r1" || n == "r2" || n == "unif" || n == "ugamma" || n == "i1" ||
+             n == "i2" || n == "iz" || n == "ic" || n == "usnooker" || n == "usn_offset") {
+    return get_stream(n, out, capacity);
   } else fail("bart_mcmc_get: unknown name '%s'", name);
   if (!src) return 0;
   if (cnt > capacity) fail("bart_mcmc_get(%s): capacity %lld < %lld", name, capacity, cnt);

@@ -275,7 +275,8 @@ def start_points(params, nchains, stepsize, pmin, pmax, rng):
 
 def run_demc(transit, data, uncert, params, pmin, pmax, stepsize, numit, nchains, prior=None,
              priorlow=None, burnin=0, fgamma=1.0, fepsilon=0.0, rng=np.random, draws=None,
-             savefile=None, savemodel=None, grtest=False, grexit=False, thinning=1, resume=False):
+             savefile=None, savemodel=None, grtest=False, grexit=False, thinning=1, resume=False,
+             seed=None):
     """`MCcubed.mc.mcmc(..., walk='demc', leastsq=False)` with the whole generation loop on the
     GPU: the host only draws the random streams (once, up front, exactly like mcmc.py does) and
     reads the trace back at the end.  `transit` must have its converter and filters set
@@ -284,7 +285,10 @@ def run_demc(transit, data, uncert, params, pmin, pmax, stepsize, numit, nchains
     resume=True continues the run whose `savefile` (and `savemodel`) are on disk, like
     mcmc.py:254-269: chains restart from their last states, the new iterations are appended to the
     old traces, burn-in and the convergence test count from the old run's first iteration.
-    The run is an ensemble of one (see _retrieve)."""
+    seed (an int or a pair of uint64 words, see seed_key; not with `draws`): the random streams are
+    drawn on the device from that Philox key instead of from `rng` (start points still come from
+    `rng`); a resumed seeded run draws from iteration nold on.  The run is an ensemble of one (see
+    _retrieve)."""
     old = None
     if resume:
         oldparams = np.load(savefile)
@@ -297,7 +301,8 @@ def run_demc(transit, data, uncert, params, pmin, pmax, stepsize, numit, nchains
                      np.asarray(uncert, dtype=float)[None], [params], pmin, pmax, stepsize, numit,
                      nchains, [rng], None if draws is None else [draws], [savefile], [savemodel],
                      prior=prior, priorlow=priorlow, burnin=burnin, fgamma=fgamma, fepsilon=fepsilon,
-                     thinning=thinning, grtest=grtest, grexit=grexit, old=old)[0]
+                     thinning=thinning, grtest=grtest, grexit=grexit, old=old,
+                     seeds=None if seed is None else [seed])[0]
 
 
 def gelman_rubin(chains):
@@ -368,6 +373,29 @@ def _save_mc3_files(out, savefile, savemodel):
         np.save(savemodel, out["allmodel"])
 
 
+def snooker_z0(rng, nchains, hsize, pmin_free, pmax_free):
+    """MC3's M0 = hsize x nchains initial history samples (mcmc.py:421-424), uniform in the free
+    parameters' bounds, one parameter after the other."""
+    z0 = np.zeros((hsize, nchains, len(pmin_free)))
+    for f in range(len(pmin_free)):
+        z0[:, :, f] = rng.uniform(pmin_free[f], pmax_free[f], (hsize, nchains))
+    return z0
+
+
+def seed_key(seed):
+    """The 128-bit Philox key (k0, k1) of a seeded run: an int k in [0, 2^128) is (k mod 2^64,
+    k >> 64); a pair of uint64 words is taken as is."""
+    if isinstance(seed, (int, np.integer)):
+        seed = int(seed)
+        if not 0 <= seed < 1 << 128:
+            raise ValueError("a seed must be in [0, 2**128)")
+        return (seed & 0xFFFFFFFFFFFFFFFF, seed >> 64)
+    k = [int(w) for w in seed]
+    if len(k) != 2 or not all(0 <= w < 1 << 64 for w in k):
+        raise ValueError("a seed is an int or a pair of uint64 words")
+    return tuple(k)
+
+
 def snooker_draws(rng, nchains, nfree, chainsize, hsize, thinning, step_free, pmin_free, pmax_free):
     """The random numbers MC3's walk='snooker' consumes, in its order: the M0 initial history
     samples (mcmc.py:421-424), support / unif / ugamma (490-497), then per generation i1, i2 with
@@ -375,9 +403,7 @@ def snooker_draws(rng, nchains, nfree, chainsize, hsize, thinning, step_free, pm
     generation's snooker chains (545-556; the reference's two calls take, together,
     [chains with ugamma < 0.1][nfree] values however they split).  None of these depends on the
     chain states, so the host draws them up front and the generation loop stays on the device."""
-    z0 = np.zeros((hsize, nchains, nfree))
-    for f in range(nfree):
-        z0[:, :, f] = rng.uniform(pmin_free[f], pmax_free[f], (hsize, nchains))
+    z0 = snooker_z0(rng, nchains, hsize, pmin_free, pmax_free)
     support = rng.normal(0, step_free, (chainsize, nchains, nfree))
     unif = rng.uniform(0, 1, (chainsize, nchains))
     ugamma = rng.uniform(0, 1, (chainsize, nchains))
@@ -407,16 +433,19 @@ def snooker_draws(rng, nchains, nfree, chainsize, hsize, thinning, step_free, pm
 
 def run_snooker(transit, data, uncert, params, pmin, pmax, stepsize, numit, nchains, prior=None,
                 priorlow=None, burnin=0, thinning=1, fgamma=1.0, fepsilon=0.0, hsize=1,
-                rng=np.random, draws=None, savefile=None, savemodel=None, grtest=False, grexit=False):
+                rng=np.random, draws=None, savefile=None, savemodel=None, grtest=False, grexit=False,
+                seed=None):
     """`MCcubed.mc.mcmc(..., walk='snooker', leastsq=False)` -- the walk BART's examples configure
     -- with the sample history Z, the proposals, the Metropolis rule and the forward models all on
-    the GPU.  Returns MC3's arrays (see run_demc) plus Z and Zchisq.  The run is an ensemble of
-    one (see _retrieve)."""
+    the GPU.  Returns MC3's arrays (see run_demc) plus Z and Zchisq.  seed: streams drawn on the
+    device as in run_demc (start points and the initial history z0 still come from `rng`).  The run
+    is an ensemble of one (see _retrieve)."""
     return _retrieve(transit, "snooker", np.asarray(data, dtype=float)[None],
                      np.asarray(uncert, dtype=float)[None], [params], pmin, pmax, stepsize, numit,
                      nchains, [rng], None if draws is None else [draws], [savefile], [savemodel],
                      prior=prior, priorlow=priorlow, burnin=burnin, fgamma=fgamma, fepsilon=fepsilon,
-                     thinning=thinning, hsize=hsize, grtest=grtest, grexit=grexit)[0]
+                     thinning=thinning, hsize=hsize, grtest=grtest, grexit=grexit,
+                     seeds=None if seed is None else [seed])[0]
 
 
 # ---------------------------------------------------------------------------------------------
@@ -424,10 +453,11 @@ def run_snooker(transit, data, uncert, params, pmin, pmax, stepsize, numit, ncha
 # (Transit.mcmc_init_ensemble), a lone run_demc / run_snooker being R = 1.  Every generation
 # evaluates R x nchains models as one batch.  Long runs go through the device in segments of at most
 # _segment_cap generations, so the stacked stream and trace arrays of one device call stay under
-# ENSEMBLE_CALL_BYTES.  Total host memory is not bounded: every retrieval's streams are drawn up
-# front in MC3's order (what makes its chains MC3's), and the returned traces hold every
-# generation -- at R = 64, 10 chains, 9 free parameters and 1e5 generations the `support` draws
-# alone are 4.6 GB.
+# ENSEMBLE_CALL_BYTES.  With host streams (the default) total host memory is not bounded: every
+# retrieval's streams are drawn up front in MC3's order (what makes its chains MC3's) -- at R = 64,
+# 10 chains, 9 free parameters and 1e5 generations the `support` draws alone are 4.6 GB.  Seeded
+# runs (seeds=...) draw their streams on the device, call by call, and hold none on the host; in
+# either mode the returned traces hold every generation.
 ENSEMBLE_CALL_BYTES = 1 << 28          # host stream + trace arrays of one device call
 
 
@@ -454,36 +484,47 @@ def stack_snooker_draws(draws, lo, hi):
             np.stack(offs), st("unif"), st("ugamma"))
 
 
-def _segment_cap(nretr, nchains, nfree, ndata, extra=0):
-    """Generations of one device call so that its host arrays stay under ENSEMBLE_CALL_BYTES."""
+def _segment_cap(nretr, nchains, nfree, ndata, extra=0, streams=True):
+    """Generations of one device call so that its host arrays stay under ENSEMBLE_CALL_BYTES
+    (streams=False: a seeded call, trace arrays only)."""
+    if not streams:
+        return max(1, int(ENSEMBLE_CALL_BYTES // (nretr * nchains * 8 * (nfree + ndata))))
     per_gen = nretr * nchains * (8 * (2 * nfree + ndata + 2 + extra) + 2 * 4)
     return max(1, int(ENSEMBLE_CALL_BYTES // per_gen))
 
 
 def _retrieve(transit, walk, data, uncert, params, pmin, pmax, stepsize, numit, nchains, rngs, draws,
               savefile, savemodel, prior=None, priorlow=None, burnin=0, fgamma=1.0, fepsilon=0.0,
-              thinning=1, hsize=1, grtest=False, grexit=False, old=None):
+              thinning=1, hsize=1, grtest=False, grexit=False, old=None, seeds=None):
     """R retrievals of `walk` ('demc' or 'snooker') in one device loop.  data / uncert[R][ndata];
     params, rngs, draws, savefile and savemodel one entry per retrieval (rngs, draws, savefile and
     savemodel may also be None); draws that are not given are drawn from the rngs after the start
     points.  `old` = (allparams[R][C][F][nold], allmodel[R][C][D][nold], last model column[R][C][D]
-    or None) of the runs being resumed.  Returns R dicts of MC3's arrays, each also written to its
-    savefile / savemodel."""
+    or None) of the runs being resumed.  seeds: one seed_key argument per retrieval; the streams
+    are then drawn on the device from those keys (draws must be None).  Returns R dicts of MC3's
+    arrays, each also written to its savefile / savemodel."""
     data = np.asarray(data, dtype=float)
     uncert = np.asarray(uncert, dtype=float)
     nretr = data.shape[0]
     if nretr < 1 or data.ndim != 2 or uncert.shape != data.shape or len(params) != nretr:
         raise ValueError("data, uncert and params need one entry per retrieval")
-    for name, v in (("rngs", rngs), ("draws", draws)):
+    for name, v in (("rngs", rngs), ("draws", draws), ("seeds", seeds)):
         if v is not None and len(v) != nretr:
             raise ValueError("%s needs one entry per retrieval (%d)" % (name, nretr))
+    if seeds is not None and draws is not None:
+        raise ValueError("seed and draws are mutually exclusive: a seeded run draws its streams on "
+                         "the device")
+    keys = None if seeds is None else np.array([seed_key(s) for s in seeds], dtype=np.uint64)
+    if keys is not None and walk == "demc" and nchains < 3:
+        raise ValueError("DE-MC needs at least 3 chains (got %d)" % nchains)
     pmin, pmax, stepsize = (np.asarray(a, dtype=float) for a in (pmin, pmax, stepsize))
     ifree = np.where(stepsize > 0)[0]
     chainsize = int(np.ceil(numit / nchains))
     starts = []
     for r in range(nretr):
         rng = rngs[r] if rngs is not None else None
-        if rng is None and (np.atleast_2d(params[r]).shape[0] != nchains or draws is None):
+        drawn = draws is None and (keys is None or walk == "snooker")       # streams or z0 from rng
+        if rng is None and (np.atleast_2d(params[r]).shape[0] != nchains or drawn):
             raise ValueError("retrieval %d needs an rng (its start points or random streams are "
                              "drawn)" % r)
         starts.append(start_points(params[r], nchains, stepsize, pmin, pmax, rng))
@@ -492,27 +533,37 @@ def _retrieve(transit, walk, data, uncert, params, pmin, pmax, stepsize, numit, 
     nold = 0 if old is None else old[0].shape[-1]
     if old is not None:
         transit.mcmc_resume(nold, old[2])
+    if keys is not None:
+        transit.mcmc_seed(keys)
     if walk == "demc":
-        if draws is None:
-            draws = [demc_draws(rng, nchains, chainsize, stepsize[ifree]) for rng in rngs]
-        run = lambda lo, hi: transit.mcmc_run(*stack_demc_draws(draws, lo, hi))
-        keys, extra = (), 0
+        if keys is not None:
+            run = lambda lo, hi: transit.mcmc_run_seeded(hi - lo)
+        else:
+            if draws is None:
+                draws = [demc_draws(rng, nchains, chainsize, stepsize[ifree]) for rng in rngs]
+            run = lambda lo, hi: transit.mcmc_run(*stack_demc_draws(draws, lo, hi))
+        zkeys, extra = (), 0
     else:
         if hsize < nchains:                                          # mcmc.py:233-235
             hsize = nchains + 1
-        if draws is None:
-            draws = [snooker_draws(rng, nchains, len(ifree), chainsize, hsize, thinning,
-                                   stepsize[ifree], pmin[ifree], pmax[ifree]) for rng in rngs]
-        transit.mcmc_snooker_init(np.stack([d["z0"] for d in draws]), thinning)
-        run = lambda lo, hi: transit.mcmc_run_snooker(*stack_snooker_draws(draws, lo, hi))
-        keys, extra = ("Z", "Zchisq"), len(ifree) / 5 + 2
+        if keys is not None:
+            z0 = np.stack([snooker_z0(rng, nchains, hsize, pmin[ifree], pmax[ifree]) for rng in rngs])
+            run = lambda lo, hi: transit.mcmc_run_seeded(hi - lo)
+        else:
+            if draws is None:
+                draws = [snooker_draws(rng, nchains, len(ifree), chainsize, hsize, thinning,
+                                       stepsize[ifree], pmin[ifree], pmax[ifree]) for rng in rngs]
+            z0 = np.stack([d["z0"] for d in draws])
+            run = lambda lo, hi: transit.mcmc_run_snooker(*stack_snooker_draws(draws, lo, hi))
+        transit.mcmc_snooker_init(z0, thinning)
+        zkeys, extra = ("Z", "Zchisq"), len(ifree) / 5 + 2
     allp, allm, history, chainlen = run_segments(
         run, lambda: (transit.mcmc_get("allparams"), transit.mcmc_get("allmodel")), chainsize,
         burnin=burnin, thinning=thinning, grtest=grtest, grexit=grexit, nold=nold,
         old=None if old is None else old[:2],
-        max_segment=_segment_cap(nretr, nchains, len(ifree), data.shape[1], extra))
+        max_segment=_segment_cap(nretr, nchains, len(ifree), data.shape[1], extra, streams=keys is None))
     got = {k: transit.mcmc_get(k) for k in ("params", "currchisq", "numaccept", "outbounds", "bestp",
-                                            "bestmodel", "models") + keys}
+                                            "bestmodel", "models") + zkeys}
     bestchisq = transit.mcmc_get("bestchisq")
     outs = []
     for r in range(nretr):
@@ -530,12 +581,14 @@ def _retrieve(transit, walk, data, uncert, params, pmin, pmax, stepsize, numit, 
 def run_demc_ensemble(transit, data, uncert, params, pmin, pmax, stepsize, numit, nchains,
                       prior=None, priorlow=None, burnin=0, fgamma=1.0, fepsilon=0.0, rngs=None,
                       draws=None, savefile=None, savemodel=None, grtest=False, grexit=False,
-                      thinning=1):
+                      thinning=1, seeds=None):
     """`run_demc` for R retrievals of the same configuration in one device loop: data /
     uncert[R][ndata], params[R] (each what run_demc takes: one start point, scattered with that
     retrieval's rng as mcmc.py:296-306 does, or one row per chain), rngs / draws one per retrieval
     (draws as demc_draws returns them), savefile / savemodel one path per retrieval.  Returns a list
     of R dicts with run_demc's keys; retrieval r equals run_demc on its own data and streams.
+    seeds: one seed per retrieval (see run_demc's seed; not with draws); retrieval r then equals
+    run_demc with seed=seeds[r].
     grexit is refused: the retrievals would stop at different iterations.  One device call's host
     arrays are bounded, the whole run's are not (see ENSEMBLE_CALL_BYTES)."""
     if grexit:
@@ -543,19 +596,21 @@ def run_demc_ensemble(transit, data, uncert, params, pmin, pmax, stepsize, numit
                          "different iterations")
     return _retrieve(transit, "demc", data, uncert, params, pmin, pmax, stepsize, numit, nchains,
                      rngs, draws, savefile, savemodel, prior=prior, priorlow=priorlow, burnin=burnin,
-                     fgamma=fgamma, fepsilon=fepsilon, thinning=thinning, grtest=grtest)
+                     fgamma=fgamma, fepsilon=fepsilon, thinning=thinning, grtest=grtest, seeds=seeds)
 
 
 def run_snooker_ensemble(transit, data, uncert, params, pmin, pmax, stepsize, numit, nchains,
                          prior=None, priorlow=None, burnin=0, thinning=1, fgamma=1.0, fepsilon=0.0,
                          hsize=1, rngs=None, draws=None, savefile=None, savemodel=None,
-                         grtest=False, grexit=False):
+                         grtest=False, grexit=False, seeds=None):
     """`run_snooker` for R retrievals in one device loop (arguments as run_demc_ensemble; draws as
     snooker_draws returns them).  hsize and thinning are shared, so every retrieval's history grows
-    on the same schedule.  Returns a list of R dicts with run_snooker's keys."""
+    on the same schedule.  seeds as in run_demc_ensemble.  Returns a list of R dicts with
+    run_snooker's keys."""
     if grexit:
         raise ValueError("grexit is not offered for ensembles: the retrievals would stop at "
                          "different iterations")
     return _retrieve(transit, "snooker", data, uncert, params, pmin, pmax, stepsize, numit, nchains,
                      rngs, draws, savefile, savemodel, prior=prior, priorlow=priorlow, burnin=burnin,
-                     fgamma=fgamma, fepsilon=fepsilon, thinning=thinning, hsize=hsize, grtest=grtest)
+                     fgamma=fgamma, fepsilon=fepsilon, thinning=thinning, hsize=hsize, grtest=grtest,
+                     seeds=seeds)

@@ -313,13 +313,27 @@ int  bart_mcmc_snooker_init(int hsize, int thinning, const double *z0);
 int  bart_mcmc_run_snooker(int niter, const double *support, const int *i1, const int *i2,
                            const int *iz, const int *ic, const double *usnooker,
                            const int *usn_offset, const double *unif, const double *ugamma);
+/* Seeded runs: random streams drawn on the device instead of passed in.  bart_mcmc_seed, after
+ * bart_mcmc_init(_ensemble), sets keys[nretr][2], one 128-bit Philox4x64-10 key per retrieval.
+ * bart_mcmc_run_seeded(niter) then runs niter generations of the initialised walk (DE-MC, or
+ * snooker after bart_mcmc_snooker_init) with MC3's proposal constructions fed by draws that are
+ * pure functions of (key, purpose, global iteration, chain, element) -- the counter layout is in
+ * bart_b200/csrc/philox.cuh -- so retrieval r of an ensemble equals a lone run with r's key, and
+ * host-stream and seeded calls may alternate.  A seeded chain is not MC3's chain (the random
+ * numbers differ); it is replayed exactly by bart_mcmc_run* fed the streams bart_mcmc_get returns.
+ * bart_mcmc_run_seeded refuses to run before bart_mcmc_seed.                                     */
+int  bart_mcmc_seed(const unsigned long long *keys);
+int  bart_mcmc_run_seeded(int niter);
 /* "allparams" [nchains][nfree][niter] (MC3's `savefile` array, BART's output.npy), "allmodel"
  * [nchains][ndata][niter] (MC3's `savemodel` array, mcmc.py:636-651,849-850: the model of every
  * chain's current state, zeros until its first acceptance like the reference), "params",
  * "currchisq", "numaccept", "outbounds", "bestp", "bestchisq", "bestmodel", "models", and for
  * snooker "Z" [Zsize][nchains][npars], "Zchisq" [Zsize][nchains]; each behind a leading [nretr]
  * (bestp [nretr][npars], bestchisq [nretr], bestmodel [nretr][ndata]), retrieval-major; with
- * nretr = 1 the layouts are those of one retrieval.  Returns the number of doubles written or < 0. */
+ * nretr = 1 the layouts are those of one retrieval.  The last run call's random streams, host or
+ * seeded, come back as doubles in the layouts bart_mcmc_run / bart_mcmc_run_snooker take them:
+ * "support", "unif", "ugamma", and "r1", "r2" after a DE-MC call or "i1", "i2", "iz", "ic",
+ * "usnooker", "usn_offset" after a snooker call.  Returns the number of doubles written or < 0. */
 long long bart_mcmc_get(const char *name, double *out, long long capacity);
 
 #ifdef __cplusplus

@@ -6,9 +6,17 @@ For every ensemble size R it reports, under CUDA-graph replay,
   retrieval_generations_per_s          R / (generation time)
   models_per_s                         R x 10 / (generation time)
 and the wall time of driver.run_demc_ensemble for a fixed number of generations against R
-sequential driver.run_demc calls on the same data and streams.  The card's name and power limit
-are read in the same run.
-usage: bench_ensemble.py [--sizes 1,2,4,8,16,32,64] [--gens 600] [--wall-gens 200] [--out file]"""
+sequential driver.run_demc calls on the same data and streams.  --draws host,device adds, per walk,
+  <walk>_host_streams_wall_s      run_<walk>_ensemble with streams drawn on the host from the rngs
+                                  (host drawing included)
+  <walk>_host_draw_s              that host drawing on its own (demc_draws / snooker_draws)
+  <walk>_host_draw_share          the two above's ratio
+  <walk>_seeded_wall_s            run_<walk>_ensemble(seeds=...): streams drawn on the device
+  <walk>_draw_kernel_ms_per_call  the draw launches of one seeded call of --wall-gens generations
+                                  (bart_kernel_stats, a profiled call of its own)
+The card's name, power limit and max SM clock are read in the same run.
+usage: bench_ensemble.py [--sizes 1,2,4,8,16,32,64] [--gens 600] [--wall-gens 200]
+                         [--draws host,device] [--out file]"""
 import argparse, json, os, subprocess, sys, tempfile, time
 import numpy as np
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -20,9 +28,12 @@ ap.add_argument("--sizes", default="1,2,4,8,16,32,64")
 ap.add_argument("--chains", type=int, default=10)
 ap.add_argument("--gens", type=int, default=600)
 ap.add_argument("--wall-gens", type=int, default=200)
+ap.add_argument("--draws", default="", help="host,device: time the drivers with each stream source")
 ap.add_argument("--out", default=None)
 a = ap.parse_args()
 sizes = [int(x) for x in a.sizes.split(",")]
+draw_modes = [m for m in a.draws.split(",") if m]
+assert all(m in ("host", "device") for m in draw_modes), a.draws
 
 
 def gpu_info():
@@ -111,6 +122,39 @@ for R in sizes:
     # same kernel family (tests/test_gpu_retrieval_ensemble.py)
     row["ensemble_equals_lone_allparams"] = all(np.array_equal(e["allparams"], l["allparams"])
                                                 for e, l in zip(ens, lone))
+    for walk in ("demc", "snooker") if draw_modes else ():
+        run = driver.run_demc_ensemble if walk == "demc" else driver.run_snooker_ensemble
+        rngs = lambda: [np.random.RandomState(600 + r) for r in range(R)]
+        args = (tr, data[:R], uncert[:R], list(starts[:R]), pmin, pmax, stepsize, wg * nch, nch)
+        if "host" in draw_modes:
+            t0 = time.perf_counter()
+            for g in rngs():
+                if walk == "demc":
+                    driver.demc_draws(g, nch, wg, stepsize[free])
+                else:
+                    driver.snooker_draws(g, nch, nfree, wg, hsize, 1, stepsize[free], pmin[free], pmax[free])
+            row[walk + "_host_draw_s"] = time.perf_counter() - t0
+            t0 = time.perf_counter()
+            run(*args, rngs=rngs())
+            row[walk + "_host_streams_wall_s"] = time.perf_counter() - t0
+            row[walk + "_host_draw_share"] = row[walk + "_host_draw_s"] / row[walk + "_host_streams_wall_s"]
+        if "device" in draw_modes:
+            keys = [(700 + r, 1) for r in range(R)]
+            t0 = time.perf_counter()
+            run(*args, rngs=rngs(), seeds=keys)
+            row[walk + "_seeded_wall_s"] = time.perf_counter() - t0
+            tr.mcmc_init_ensemble(starts[:R], pmin, pmax, stepsize, data[:R], uncert[:R])
+            if walk == "snooker":
+                tr.mcmc_snooker_init(np.stack([d["z0"] for d in snk[:R]]), 1)
+            tr.mcmc_seed(np.array(keys, dtype=np.uint64))
+            L = api.lib()
+            L.bart_profile_enable(1)
+            L.bart_profile_reset()
+            tr.mcmc_run_seeded(wg)
+            L.bart_profile_enable(0)
+            st = api.kernel_stats().get("mcmc_draws", dict(launches=0, ms=float("nan")))
+            row[walk + "_draw_kernel_ms_per_call"] = st["ms"] / max(1, st["launches"])
+            L.bart_profile_reset()
     rows.append(row)
     print(json.dumps(row), flush=True)
 
@@ -120,6 +164,7 @@ out = {"workload": "WASP-12b eclipse shape, %d chains per retrieval, 9 parameter
        "device": api.device_info() if hasattr(api, "device_info") else None,
        "nvidia_smi_name_power_limit_max_sm_clock": gpu_info(),
        "generations_timed": ngen,
+       "draws": draw_modes,
        "rows": rows,
        "demc_speedup_vs_R1_per_retrieval_generation": {
            r["nretr"]: r["demc_retrieval_generations_per_s"] / base["demc_retrieval_generations_per_s"]
