@@ -107,6 +107,7 @@ def lib():
     L.bart_mcmc_run_snooker.argtypes = [C.c_int, dp, ip, ip, ip, ip, dp, ip, dp, dp]
     L.bart_mcmc_seed.argtypes = [C.POINTER(C.c_ulonglong)]
     L.bart_mcmc_run_seeded.argtypes = [C.c_int]
+    L.bart_mcmc_retain.argtypes = [C.c_int, ip]
     L.bart_mcmc_get.restype = C.c_longlong
     L.bart_mcmc_get.argtypes = [C.c_char_p, dp, C.c_longlong]
     L.bart_set_error_mode(1)
@@ -446,6 +447,17 @@ class Transit:
             self._mc_niter = niter
             if self._mc_walk == "snooker":
                 self._mc_zsize += len(range(0, niter, self._mc_thinning)) + 1
+
+    def mcmc_retain(self, keep):
+        """Keep retrievals keep[0] < keep[1] < ... (positions in the current loop) and drop the
+        others (bart_mcmc_retain): afterwards the mcmc_* calls take and return arrays behind
+        [len(keep)], retrieval j being the old keep[j].  What describes the last run call
+        (allparams, allmodel, models, the streams) is refused until the next run call."""
+        keep = np.ascontiguousarray(keep, dtype=np.int32)
+        if keep.ndim != 1:
+            raise BartError("keep must be a list of retrieval positions")
+        _check(lib().bart_mcmc_retain(len(keep), keep.ctypes.data_as(ip)))
+        self._mc_shape = (len(keep),) + self._mc_shape[1:]
 
     # the last run call's random streams: shape behind [R] and dtype
     _STREAMS = {"support": (("n", "c", "f"), np.float64), "unif": (("n", "c"), np.float64),

@@ -848,4 +848,73 @@ void launch_mcmc_draws(const DrawArgs &d, cudaStream_t s) {
   usn_rows_kernel<<<blocks, 256, 0, s>>>(d);
 }
 
+// ---------------------------------------------------------------------------------------
+// bart_mcmc_retain: a batched strided gather.  Entry k owns blocks [first, first + nblocks) of the
+// one launch; a group of `gs` threads (a power of two <= 32) copies one retrieval block
+// ("row": outer index o, kept retrieval j) in vectors of `vec` bytes, so the snooker history,
+// which is most of the bytes, moves in 16-byte loads and stores.  Integer division happens once
+// per row, not per vector.
+constexpr int kRetainThreads = 256;
+struct RetainJob {
+  const void *src;
+  void *dst;
+  unsigned rows, filled, n_in;             // rows = outer * nkeep; n_in vectors per row
+  int vec, gs_log2, first, nblocks;
+};
+struct RetainLaunch {
+  RetainJob j[kMaxRetainCopies];
+  int n, nretr, nkeep;
+  const int *keep;
+};
+
+template <class V>
+__device__ __forceinline__ void retain_rows(const RetainJob &c, const RetainLaunch &a) {
+  const unsigned gs = 1u << c.gs_log2, lane = threadIdx.x & (gs - 1);
+  const unsigned ngroups = (unsigned)c.nblocks * (kRetainThreads >> c.gs_log2);
+  const V *src = (const V *)c.src;
+  V *dst = (V *)c.dst;
+  for (unsigned s = ((blockIdx.x - c.first) * kRetainThreads + threadIdx.x) >> c.gs_log2; s < c.rows;
+       s += ngroups) {
+    const unsigned o = s / (unsigned)a.nkeep, j = s - o * (unsigned)a.nkeep;
+    const V *from = src + ((size_t)min(o, c.filled) * a.nretr + __ldg(a.keep + j)) * c.n_in;
+    V *to = dst + (size_t)s * c.n_in;
+    for (unsigned e = lane; e < c.n_in; e += gs) to[e] = from[e];
+  }
+}
+
+__global__ void __launch_bounds__(kRetainThreads) mcmc_retain_kernel(const __grid_constant__ RetainLaunch a) {
+  int k = 0;
+  while (k + 1 < a.n && (int)blockIdx.x >= a.j[k + 1].first) k++;
+  const RetainJob &c = a.j[k];
+  if (c.vec == 16) retain_rows<int4>(c, a);
+  else if (c.vec == 8) retain_rows<int2>(c, a);
+  else retain_rows<int>(c, a);
+}
+
+void launch_mcmc_retain(const RetainArgs &a, cudaStream_t s) {
+  RetainLaunch L{};
+  L.nretr = a.nretr; L.nkeep = a.nkeep; L.keep = a.keep;
+  int blocks = 0;
+  for (int k = 0; k < a.n; k++) {
+    const RetainCopy &c = a.c[k];
+    const uintptr_t align = (uintptr_t)c.src | (uintptr_t)c.dst | (uintptr_t)c.inner;
+    const int vec = align % 16 == 0 ? 16 : align % 8 == 0 ? 8 : 4;
+    RetainJob &j = L.j[L.n];
+    j.src = c.src; j.dst = c.dst; j.vec = vec;
+    j.rows = (unsigned)(c.outer * a.nkeep);
+    j.filled = (unsigned)std::min(c.filled, c.outer - 1);
+    j.n_in = (unsigned)(c.inner / vec);
+    j.gs_log2 = 0;
+    while ((1u << j.gs_log2) < j.n_in && j.gs_log2 < 5) j.gs_log2++;
+    const long long threads = (long long)j.rows << j.gs_log2;
+    if (threads == 0) continue;
+    j.first = blocks;
+    j.nblocks = (int)std::min<long long>((threads + kRetainThreads - 1) / kRetainThreads, 148 * 16);
+    blocks += j.nblocks;
+    L.n++;
+  }
+  if (!blocks) return;
+  mcmc_retain_kernel<<<blocks, kRetainThreads, 0, s>>>(L);
+}
+
 }  // namespace bart

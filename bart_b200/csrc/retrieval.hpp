@@ -10,6 +10,7 @@
 //   K11 mcmc_draw_kernel,       the random streams of a seeded call from per-retrieval Philox
 //       usn_scan_kernel,        keys (philox.cuh): MC3's constructions (mcmc.py:484-507,529-556),
 //       usn_rows_kernel         other random numbers
+//   K12 mcmc_retain_kernel      compaction of the loop state to a subset of its retrievals
 #pragma once
 #include "device.cuh"
 #include <cuda_runtime.h>
@@ -125,6 +126,23 @@ struct DrawArgs {
 };
 // draw kernel, then (snooker) the usn_off scan and the factor rows
 void launch_mcmc_draws(const DrawArgs &d, cudaStream_t s);
+
+// bart_mcmc_retain: every array of the loop state is laid out [outer][nretr][inner]; one entry
+// gathers retrievals keep[0..nkeep) of one array into a new one laid out [outer][nkeep][inner].
+// Outer rows >= `filled` are alike (unfilled history rows) and are all read from row `filled`.
+struct RetainCopy {
+  const void *src;
+  void *dst;
+  long long outer, filled, inner;          // inner: bytes of one retrieval's block
+};
+constexpr int kMaxRetainCopies = 32;
+struct RetainArgs {
+  RetainCopy c[kMaxRetainCopies];
+  int n, nretr, nkeep;
+  const int *keep;                         // device, [nkeep]
+};
+// one launch for every entry
+void launch_mcmc_retain(const RetainArgs &a, cudaStream_t s);
 
 // one warp per (retrieval, chain)
 void launch_demc_propose(const McmcDev &mc, cudaStream_t s);

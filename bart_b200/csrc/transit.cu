@@ -26,7 +26,9 @@
 #include <map>
 #include <algorithm>
 #include <functional>
+#include <memory>
 #include <optional>
+#include <type_traits>
 #include <sys/stat.h>
 
 namespace bart {
@@ -145,6 +147,9 @@ struct Config {
   DevBuf<unsigned long long> d_mckeys;
   DevBuf<double> d_mcstep;
   bool mc_seeded = false;
+  // bart_mcmc_retain dropped retrievals since the last run call: that call's traces, models and
+  // streams no longer match the loop's retrievals
+  bool mc_retained = false;
 };
 
 // The process: the device, its streams, the communicator and peer window, profiling and debug
@@ -848,9 +853,21 @@ static void rank_barrier() {
   if (e != cudaSuccess) fail("CUDA execution failed: %s", cudaGetErrorString(e));
 }
 
+// this rank's block of the flattened population and the band-flux buffers of its size (the MCMC
+// bookkeeping is replicated, so every rank computes the same partition)
+static void mcmc_partition() {
+  const int ntot = G.mc.nretr * G.mc.nchains, ndata = G.mc.ndata;
+  chain_block(ntot, G.world, G.rank, &G.mc_lo, &G.mc_hi);
+  G.mc_pad = ntot / G.world + (ntot % G.world ? 1 : 0);
+  G.d_mcband.ensure((size_t)G.mc_pad * ndata);
+  G.d_mcgather.ensure((size_t)G.mc_pad * ndata * G.world);
+  CUDA_OK(cudaMemsetAsync(G.d_mcband.p, 0, (size_t)G.mc_pad * ndata * 8, G.stream));
+}
+
 // niter generations of the walk set up in G.mc, queued and awaited
 static void mcmc_run_generations(int niter) {
   McmcDev &mc = G.mc;
+  G.mc_retained = false;
   CUDA_OK(cudaMemsetAsync(mc.iter, 0, (size_t)mc.nretr * sizeof(int), G.stream));
   if (G.mc_graph) { cudaGraphExecDestroy(G.mc_graph); G.mc_graph = nullptr; }
   ensure_params_buffers(G.mc_hi - G.mc_lo);
@@ -1906,15 +1923,11 @@ int bart_mcmc_init_ensemble(int nretr, int nchains, int npars, const double *par
   std::vector<double> step;
   for (int f = 0; f < mc.nfree; f++) step.push_back(stepsize[mc.ifree[f]]);
   upload(G.d_mcstep, step);
-  G.mc_seeded = false;
+  G.mc_seeded = G.mc_retained = false;
   G.mc = mc;
   G.mc_ztemplate = p0;
   G.mc_zsize = 0;
-  chain_block(ntot, G.world, G.rank, &G.mc_lo, &G.mc_hi);
-  G.mc_pad = ntot / G.world + (ntot % G.world ? 1 : 0);
-  G.d_mcband.ensure((size_t)G.mc_pad * ndata);
-  G.d_mcgather.ensure((size_t)G.mc_pad * ndata * G.world);
-  CUDA_OK(cudaMemsetAsync(G.d_mcband.p, 0, (size_t)G.mc_pad * ndata * 8, G.stream));
+  mcmc_partition();
   G.d_mccur.ensure((size_t)ntot * ndata);
   CUDA_OK(cudaMemsetAsync(G.d_mccur.p, 0, (size_t)ntot * ndata * 8, G.stream));
   G.mc.curmodel = G.d_mccur.p;
@@ -2216,6 +2229,85 @@ int bart_mcmc_run_seeded(int niter) {
   API_END_INT
 }
 
+// keep retrievals keep[0] < ... < keep[nkeep-1] of the loop and drop the others.  One gather launch
+// moves every per-retrieval and per-chain array and the snooker history into buffers sized for
+// nkeep, which replace the old ones, so the dropped retrievals' memory is freed; everything sized by
+// the population (rank partition, band buffers, the generation graph) follows.  Generation counters
+// are untouched: a seeded retrieval keeps drawing what it would have drawn.
+int bart_mcmc_retain(int nkeep, const int *keep) {
+  API_BEGIN
+  if (!G.mc_ready) fail("bart_mcmc_init has not been called");
+  McmcDev &mc = G.mc;
+  const int nr = mc.nretr;
+  if (nkeep < 1 || nkeep > nr)
+    fail("bart_mcmc_retain: %d retrievals to keep, the loop has %d (keep 1 to %d)", nkeep, nr, nr);
+  if (!keep) fail("bart_mcmc_retain: no positions");
+  for (int j = 0; j < nkeep; j++) {
+    if (keep[j] < 0 || keep[j] >= nr)
+      fail("bart_mcmc_retain: keep[%d] = %d is not a position of the loop's %d retrievals", j, keep[j], nr);
+    if (j > 0 && keep[j] <= keep[j - 1])
+      fail("bart_mcmc_retain: keep[%d] = %d follows %d: positions must be strictly increasing, without "
+           "repeats", j, keep[j], keep[j - 1]);
+  }
+  if (nkeep == nr) return 0;                   // strictly increasing in [0, nr): every retrieval
+  const size_t nc = mc.nchains, np = mc.npars, nd = mc.ndata;
+  DevBuf<int> d_keep;
+  upload(d_keep, std::vector<int>(keep, keep + nkeep));
+  RetainArgs a{};
+  a.nretr = nr; a.nkeep = nkeep; a.keep = d_keep.p;
+  std::vector<std::function<void()>> swap;
+  // array `buf` laid out [outer][nr][inner] -> a new buffer [outer][nkeep][inner] that replaces it
+  auto add = [&](auto &buf, size_t outer, size_t inner, size_t filled) {
+    using T = std::remove_reference_t<decltype(*buf.p)>;
+    if (a.n == kMaxRetainCopies || outer * nkeep >= (1ull << 31)) fail("bart_mcmc_retain: state too large");
+    auto nb = std::make_shared<DevBuf<T>>(outer * nkeep * inner);
+    a.c[a.n++] = RetainCopy{buf.p, nb->p, (long long)outer, (long long)filled, (long long)(inner * sizeof(T))};
+    swap.push_back([&buf, nb] { buf = std::move(*nb); });
+  };
+  auto add1 = [&](auto &buf, size_t inner) { add(buf, 1, inner, 1); };
+  auto &mb = G.mcb;
+  add1(mb.data, nd); add1(mb.uncert, nd); add1(mb.bestp, np); add1(mb.bestchisq, 1);
+  add1(mb.bestmodel, nd); add1(mb.iter, 1);
+  add1(mb.params, nc * np); add1(mb.nextp, nc * np); add1(mb.currchisq, nc); add1(mb.nextchisq, nc);
+  add1(mb.c2, nc); add1(mb.numaccept, nc); add1(mb.outbounds, nc * mc.nfree); add1(mb.outflag, nc);
+  add1(G.d_mccur, nc * nd);
+  if (G.mc_seeded) add1(G.d_mckeys, 2);
+  if (mc.Z) {
+    add1(mb.zsize, 1); add1(mb.zbest, 1 + np + nd); add1(mb.noproj, nc); add1(mb.slot, nc);
+    // rows from mc_zsize on are unfilled: each holds the template, so all are read from that row
+    add(G.d_Z, G.mc_zcap, nc * np, G.mc_zsize);
+    add(G.d_Zchisq, G.mc_zcap, nc, G.mc_zsize);
+  }
+  {
+    KernelScope ks("mcmc_retain");
+    launch_mcmc_retain(a, G.stream);
+    check_launch("mcmc_retain");
+  }
+  finish_stream();
+  for (auto &f : swap) f();
+  mc.data = mb.data.p; mc.uncert = mb.uncert.p; mc.bestp = mb.bestp.p; mc.bestchisq = mb.bestchisq.p;
+  mc.bestmodel = mb.bestmodel.p; mc.iter = mb.iter.p;
+  mc.params = mb.params.p; mc.nextp = mb.nextp.p; mc.currchisq = mb.currchisq.p;
+  mc.nextchisq = mb.nextchisq.p; mc.c2 = mb.c2.p; mc.numaccept = mb.numaccept.p;
+  mc.outbounds = mb.outbounds.p; mc.outflag = mb.outflag.p; mc.curmodel = G.d_mccur.p;
+  if (mc.Z) {
+    mc.zsize = mb.zsize.p; mc.zbest = mb.zbest.p; mc.noproj = mb.noproj.p; mc.slot = mb.slot.p;
+    mc.Z = G.d_Z.p; mc.Zchisq = G.d_Zchisq.p;
+  }
+  std::vector<double> tpl((size_t)nkeep * nc * np);
+  for (int j = 0; j < nkeep; j++)
+    std::copy_n(G.mc_ztemplate.begin() + (size_t)keep[j] * nc * np, nc * np, tpl.begin() + (size_t)j * nc * np);
+  G.mc_ztemplate.swap(tpl);
+  mc.nretr = nkeep;
+  if (G.mc_graph) { cudaGraphExecDestroy(G.mc_graph); G.mc_graph = nullptr; }
+  mcmc_partition();
+  ensure_params_buffers(G.mc_hi - G.mc_lo);
+  finish_stream();
+  G.mc_retained = true;
+  return 0;
+  API_END_INT
+}
+
 // the last run call's random streams as doubles, in the layouts bart_mcmc_run (support, r1, r2,
 // unif, ugamma) / bart_mcmc_run_snooker (support, i1, i2, iz, ic, usnooker, usn_offset, unif,
 // ugamma) take them; 0 before the first run
@@ -2269,6 +2361,12 @@ long long bart_mcmc_get(const char *name, double *out, long long capacity) {
   const McmcDev &mc = G.mc;
   const long long ntot = (long long)mc.nretr * mc.nchains;
   std::string n(name);
+  const bool of_last_call = n == "allparams" || n == "allmodel" || n == "models" || n == "support" ||
+                            n == "r1" || n == "r2" || n == "unif" || n == "ugamma" || n == "i1" ||
+                            n == "i2" || n == "iz" || n == "ic" || n == "usnooker" || n == "usn_offset";
+  if (of_last_call && G.mc_retained)
+    fail("bart_mcmc_get(%s): it describes the last run call, whose retrievals bart_mcmc_retain has "
+         "changed since; fetch it before retaining or after the next run call", name);
   const double *src = nullptr;
   long long cnt = 0;
   if (n == "allparams") { src = mc.allparams; cnt = ntot * mc.nfree * mc.chainsize; }

@@ -326,7 +326,7 @@ def gr_checkpoints(chainsize):
 
 
 def run_segments(run, fetch, chainsize, burnin=0, thinning=1, grtest=False, grexit=False, nold=0,
-                 old=None, max_segment=None):
+                 old=None, max_segment=None, retire=None):
     """Drive a device-resident walk in the segments MC3's loop is observable in (mcmc.py:662-690).
     `run(lo, hi)` advances generations [lo, hi) (state stays on the device); `fetch()` returns that
     call's allparams / allmodel pieces, [nchains][...][hi - lo] behind any leading axes (the
@@ -334,32 +334,77 @@ def run_segments(run, fetch, chainsize, burnin=0, thinning=1, grtest=False, grex
     caps the generations of one call (the host arrays of a call stay bounded).  `old` =
     (allparams, allmodel) of the runs being resumed (nold iterations).  Returns (allparams,
     allmodel, psrf history [(iteration, psrf[leading axes...][nfree])], number of iterations in
-    the traces)."""
+    the traces).
+
+    grexit="each" (with grtest, traces [R][nchains][...]): MC3's exit rule for every retrieval on
+    its own.  A retrieval whose PSRF passes at two consecutive checkpoints stops there, exactly as
+    that retrieval alone with grexit=True would.  `retire(done, keep)` is then called, before the
+    next segment, with the positions (in the current fetch) of the retrievals that stop and of those
+    that go on (possibly none); it must leave `run` and `fetch` serving the `keep` ones only, and
+    returns the `max_segment` of the smaller population (anything when `keep` is empty).  The run ends when every retrieval has stopped or at
+    chainsize.  Returns per-retrieval lists, in the original order: (allparams, allmodel, psrf
+    history [(iteration, psrf[nfree])], number of iterations in the traces)."""
+    each = grexit == "each"
+    if each and (not grtest or retire is None):
+        raise ValueError('grexit="each" needs grtest=True and a retire callback')
     cuts = gr_checkpoints(chainsize) if grtest else []
-    bounds = list(range(max_segment, chainsize, max_segment)) if max_segment else []
-    edges = sorted(set([c + 1 for c in cuts] + bounds + [chainsize]))
     pieces_p, pieces_m, history = [], [], []
     if old is not None:
         pieces_p.append(old[0]); pieces_m.append(old[1])
+    live = None                      # "each": original indices of the running retrievals
     lo, grflag = 0, False
-    for hi in edges:
+    while lo < chainsize:
+        hi = min([c + 1 for c in cuts if c + 1 > lo] + [chainsize] +
+                 ([(lo // max_segment + 1) * max_segment] if max_segment else []))
         run(lo, hi)
         pp, pm = fetch()
-        pieces_p.append(pp); pieces_m.append(pm)
         lo = hi
         i = hi - 1
-        if grtest and i in cuts and (i + nold) > burnin:
-            allp = np.concatenate(pieces_p, axis=-1)[..., burnin:i + nold + 1:thinning]
-            lead = allp.shape[:-3]
-            psrf = np.array([gelman_rubin(a) for a in allp.reshape((-1,) + allp.shape[-3:])])
-            psrf = psrf.reshape(lead + psrf.shape[-1:])
-            history.append((i, psrf))
-            if np.all(psrf < 1.01):
-                if grexit and grflag:                        # two consecutive passes (mcmc.py:676-683)
+        if not each:
+            pieces_p.append(pp); pieces_m.append(pm)
+        else:
+            if live is None:         # per retrieval: trace pieces, psrf history, grflag, length
+                live = list(range(len(pp)))
+                P = [[old[0][r]] if old is not None else [] for r in live]
+                M = [[old[1][r]] if old is not None else [] for r in live]
+                H, flag, length = [[] for _ in live], [False] * len(live), [nold + chainsize] * len(live)
+            for k, r in enumerate(live):
+                P[r].append(pp[k]); M[r].append(pm[k])
+        if not (grtest and i in cuts and (i + nold) > burnin):
+            continue
+        if each:
+            done = []
+            for k, r in enumerate(live):
+                psrf = gelman_rubin(np.concatenate(P[r], axis=-1)[..., burnin:i + nold + 1:thinning])
+                H[r].append((i, psrf))
+                if np.all(psrf < 1.01):
+                    if flag[r]:                              # two consecutive passes (mcmc.py:676-683)
+                        done.append(k)
+                        length[r] = nold + lo
+                    flag[r] = True
+                else:
+                    flag[r] = False
+            if done and lo < chainsize:               # at the end nobody needs a smaller loop
+                keep = [k for k in range(len(live)) if k not in done]
+                max_segment = retire(done, keep)
+                live = [live[k] for k in keep]
+                if not live:
                     break
-                grflag = True
-            else:
-                grflag = False
+            continue
+        allp = np.concatenate(pieces_p, axis=-1)[..., burnin:i + nold + 1:thinning]
+        lead = allp.shape[:-3]
+        psrf = np.array([gelman_rubin(a) for a in allp.reshape((-1,) + allp.shape[-3:])])
+        psrf = psrf.reshape(lead + psrf.shape[-1:])
+        history.append((i, psrf))
+        if np.all(psrf < 1.01):
+            if grexit and grflag:                            # two consecutive passes (mcmc.py:676-683)
+                break
+            grflag = True
+        else:
+            grflag = False
+    if each:
+        return ([np.concatenate(p, axis=-1) for p in P], [np.concatenate(m, axis=-1) for m in M], H,
+                length)
     return np.concatenate(pieces_p, axis=-1), np.concatenate(pieces_m, axis=-1), history, nold + lo
 
 
@@ -535,13 +580,14 @@ def _retrieve(transit, walk, data, uncert, params, pmin, pmax, stepsize, numit, 
         transit.mcmc_resume(nold, old[2])
     if keys is not None:
         transit.mcmc_seed(keys)
+    active = list(range(nretr))          # the loop's retrievals (grexit="each" retains a subset)
     if walk == "demc":
         if keys is not None:
             run = lambda lo, hi: transit.mcmc_run_seeded(hi - lo)
         else:
             if draws is None:
                 draws = [demc_draws(rng, nchains, chainsize, stepsize[ifree]) for rng in rngs]
-            run = lambda lo, hi: transit.mcmc_run(*stack_demc_draws(draws, lo, hi))
+            run = lambda lo, hi: transit.mcmc_run(*stack_demc_draws([draws[r] for r in active], lo, hi))
         zkeys, extra = (), 0
     else:
         if hsize < nchains:                                          # mcmc.py:233-235
@@ -554,24 +600,42 @@ def _retrieve(transit, walk, data, uncert, params, pmin, pmax, stepsize, numit, 
                 draws = [snooker_draws(rng, nchains, len(ifree), chainsize, hsize, thinning,
                                        stepsize[ifree], pmin[ifree], pmax[ifree]) for rng in rngs]
             z0 = np.stack([d["z0"] for d in draws])
-            run = lambda lo, hi: transit.mcmc_run_snooker(*stack_snooker_draws(draws, lo, hi))
+            run = lambda lo, hi: transit.mcmc_run_snooker(
+                *stack_snooker_draws([draws[r] for r in active], lo, hi))
         transit.mcmc_snooker_init(z0, thinning)
         zkeys, extra = ("Z", "Zchisq"), len(ifree) / 5 + 2
+    cap = lambda n: _segment_cap(n, nchains, len(ifree), data.shape[1], extra, streams=keys is None)
+    state = {}                            # original index -> final state of the loop's arrays
+
+    def take_state(positions):
+        got = {k: transit.mcmc_get(k) for k in ("params", "currchisq", "numaccept", "outbounds", "bestp",
+                                                "bestchisq", "bestmodel", "models") + zkeys}
+        for k in positions:
+            state[active[k]] = {name: v[k] for name, v in got.items()}
+
+    def retire(done, keep):               # grexit="each": `done` stop, the loop keeps `keep`
+        take_state(done)
+        if keep:
+            transit.mcmc_retain(keep)
+        active[:] = [active[k] for k in keep]
+        return cap(len(active)) if active else None     # none left: the run ends here
+
     allp, allm, history, chainlen = run_segments(
         run, lambda: (transit.mcmc_get("allparams"), transit.mcmc_get("allmodel")), chainsize,
         burnin=burnin, thinning=thinning, grtest=grtest, grexit=grexit, nold=nold,
-        old=None if old is None else old[:2],
-        max_segment=_segment_cap(nretr, nchains, len(ifree), data.shape[1], extra, streams=keys is None))
-    got = {k: transit.mcmc_get(k) for k in ("params", "currchisq", "numaccept", "outbounds", "bestp",
-                                            "bestmodel", "models") + zkeys}
-    bestchisq = transit.mcmc_get("bestchisq")
+        old=None if old is None else old[:2], max_segment=cap(nretr), retire=retire)
+    if active:
+        take_state(range(len(active)))
+    if grexit != "each":                  # one length and psrf history for all: split them
+        history = [[(i, psrf[r]) for i, psrf in history] for r in range(nretr)]
+        chainlen = [chainlen] * nretr
     outs = []
     for r in range(nretr):
-        out = {k: v[r] for k, v in got.items()}
+        out = dict(state[r])
         out["allparams"], out["allmodel"] = allp[r], allm[r]
-        out["psrf"] = [(i, psrf[r]) for i, psrf in history]
-        out["bestchisq"] = float(bestchisq[r])
-        out["allstack"] = np.hstack([allp[r, c, :, burnin:chainlen] for c in range(nchains)])  # mcmc.py:692-695
+        out["psrf"] = history[r]
+        out["bestchisq"] = float(out.pop("bestchisq"))
+        out["allstack"] = np.hstack([allp[r][c, :, burnin:chainlen[r]] for c in range(nchains)])  # mcmc.py:692-695
         _save_mc3_files(out, savefile[r] if savefile is not None else None,
                         savemodel[r] if savemodel is not None else None)
         outs.append(out)
@@ -589,14 +653,26 @@ def run_demc_ensemble(transit, data, uncert, params, pmin, pmax, stepsize, numit
     of R dicts with run_demc's keys; retrieval r equals run_demc on its own data and streams.
     seeds: one seed per retrieval (see run_demc's seed; not with draws); retrieval r then equals
     run_demc with seed=seeds[r].
-    grexit is refused: the retrievals would stop at different iterations.  One device call's host
+    grexit="each" (with grtest=True) stops every retrieval at its own convergence, by MC3's rule
+    (two consecutive checkpoints with every PSRF < 1.01): its outputs are then those of run_demc
+    with grexit=True on its own, and the retrievals still running go on without it in a smaller
+    loop (Transit.mcmc_retain).  grexit=True is refused as ambiguous.  One device call's host
     arrays are bounded, the whole run's are not (see ENSEMBLE_CALL_BYTES)."""
-    if grexit:
-        raise ValueError("grexit is not offered for ensembles: the retrievals would stop at "
-                         "different iterations")
+    _check_ensemble_grexit(grtest, grexit)
     return _retrieve(transit, "demc", data, uncert, params, pmin, pmax, stepsize, numit, nchains,
                      rngs, draws, savefile, savemodel, prior=prior, priorlow=priorlow, burnin=burnin,
-                     fgamma=fgamma, fepsilon=fepsilon, thinning=thinning, grtest=grtest, seeds=seeds)
+                     fgamma=fgamma, fepsilon=fepsilon, thinning=thinning, grtest=grtest, grexit=grexit,
+                     seeds=seeds)
+
+
+def _check_ensemble_grexit(grtest, grexit):
+    if grexit == "each":
+        if not grtest:
+            raise ValueError('grexit="each" needs grtest=True: retrievals stop at the convergence '
+                             'checkpoints')
+    elif grexit:
+        raise ValueError('grexit=True is not offered for ensembles: the retrievals converge at '
+                         'different iterations; grexit="each" stops each one at its own')
 
 
 def run_snooker_ensemble(transit, data, uncert, params, pmin, pmax, stepsize, numit, nchains,
@@ -606,11 +682,9 @@ def run_snooker_ensemble(transit, data, uncert, params, pmin, pmax, stepsize, nu
     """`run_snooker` for R retrievals in one device loop (arguments as run_demc_ensemble; draws as
     snooker_draws returns them).  hsize and thinning are shared, so every retrieval's history grows
     on the same schedule.  seeds as in run_demc_ensemble.  Returns a list of R dicts with
-    run_snooker's keys."""
-    if grexit:
-        raise ValueError("grexit is not offered for ensembles: the retrievals would stop at "
-                         "different iterations")
+    run_snooker's keys.  grexit="each" as in run_demc_ensemble."""
+    _check_ensemble_grexit(grtest, grexit)
     return _retrieve(transit, "snooker", data, uncert, params, pmin, pmax, stepsize, numit, nchains,
                      rngs, draws, savefile, savemodel, prior=prior, priorlow=priorlow, burnin=burnin,
                      fgamma=fgamma, fepsilon=fepsilon, thinning=thinning, hsize=hsize, grtest=grtest,
-                     seeds=seeds)
+                     grexit=grexit, seeds=seeds)

@@ -204,7 +204,10 @@ int  bart_voigt_profile(int idop, int ilor, float *out, long long capacity, long
 /* ===================================================================================== */
 /* Part 3 -- the retrieval loop around the forward model, on the device (additive).
  * In the reference these run in Python on the host, once per proposal and per chain:
- * code/BARTfunc.py:309-399 (one MPI worker per chain) and modules/MCcubed/MCcubed/mc/mcmc.py.   */
+ * code/BARTfunc.py:309-399 (one MPI worker per chain) and modules/MCcubed/MCcubed/mc/mcmc.py.
+ * One loop holds an ensemble of independent retrievals (bart_mcmc_init_ensemble); between run
+ * calls bart_mcmc_retain shrinks it to the retrievals still running, which is how the driver
+ * stops each retrieval at its own MC3 convergence checkpoint (driver.py, grexit="each").        */
 
 #define BART_REJ_TBOUNDS 16  /* temperature profile outside [Tmin, Tmax] (BARTfunc.py:327-330)   */
 #define BART_REJ_ABUND   32  /* sum of metal abundances > 1 (BARTfunc.py:339-344)                */
@@ -324,6 +327,21 @@ int  bart_mcmc_run_snooker(int niter, const double *support, const int *i1, cons
  * bart_mcmc_run_seeded refuses to run before bart_mcmc_seed.                                     */
 int  bart_mcmc_seed(const unsigned long long *keys);
 int  bart_mcmc_run_seeded(int niter);
+/* Keep retrievals keep[0] < keep[1] < ... < keep[nkeep-1] (positions in the current loop) and
+ * drop the others: afterwards the loop has nkeep retrievals, retrieval j being the old keep[j], and
+ * every call takes and returns arrays behind the new [nkeep] axis.  This is how an ensemble stops
+ * each retrieval at its own convergence: the retrievals that are done leave, and the next run
+ * calls evaluate only the others' models.  One gather launch moves the kept retrievals' state
+ * (chains, best fits, data, Philox keys, snooker histories) into buffers sized for nkeep; the
+ * dropped retrievals' device memory is freed.  A kept retrieval's chains are unchanged: it goes on
+ * exactly as it would have in the larger loop, seeded calls included (draws depend on the global
+ * iteration, which retaining does not touch).  bart_mcmc_get returns the kept retrievals' state;
+ * what describes the last run call ("allparams", "allmodel", "models", the streams) is refused
+ * until the next run call, so fetch it before retaining.  Allowed any time after
+ * bart_mcmc_init_ensemble, before the first run and before bart_mcmc_snooker_init too; keeping
+ * every retrieval is a no-op.  Refused: nkeep < 1 or > nretr, positions out of range, not strictly
+ * increasing, or repeated.                                                                      */
+int  bart_mcmc_retain(int nkeep, const int *keep);
 /* "allparams" [nchains][nfree][niter] (MC3's `savefile` array, BART's output.npy), "allmodel"
  * [nchains][ndata][niter] (MC3's `savemodel` array, mcmc.py:636-651,849-850: the model of every
  * chain's current state, zeros until its first acceptance like the reference), "params",
